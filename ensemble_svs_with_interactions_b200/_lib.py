@@ -99,6 +99,22 @@ class WavenetBlockParams(C.Structure):
     ]
 
 
+class WavenetArParams(C.Structure):
+    _fields_ = [
+        ("wpack", C.c_void_p), ("cproj", C.c_void_p), ("u", C.c_void_p), ("y", C.c_void_p), ("logits", C.c_void_p),
+        ("hist", C.c_void_p),
+        ("B", C.c_int32), ("T", C.c_int32), ("steps", C.c_int32), ("out_dim", C.c_int32), ("R", C.c_int32), ("G", C.c_int32),
+        ("S", C.c_int32), ("layers", C.c_int32), ("stacks", C.c_int32), ("ksize", C.c_int32),
+    ]
+
+
+class WavenetArWeights(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in (
+        "first_v", "first_g", "first_b", "conv_v", "conv_g", "conv_b", "cond_v", "cond_g", "skip_v", "skip_g", "skip_b",
+        "out_v", "out_g", "out_b", "last1_v", "last1_g", "last1_b", "last3_v", "last3_g", "last3_b")] + [
+        (n, C.c_int32) for n in ("out_dim", "R", "G", "S", "cin", "layers", "stacks", "ksize")]
+
+
 class SegGemmParams(C.Structure):
     _fields_ = [
         ("x", C.c_void_p * 4), ("ldx", C.c_int32 * 4), ("kx", C.c_int32 * 4), ("shift", C.c_int32 * 4), ("nseg", C.c_int32),
@@ -173,6 +189,10 @@ _SIGNATURES = {
     "svsk_diffnet_pack_block": [_V, _V, _V, _V, _V, _I, _I, _V],
     "svsk_wavenet_block_f32": [C.POINTER(WavenetBlockParams), _V],
     "svsk_wavenet_pack_f32": [_V, _V, _V, _V, _V, _V, _I, _I, _I, _I, _I, _V],
+    "svsk_wavenet_ar_f32": [C.POINTER(WavenetArParams), _V],
+    "svsk_wavenet_ar_supported": [_I, _I, _I, _I, _I, _I, _I],
+    "svsk_wavenet_ar_sizes": [_I, _I, _I, _I, _I, _I, _I, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)],
+    "svsk_wavenet_ar_pack_f32": [C.POINTER(WavenetArWeights), _V, _V, _V],
     "svsk_usfgan_source": [_V, _V, _V, C.c_longlong, _V, _V, _I, _I, _I, _I, _I, _F, _F, _V],
     "svsk_seggemm_bf16": [C.POINTER(SegGemmParams), _V],
     "svsk_wgrad_bf16": [C.POINTER(WgradParams), _V],

@@ -242,6 +242,68 @@ def wavenet_block_f32(x, c, w1t, b1, w2t, b2, skips, *, ksize, dilation, first, 
     return out
 
 
+def wavenet_ar_supported(out_dim, R, G, S, layers, stacks, ksize):
+    return bool(L.lib().svsk_wavenet_ar_supported(out_dim, R, G, S, layers, stacks, ksize))
+
+
+def wavenet_ar_sizes(out_dim, R, G, S, layers, stacks, ksize):
+    """(floats of the packed weights, floats of one track's tap ring buffer) of svsk_wavenet_ar_f32."""
+    pack, hist = C.c_longlong(), C.c_longlong()
+    rc = L.lib().svsk_wavenet_ar_sizes(out_dim, R, G, S, layers, stacks, ksize, C.byref(pack), C.byref(hist))
+    if rc != 0:
+        raise RuntimeError(f"libsvsk wavenet_ar_sizes failed (code {rc}): {L.lib().svsk_last_error().decode()}")
+    return pack.value, hist.value
+
+
+_AR_WEIGHTS = ("first_v", "first_g", "first_b", "conv_v", "conv_g", "conv_b", "cond_v", "cond_g", "skip_v", "skip_g", "skip_b",
+               "out_v", "out_g", "out_b", "last1_v", "last1_g", "last1_b", "last3_v", "last3_g", "last3_b")
+
+
+def wavenet_ar_pack_f32(w, *, out_dim, R, G, S, cin, layers, stacks, ksize):
+    """svsk_wavenet_ar_pack_f32.  w: dict of the fields of svsk_wavenet_ar_weights (fp32 CUDA tensors, per-layer ones
+    stacked over the layers; the *_g gains and conv_b may be None) -> (wpack [pack_floats], wcond [layers*G, cin, 1])."""
+    npack, _ = wavenet_ar_sizes(out_dim, R, G, S, layers, stacks, ksize)
+    dev = w["first_v"].device
+    wpack = torch.empty(npack, device=dev, dtype=f32)
+    wcond = torch.empty((layers * G, cin, 1), device=dev, dtype=f32)
+    p = L.WavenetArWeights()
+    for n in _AR_WEIGHTS:
+        setattr(p, n, L.ptr(w.get(n), f32, n).value)
+    p.out_dim, p.R, p.G, p.S, p.cin, p.layers, p.stacks, p.ksize = out_dim, R, G, S, cin, layers, stacks, ksize
+    L.check(L.lib().svsk_wavenet_ar_pack_f32(C.byref(p), L.ptr(wpack), L.ptr(wcond), L.stream_ptr()), "wavenet_ar_pack_f32")
+    return wpack, wcond
+
+
+def wavenet_ar_f32(wpack, cproj, u, *, out_dim, R, G, S, layers, stacks, ksize, logits=None):
+    """svsk_wavenet_ar_f32: steps = u.shape[1] autoregressive WaveNet steps for B tracks in one launch.
+    wpack from wavenet_ar_pack_f32; cproj [B, layers*G, T] = conv1d_f32(c, wcond) (no bias); u [B, steps] uniforms in
+    [0, 1).  Returns the one-hot samples [B, steps, out_dim]; logits: optional [B, steps, out_dim] output."""
+    npack, nhist = wavenet_ar_sizes(out_dim, R, G, S, layers, stacks, ksize)
+    if u.dim() != 2 or cproj.dim() != 3:
+        raise ValueError(f"wavenet_ar_f32: u must be [B, steps] and cproj [B, layers*G, T], got {tuple(u.shape)} and "
+                         f"{tuple(cproj.shape)}")
+    B, steps = u.shape
+    T = cproj.shape[2]
+    if tuple(cproj.shape[:2]) != (B, layers * G):
+        raise ValueError(f"wavenet_ar_f32: cproj must be [B={B}, layers*G={layers * G}, T], got {tuple(cproj.shape)}")
+    if steps < 1 or steps > T:
+        raise ValueError(f"wavenet_ar_f32: steps={steps} must be in [1, T={T}] (one conditioning frame per step)")
+    if wpack.dim() != 1 or wpack.numel() != npack:
+        raise ValueError(f"wavenet_ar_f32: wpack must hold {npack} floats, got {tuple(wpack.shape)}")
+    if logits is not None and tuple(logits.shape) != (B, steps, out_dim):
+        raise ValueError(f"wavenet_ar_f32: logits must be [{B}, {steps}, {out_dim}], got {tuple(logits.shape)}")
+    p = L.WavenetArParams()
+    p.wpack, p.cproj, p.u = L.ptr(wpack, f32, "wpack"), L.ptr(cproj, f32, "cproj"), L.ptr(u, f32, "u")
+    p.logits = L.ptr(logits, f32, "logits")
+    y = torch.empty((B, steps, out_dim), device=u.device, dtype=f32)
+    hist = torch.empty(B * nhist, device=u.device, dtype=f32)
+    p.y, p.hist = L.ptr(y), L.ptr(hist)
+    p.B, p.T, p.steps, p.out_dim, p.R, p.G, p.S = B, T, steps, out_dim, R, G, S
+    p.layers, p.stacks, p.ksize = layers, stacks, ksize
+    L.check(L.lib().svsk_wavenet_ar_f32(C.byref(p), L.stream_ptr()), "wavenet_ar_f32")
+    return y
+
+
 def usfgan_source(f0, *, hop, sample_rate, dense_factor=4, sine_amp=0.1, noise_amp=0.0, noise=None, sine_out=None,
                   want_sine=True, want_d=True):
     """f0 [B, F] float64 CUDA (Hz, 0 = unvoiced) -> (sine [B, 1, F*hop] fp32 or None, d [B, 1, F*hop] fp32 or None): the

@@ -1,6 +1,6 @@
 """``Conv1d`` parameter holder with the incremental (one-sample) evaluation API of ``nnsvs.wavenet.conv``
-(nnsvs/wavenet/conv.py:9-69).  Used by ``WaveNet.inference`` (autoregressive sampling — sequential, latency-bound,
-outside the metric; SURVEY.md a18 keeps it in PyTorch)."""
+(nnsvs/wavenet/conv.py:9-69).  Used by ``WaveNet.incremental_logits`` and by the host loop of
+``WaveNet.inference`` for CPU tensors and shapes the device sampler (svsk_wavenet_ar_f32) does not cover."""
 import torch
 from torch import nn
 from torch.nn import functional as F

@@ -86,9 +86,74 @@ class WaveNet(nn.Module):
         _L.launch_count += n
         return out.clone().transpose(1, 2)
 
+    def _ar_config(self):
+        """(out_dim, R, G, S, layers, stacks, ksize) when svsk_wavenet_ar_f32 covers this network, else None."""
+        blocks = self.main_conv_layers
+        L = len(blocks)
+        dil = [f.dilation for f in blocks]
+        per = dil.index(1, 1) if 1 in dil[1:] else L
+        if L % per or dil != [2 ** (i % per) for i in range(L)] or len({f.kernel_size for f in blocks}) != 1:
+            return None
+        cfg = (self.out_dim, self.first_conv.out_channels, blocks[0].conv.out_channels, blocks[0].conv1x1_skip.out_channels,
+               L, L // per, blocks[0].kernel_size)
+        return cfg if ops.wavenet_ar_supported(*cfg) else None
+
+    def _ar_packed(self, cfg):
+        """Folded, laid-out weights of the device sampler, rebuilt when any parameter changes."""
+        key = (cfg,) + tuple((q.data_ptr(), q._version) for q in self.parameters())
+        if self.__dict__.get("_ar_key") != key:
+            def vg(mods):
+                if all(hasattr(m, "weight_g") for m in mods):
+                    return (torch.stack([m.weight_v.detach() for m in mods]).to(f32).contiguous(),
+                            torch.stack([m.weight_g.detach().reshape(-1) for m in mods]).to(f32).contiguous())
+                return torch.stack([_w(m) for m in mods]).to(f32).contiguous(), None
+
+            def bias(mods):
+                if any(m.bias is None for m in mods):
+                    return None
+                return torch.stack([m.bias.detach() for m in mods]).to(f32).contiguous()
+
+            blocks = self.main_conv_layers
+            w = {}
+            for name, mods in (("first", [self.first_conv]), ("conv", [f.conv for f in blocks]),
+                               ("cond", [f.conv1x1c for f in blocks]), ("skip", [f.conv1x1_skip for f in blocks]),
+                               ("out", [f.conv1x1_out for f in blocks]), ("last1", [self.last_conv_layers[1]]),
+                               ("last3", [self.last_conv_layers[3]])):
+                w[name + "_v"], w[name + "_g"] = vg(mods)
+                if name != "cond":
+                    w[name + "_b"] = bias(mods)
+            out_dim, R, G, S, layers, stacks, k = cfg
+            self.__dict__["_ar_pack"] = ops.wavenet_ar_pack_f32(
+                w, out_dim=out_dim, R=R, G=G, S=S, cin=blocks[0].conv1x1c.in_channels, layers=layers, stacks=stacks, ksize=k)
+            self.__dict__["_ar_key"] = key
+        return self.__dict__["_ar_pack"]
+
     @torch.no_grad()
-    def inference(self, c, num_time_steps=100, tqdm=lambda x: x):
-        """Autoregressive sampling (wavenet.py:89-149): per-sample ring buffers + categorical draw."""
+    def inference(self, c, num_time_steps=100, tqdm=lambda x: x, *, u=None, logits=None):
+        """Autoregressive sampling (wavenet.py:89-149): c (B, T >= num_time_steps, in_dim) -> one-hot samples
+        (B, num_time_steps, out_dim).
+
+        On CUDA in eval mode, for the shapes svsk_wavenet_ar_supported covers, all steps run in one launch
+        (svsk_wavenet_ar_f32, after one svsk_conv1d_f32 for the conditioning of every layer); ``tqdm`` is not used there.
+        Step t draws the smallest class whose cumulative softmax probability exceeds u[b, t]: ``u`` (B, num_time_steps)
+        fp32 uniforms in [0, 1) is drawn with torch.rand unless given; ``logits`` (B, num_time_steps, out_dim) fp32, if
+        given, receives the logits of every step.  Other inputs run the per-step host loop of the reference (per-layer
+        ring buffers, OneHotCategorical), which takes neither ``u`` nor ``logits``."""
+        cfg = self._ar_config() if c.is_cuda and not self.training else None
+        if cfg is not None:
+            out_dim, R, G, S, layers, stacks, k = cfg
+            self.clear_buffer()
+            wpack, wcond = self._ar_packed(cfg)
+            cproj = ops.conv1d_f32(c[:, :num_time_steps].to(f32).transpose(1, 2).contiguous(), wcond)
+            if u is None:
+                u = torch.rand((c.shape[0], num_time_steps), device=c.device)
+            y = ops.wavenet_ar_f32(wpack, cproj, u, out_dim=out_dim, R=R, G=G, S=S, layers=layers, stacks=stacks, ksize=k,
+                                   logits=logits)
+            self.clear_buffer()
+            return y
+        if u is not None or logits is not None:
+            raise ValueError("WaveNet.inference: u= and logits= need the device sampler (CUDA tensors, eval mode, a shape "
+                             "svsk_wavenet_ar_supported covers)")
         self.clear_buffer()
         B = c.shape[0]
         outputs = []

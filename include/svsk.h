@@ -509,6 +509,51 @@ SVSK_API int svsk_wavenet_block_f32(const svsk_wavenet_block_params* p, void* st
 SVSK_API int svsk_wavenet_pack_f32(const float* wconv, const float* wc, const float* wskip, const float* wout, float* w1t,
                                    float* w2t, int R, int G, int S, int Cc, int ksize, void* stream);
 
+/* WaveNet autoregressive sampling, fp32 — replaces WaveNet.inference (nnsvs/wavenet/wavenet.py:89-149) for B tracks in
+ * one launch.  Per track and step t < steps:
+ *   x_0 = first_conv(onehot(y[t-1])) (the bias alone at t = 0); for each layer l (dilation 2^(l mod layers/stacks)):
+ *   a = conv_l(x_l)[t] (taps at t - (k-1-j) d, zeros before frame 0) + b_l + cproj[b][l G + g][t];
+ *   z = tanh(a[:G/2]) * sigmoid(a[G/2:]);  skip += conv1x1_skip_l(z);  x_{l+1} = conv1x1_out_l(z) + x_l;
+ *   logits = last3(relu(last1(relu(skip))));  p = softmax(logits);
+ *   y[t] = smallest c with u[b][t] < p_0 + .. + p_c (largest c with p_c > 0 if rounding leaves none), written one-hot.
+ * cproj [B][layers G][T] holds conv1x1c of every layer on the conditioning c [B][cin][T]: svsk_conv1d_f32 with
+ * w = wcond [layers G][cin][1] from svsk_wavenet_ar_pack_f32, no bias.  u [B][steps] uniforms in [0, 1) (the caller's
+ * random numbers); y [B][steps][out_dim]; logits [B][steps][out_dim] or NULL; hist: workspace of B * hist_floats
+ * (svsk_wavenet_ar_sizes), no initialisation needed.  steps <= T.  Shapes: svsk_wavenet_ar_supported. */
+typedef struct svsk_wavenet_ar_params {
+  const float* wpack;
+  const float* cproj;
+  const float* u;
+  float* y;
+  float* logits;
+  float* hist;
+  int32_t B, T, steps, out_dim, R, G, S, layers, stacks, ksize;
+} svsk_wavenet_ar_params;
+SVSK_API int svsk_wavenet_ar_f32(const svsk_wavenet_ar_params* p, void* stream);
+/* 1 when svsk_wavenet_ar_f32 covers the WaveNet (out_dim, residual R, gate G, skip S channels, layers, stacks, kernel
+ * size): k R <= 256, G / 2 <= 64, S <= 64, S + R <= 128, out_dim <= 256, layers <= 64 with layers / stacks <= 16. */
+SVSK_API int svsk_wavenet_ar_supported(int out_dim, int R, int G, int S, int layers, int stacks, int ksize);
+/* Floats of the packed weights and of the per-track ring buffer (hist) of a supported WaveNet; SVSK_E_ARG otherwise. */
+SVSK_API int svsk_wavenet_ar_sizes(int out_dim, int R, int G, int S, int layers, int stacks, int ksize, long long* pack_floats,
+                                   long long* hist_floats);
+/* Parameters of a WaveNet as stored in its modules, all device pointers to fp32: each weight is v with its weight-norm
+ * gain g ([rows], NULL = v is the weight itself), per-layer tensors stacked over the layers.  Shapes: first [R][out_dim],
+ * conv [layers][G][R][ksize], cond [layers][G][cin] (no bias), skip [layers][S][G/2], out [layers][R][G/2],
+ * last1 [S][S], last3 [out_dim][S]; biases [rows] per weight (conv_b may be NULL = zeros). */
+typedef struct svsk_wavenet_ar_weights {
+  const float *first_v, *first_g, *first_b;
+  const float *conv_v, *conv_g, *conv_b;
+  const float *cond_v, *cond_g;
+  const float *skip_v, *skip_g, *skip_b;
+  const float *out_v, *out_g, *out_b;
+  const float *last1_v, *last1_g, *last1_b;
+  const float *last3_v, *last3_g, *last3_b;
+  int32_t out_dim, R, G, S, cin, layers, stacks, ksize;
+} svsk_wavenet_ar_weights;
+/* Folds weight norm (w = g v / ||v|| per output row, as torch._weight_norm(v, g, 0)) and lays the weights out for
+ * svsk_wavenet_ar_f32: wpack [pack_floats] and wcond [layers G][cin]. */
+SVSK_API int svsk_wavenet_ar_pack_f32(const svsk_wavenet_ar_weights* w, float* wpack, float* wcond, void* stream);
+
 /* Source signal and dilation factors of the uSFGAN front end from frame-level F0 (nnsvs/usfgan/utils/features.py:
  * SignalGenerator.sinusoid :145-164, dilated_factor :56-75; called per utterance by USFGANWrapper.inference,
  * nnsvs/usfgan/__init__.py:50-63).  f0 [B][F] in Hz as float64 (0 = unvoiced; the sine uses its fp32 rounding like
