@@ -115,6 +115,25 @@ class WavenetArWeights(C.Structure):
         (n, C.c_int32) for n in ("out_dim", "R", "G", "S", "cin", "layers", "stacks", "ksize")]
 
 
+class WavenetBlockTrainParams(C.Structure):
+    _fields_ = [("blk", WavenetBlockParams), ("y", C.c_void_p)]
+
+
+class WavenetDgradParams(C.Structure):
+    _fields_ = [
+        ("dy_in", C.c_void_p), ("wT", C.c_void_p), ("g_next", C.c_void_p), ("g_out", C.c_void_p), ("dS", C.c_void_p),
+        ("y_prev", C.c_void_p), ("wB", C.c_void_p), ("dy_out", C.c_void_p), ("dy_bstride", C.c_int64),
+        ("B", C.c_int32), ("T", C.c_int32), ("R", C.c_int32), ("G", C.c_int32), ("S", C.c_int32), ("ksize", C.c_int32),
+        ("dilation", C.c_int32),
+    ]
+
+
+class WavenetWgradParams(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in (
+        "x_in", "c", "xs", "ys", "gs", "dy", "dS", "skips", "h1", "dh1", "glog", "dilations", "dW", "ws")] + [
+        (n, C.c_int32) for n in ("B", "T", "out_dim", "R", "G", "S", "cin", "layers", "ksize", "splits")]
+
+
 class SegGemmParams(C.Structure):
     _fields_ = [
         ("x", C.c_void_p * 4), ("ldx", C.c_int32 * 4), ("kx", C.c_int32 * 4), ("shift", C.c_int32 * 4), ("nseg", C.c_int32),
@@ -193,6 +212,13 @@ _SIGNATURES = {
     "svsk_wavenet_ar_supported": [_I, _I, _I, _I, _I, _I, _I],
     "svsk_wavenet_ar_sizes": [_I, _I, _I, _I, _I, _I, _I, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)],
     "svsk_wavenet_ar_pack_f32": [C.POINTER(WavenetArWeights), _V, _V, _V],
+    "svsk_wavenet_block_train_f32": [C.POINTER(WavenetBlockTrainParams), _V],
+    "svsk_wavenet_train_sizes": [_I, _I, _I, _I, _I, _I, _I, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)],
+    "svsk_wavenet_train_pack_f32": [C.POINTER(WavenetArWeights), _V, _V],
+    "svsk_wavenet_dgrad_f32": [C.POINTER(WavenetDgradParams), _V],
+    "svsk_wavenet_wgrad_f32": [C.POINTER(WavenetWgradParams), _V],
+    "svsk_wavenet_wnorm_grad_f32": [C.POINTER(WavenetArWeights), _V, _V, _V],
+    "svsk_relu_mask_f32": [_V, _V, _V, C.c_longlong, _V],
     "svsk_usfgan_source": [_V, _V, _V, C.c_longlong, _V, _V, _I, _I, _I, _I, _I, _F, _F, _V],
     "svsk_seggemm_bf16": [C.POINTER(SegGemmParams), _V],
     "svsk_wgrad_bf16": [C.POINTER(WgradParams), _V],

@@ -9,65 +9,14 @@
 // effort on having a frame tile's whole block in one CTA: inputs (all taps + conditioning) staged once in shared
 // memory, the gate pre-activations and z never leave it.  Weights are pre-transposed ([K][out], folded weight norm) so
 // that a warp reads 32 consecutive output channels of one k per load.
-#include "svsk_common.cuh"
+#include "wavenet_f32.cuh"
 
 namespace svsk {
 
-constexpr int kWnTT = 16;  // frames per CTA
-constexpr int kWnKC = 32;  // weight rows staged per chunk
-
-// acc[i] += sum_k w[k][col] * in[k][tg * 8 + i] for one (column, half tile) item per thread, K rows of weights streamed
-// through shared memory in chunks of kWnKC rows: all threads fetch the NEXT chunk into registers (coalesced float4, many
-// loads in flight) before they compute on the current one, so the L2 latency of a chunk hides behind 32 k-steps of FMAs.
-// ncols is a multiple of 4; w_s holds kWnKC * ncols floats.  Must be called by all 256 threads.
-__device__ __forceinline__ void wn_gemm_tile(const float* __restrict__ w, int K, int ncols, const float* in_s, float* w_s,
-                                             int n_items, float (&acc)[2][8]) {
-  const int vec_per_chunk = kWnKC * ncols / 4;           // float4s per chunk
-  constexpr int kMaxV = 8;                               // per thread: chunk of 32 x 256 floats at most
-  float4 nxt[kMaxV];
-  auto fetch = [&](int k0) {
-#pragma unroll
-    for (int v = 0; v < kMaxV; ++v) {
-      const int i = threadIdx.x + v * 256;
-      nxt[v] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (i < vec_per_chunk) {
-        const int r = (i * 4) / ncols;
-        if (k0 + r < K) nxt[v] = *reinterpret_cast<const float4*>(w + (size_t)k0 * ncols + (size_t)i * 4);
-      }
-    }
-  };
-  fetch(0);
-  for (int k0 = 0; k0 < K; k0 += kWnKC) {
-    __syncthreads();                                      // the previous chunk has been consumed
-#pragma unroll
-    for (int v = 0; v < kMaxV; ++v) {
-      const int i = threadIdx.x + v * 256;
-      if (i < vec_per_chunk) *reinterpret_cast<float4*>(w_s + (size_t)i * 4) = nxt[v];
-    }
-    __syncthreads();
-    if (k0 + kWnKC < K) fetch(k0 + kWnKC);
-    const int kn = min(kWnKC, K - k0);
-#pragma unroll
-    for (int it = 0; it < 2; ++it) {
-      const int item = threadIdx.x + it * 256;
-      if (item >= n_items) break;
-      const int col = item % ncols, tg = item / ncols;
-      const float* xs = in_s + (size_t)k0 * kWnTT + tg * 8;
-#pragma unroll 8
-      for (int k = 0; k < kn; ++k) {
-        const float wv = w_s[k * ncols + col];
-        const float4 a = *reinterpret_cast<const float4*>(xs + k * kWnTT);
-        const float4 c4 = *reinterpret_cast<const float4*>(xs + k * kWnTT + 4);
-        acc[it][0] = fmaf(wv, a.x, acc[it][0]); acc[it][1] = fmaf(wv, a.y, acc[it][1]);
-        acc[it][2] = fmaf(wv, a.z, acc[it][2]); acc[it][3] = fmaf(wv, a.w, acc[it][3]);
-        acc[it][4] = fmaf(wv, c4.x, acc[it][4]); acc[it][5] = fmaf(wv, c4.y, acc[it][5]);
-        acc[it][6] = fmaf(wv, c4.z, acc[it][6]); acc[it][7] = fmaf(wv, c4.w, acc[it][7]);
-      }
-    }
-  }
-}
-
-__global__ void __launch_bounds__(256) wavenet_block_f32_kernel(const svsk_wavenet_block_params p) {
+// kTrain: also writes the gate pre-activations y [B][G][T] (svsk_wavenet_block_train_f32, kept for the backward); the
+// arithmetic is the same, so both instantiations give the same x_out and skips.
+template <bool kTrain>
+__global__ void __launch_bounds__(256) wavenet_block_f32_kernel(const svsk_wavenet_block_params p, float* __restrict__ y_out) {
   extern __shared__ float smem[];
   const int K1 = p.ksize * p.R + p.Cc, Gh = p.G / 2, O2 = p.S + p.R;
   float* in_s = smem;                                        // [K1][kWnTT]
@@ -115,6 +64,12 @@ __global__ void __launch_bounds__(256) wavenet_block_f32_kernel(const svsk_waven
     }
   }
   __syncthreads();
+  if constexpr (kTrain) {
+    for (int i = threadIdx.x; i < p.G * kWnTT; i += 256) {
+      const int t = t0 + i % kWnTT;
+      if (t < p.T) y_out[((size_t)b * p.G + i / kWnTT) * p.T + t] = y_s[i];
+    }
+  }
   for (int i = threadIdx.x; i < Gh * kWnTT; i += 256) {
     const float a = y_s[i], g = y_s[Gh * kWnTT + i];
     z_s[i] = tanhf(a) * (1.f / (1.f + expf(-g)));
@@ -184,9 +139,8 @@ extern "C" int svsk_wavenet_pack_f32(const float* wconv, const float* wc, const 
   return check_launch("wavenet_pack_f32");
 }
 
-extern "C" int svsk_wavenet_block_f32(const svsk_wavenet_block_params* pp, void* stream) {
-  SVSK_REQUIRE(pp != nullptr, SVSK_E_ARG, "wavenet_block_f32: null params");
-  const svsk_wavenet_block_params& p = *pp;
+// Checks shared by the inference and training entries; 0 and the dynamic shared memory in *smem, or SVSK_E_ARG.
+static int wavenet_block_check(const svsk_wavenet_block_params& p, size_t* smem_out) {
   SVSK_REQUIRE(p.x && p.c && p.w1t && p.w2t && p.b2 && p.x_out && p.skips, SVSK_E_ARG, "wavenet_block_f32: null tensor");
   SVSK_REQUIRE(p.B > 0 && p.B <= 65535 && p.T > 0 && p.R > 0 && p.G > 0 && p.G % 2 == 0 && p.S > 0 && p.Cc > 0 && p.ksize >= 1 &&
                    p.dilation >= 1, SVSK_E_ARG, "wavenet_block_f32: bad sizes");
@@ -196,13 +150,34 @@ extern "C" int svsk_wavenet_block_f32(const svsk_wavenet_block_params* pp, void*
   const int wcols = p.G > p.S + p.R ? p.G : p.S + p.R;
   const size_t smem = (((size_t)(p.ksize * p.R + p.Cc) + p.G + p.G / 2) * kWnTT + (size_t)kWnKC * wcols) * sizeof(float);
   SVSK_REQUIRE(smem <= 200 * 1024, SVSK_E_ARG, "wavenet_block_f32: %zu bytes of shared memory (k R + cin + 1.5 G too large)", smem);
+  *smem_out = smem;
+  return 0;
+}
+
+template <bool kTrain>
+static int wavenet_block_launch(const svsk_wavenet_block_params& p, float* y, size_t smem, void* stream, const char* what) {
   static size_t smem_set = 0;
   if (smem > 48 * 1024 && smem > smem_set) {
-    cudaError_t e = cudaFuncSetAttribute(wavenet_block_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return fail((int)e, "wavenet_block_f32: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    cudaError_t e = cudaFuncSetAttribute(wavenet_block_f32_kernel<kTrain>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return fail((int)e, "%s: cudaFuncSetAttribute: %s", what, cudaGetErrorString(e));
     smem_set = smem;
   }
   dim3 grid((unsigned)ceil_div(p.T, kWnTT), (unsigned)p.B);
-  wavenet_block_f32_kernel<<<grid, 256, smem, as_stream(stream)>>>(p);
-  return check_launch("wavenet_block_f32");
+  wavenet_block_f32_kernel<kTrain><<<grid, 256, smem, as_stream(stream)>>>(p, y);
+  return check_launch(what);
+}
+
+extern "C" int svsk_wavenet_block_f32(const svsk_wavenet_block_params* pp, void* stream) {
+  SVSK_REQUIRE(pp != nullptr, SVSK_E_ARG, "wavenet_block_f32: null params");
+  size_t smem = 0;
+  if (int rc = wavenet_block_check(*pp, &smem)) return rc;
+  return wavenet_block_launch<false>(*pp, nullptr, smem, stream, "wavenet_block_f32");
+}
+
+extern "C" int svsk_wavenet_block_train_f32(const svsk_wavenet_block_train_params* pp, void* stream) {
+  SVSK_REQUIRE(pp != nullptr, SVSK_E_ARG, "wavenet_block_train_f32: null params");
+  SVSK_REQUIRE(pp->y != nullptr, SVSK_E_ARG, "wavenet_block_train_f32: null tensor y");
+  size_t smem = 0;
+  if (int rc = wavenet_block_check(pp->blk, &smem)) return rc;
+  return wavenet_block_launch<true>(pp->blk, pp->y, smem, stream, "wavenet_block_train_f32");
 }

@@ -6,6 +6,7 @@ allocator (or taken from ``out=``) so whole loops are CUDA-graph capturable.
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import math
 import os
 from typing import Optional, Sequence
@@ -302,6 +303,203 @@ def wavenet_ar_f32(wpack, cproj, u, *, out_dim, R, G, S, layers, stacks, ksize, 
     p.layers, p.stacks, p.ksize = layers, stacks, ksize
     L.check(L.lib().svsk_wavenet_ar_f32(C.byref(p), L.stream_ptr()), "wavenet_ar_f32")
     return y
+
+
+def _shape(name, t, shape):
+    if t is None or tuple(t.shape) != tuple(shape):
+        raise ValueError(f"{name} must be {list(shape)}, got {None if t is None else list(t.shape)}")
+
+
+def wavenet_block_train_f32(x, c, w1t, b1, w2t, b2, skips, y, *, ksize, dilation, first, out=None):
+    """svsk_wavenet_block_train_f32: wavenet_block_f32 that also writes the gate pre-activations y [B, G, T]."""
+    B, R, T = x.shape
+    G = w1t.shape[1]
+    _shape("wavenet_block_train_f32: y", y, (B, G, T))
+    out = torch.empty_like(x) if out is None else out
+    p = L.WavenetBlockTrainParams()
+    q = p.blk
+    q.x, q.c, q.w1t, q.b1 = L.ptr(x, f32, "x"), L.ptr(c, f32, "c"), L.ptr(w1t, f32, "w1t"), L.ptr(b1, f32, "b1")
+    q.w2t, q.b2, q.x_out, q.skips = L.ptr(w2t, f32, "w2t"), L.ptr(b2, f32, "b2"), L.ptr(out, f32, "x_out"), L.ptr(skips, f32, "skips")
+    q.B, q.T, q.R, q.G, q.S, q.Cc = B, T, R, G, skips.shape[1], c.shape[1]
+    q.ksize, q.dilation, q.first = int(ksize), int(dilation), int(first)
+    p.y = L.ptr(y, f32, "y")
+    L.check(L.lib().svsk_wavenet_block_train_f32(C.byref(p), L.stream_ptr()), "wavenet_block_train_f32")
+    return out
+
+
+@functools.lru_cache(maxsize=64)
+def wavenet_train_sizes(out_dim, R, G, S, cin, layers, ksize):
+    """(floats of the training weight pack, floats of the gradient arena); raises for shapes the block rejects."""
+    pack, grad = C.c_longlong(), C.c_longlong()
+    rc = L.lib().svsk_wavenet_train_sizes(out_dim, R, G, S, cin, layers, ksize, C.byref(pack), C.byref(grad))
+    if rc != 0:
+        raise RuntimeError(f"libsvsk wavenet_train_sizes failed (code {rc}): {L.lib().svsk_last_error().decode()}")
+    return pack.value, grad.value
+
+
+@functools.lru_cache(maxsize=64)
+def wavenet_train_layout(out_dim, R, G, S, cin, layers, ksize):
+    """{name: (offset, shape)} of the weight pack and of the gradient arena (include/svsk.h, svsk_wavenet_train_pack_f32
+    and svsk_wavenet_wgrad_f32), checked against wavenet_train_sizes."""
+    Ly, k, G2 = layers, ksize, G // 2
+    Rp, G2p = (R + 3) // 4 * 4, (G2 + 3) // 4 * 4
+
+    def lay(items):
+        out, o = {}, 0
+        for name, shape in items:
+            out[name] = (o, shape)
+            o += math.prod(shape)
+        return out, o
+
+    pack, npk = lay([("w1t", (Ly, k * R + cin, G)), ("w2t", (Ly, G2, S + R)), ("wT", (Ly, k * G, Rp)), ("wB", (Ly, R + S, G2p)),
+                     ("wcT", (cin, Ly * G, 1)), ("first", (R, out_dim, 1)), ("firstT", (out_dim, R, 1)), ("last1", (S, S, 1)),
+                     ("last1T", (S, S, 1)), ("last3", (out_dim, S, 1)), ("last3T", (S, out_dim, 1))])
+    grad, ngr = lay([("conv", (Ly, G, R, k)), ("conv_b", (Ly, G)), ("cond", (Ly, G, cin, 1)), ("skip", (Ly, S, G2, 1)),
+                     ("skip_b", (Ly, S)), ("out", (Ly, R, G2, 1)), ("out_b", (Ly, R)), ("first", (R, out_dim, 1)),
+                     ("first_b", (R,)), ("last1", (S, S, 1)), ("last1_b", (S,)), ("last3", (out_dim, S, 1)), ("last3_b", (out_dim,))])
+    if (npk, ngr) != wavenet_train_sizes(out_dim, R, G, S, cin, layers, ksize):
+        raise RuntimeError("wavenet_train_layout: layout disagrees with libsvsk")
+    return pack, grad
+
+
+# the weights in the order of svsk_wavenet_wnorm_grad_f32's dg vector
+_WN_NAMES = ("first", "conv", "cond", "skip", "out", "last1", "last3")
+
+
+def _ar_weights_struct(w, out_dim, R, G, S, cin, layers, ksize):
+    p = L.WavenetArWeights()
+    for n in _AR_WEIGHTS:
+        setattr(p, n, L.ptr(w.get(n), f32, n).value)
+    p.out_dim, p.R, p.G, p.S, p.cin, p.layers, p.stacks, p.ksize = out_dim, R, G, S, cin, layers, 1, ksize
+    return p
+
+
+def _check_train_weights(w, out_dim, R, G, S, cin, layers, ksize):
+    G2 = G // 2
+    shapes = {"first": (R, out_dim, 1), "conv": (layers, G, R, ksize), "cond": (layers, G, cin, 1), "skip": (layers, S, G2, 1),
+              "out": (layers, R, G2, 1), "last1": (S, S, 1), "last3": (out_dim, S, 1)}
+    for n, shp in shapes.items():
+        _shape(f"wavenet weights: {n}_v", w.get(n + "_v"), shp)
+        if w.get(n + "_g") is not None and w[n + "_g"].numel() != math.prod(shp[:-2]):
+            raise ValueError(f"wavenet weights: {n}_g must hold {math.prod(shp[:-2])} gains, got {list(w[n + '_g'].shape)}")
+
+
+def wavenet_train_pack_f32(w, *, out_dim, R, G, S, cin, layers, ksize):
+    """svsk_wavenet_train_pack_f32.  w: the *_v / *_g tensors of svsk_wavenet_ar_weights (fp32, contiguous, stacked over
+    the layers; *_g None = no weight norm) -> {name: view} of one pack tensor (wavenet_train_layout)."""
+    _check_train_weights(w, out_dim, R, G, S, cin, layers, ksize)
+    lay, _ = wavenet_train_layout(out_dim, R, G, S, cin, layers, ksize)
+    n = sum(math.prod(s) for _, s in lay.values())
+    pack = torch.empty(n, device=w["conv_v"].device, dtype=f32)
+    p = _ar_weights_struct(w, out_dim, R, G, S, cin, layers, ksize)
+    L.check(L.lib().svsk_wavenet_train_pack_f32(C.byref(p), L.ptr(pack), L.stream_ptr()), "wavenet_train_pack_f32")
+    return {k: pack[o:o + math.prod(s)].view(s) for k, (o, s) in lay.items()}
+
+
+def wavenet_wnorm_grad_f32(w, dW, *, out_dim, R, G, S, cin, layers, ksize):
+    """svsk_wavenet_wnorm_grad_f32: turns the effective weights' gradients in dW (the arena of wavenet_wgrad_f32) into
+    those of the weight_v tensors, in place, and returns {name: gradient of the gain, shaped like the stacked weight_g}
+    for the weights that have a gain."""
+    _check_train_weights(w, out_dim, R, G, S, cin, layers, ksize)
+    _, ngr = wavenet_train_sizes(out_dim, R, G, S, cin, layers, ksize)
+    _shape("wavenet_wnorm_grad_f32: dW", dW, (ngr,))
+    rows = {"first": R, "conv": layers * G, "cond": layers * G, "skip": layers * S, "out": layers * R, "last1": S, "last3": out_dim}
+    dg = torch.empty(sum(rows.values()), device=dW.device, dtype=f32)
+    p = _ar_weights_struct(w, out_dim, R, G, S, cin, layers, ksize)
+    L.check(L.lib().svsk_wavenet_wnorm_grad_f32(C.byref(p), L.ptr(dW, f32, "dW"), L.ptr(dg), L.stream_ptr()),
+            "wavenet_wnorm_grad_f32")
+    out, o = {}, 0
+    for n in _WN_NAMES:
+        if w.get(n + "_g") is not None:
+            out[n] = dg[o:o + rows[n]].view(w[n + "_g"].shape)
+        o += rows[n]
+    return out
+
+
+def wavenet_dgrad_f32(*, dy_in, wT, g_next, g_out, dS, y_prev, wB, dy_out, ksize, dilation):
+    """svsk_wavenet_dgrad_f32 (one launch of the backward through the blocks).  dy_in / dy_out: [B, G, T] slices of a
+    [B, L, G, T] buffer (or None); g_next (or None), g_out [B, R, T]; dS [B, S, T]; y_prev [B, G, T] or None."""
+    B, R, T = g_out.shape
+    S = dS.shape[1]
+    _shape("wavenet_dgrad_f32: dS", dS, (B, S, T))
+    if g_next is not None:
+        _shape("wavenet_dgrad_f32: g_next", g_next, (B, R, T))
+    G = (dy_in if dy_in is not None else y_prev).shape[1] if (dy_in is not None or y_prev is not None) else 0
+    bstride = None
+    for name, t in (("dy_in", dy_in), ("dy_out", dy_out)):
+        if t is not None:
+            if t.dim() != 3 or tuple(t.shape) != (B, G, T) or t.stride(2) != 1 or t.stride(1) != T:
+                raise ValueError(f"wavenet_dgrad_f32: {name} must be a [{B}, {G}, {T}] slice with rows of T frames")
+            if bstride is not None and t.stride(0) != bstride:
+                raise ValueError("wavenet_dgrad_f32: dy_in and dy_out must share the batch stride")
+            bstride = t.stride(0)
+    if y_prev is not None:
+        _shape("wavenet_dgrad_f32: y_prev", y_prev, (B, G, T))
+        if dy_out is None or wB is None:
+            raise ValueError("wavenet_dgrad_f32: y_prev needs wB and dy_out")
+        _shape("wavenet_dgrad_f32: wB", wB, (R + S, (G // 2 + 3) // 4 * 4))
+    if dy_in is not None:
+        _shape("wavenet_dgrad_f32: wT", wT, (ksize * G, (R + 3) // 4 * 4))
+    p = L.WavenetDgradParams()
+
+    def sl(t, name):
+        if t is None:
+            return C.c_void_p(0)
+        if not t.is_cuda or t.dtype != f32:
+            raise RuntimeError(f"{name} must be a CUDA fp32 tensor")
+        return C.c_void_p(t.data_ptr())
+
+    p.dy_in, p.dy_out = sl(dy_in, "dy_in"), sl(dy_out, "dy_out")
+    p.wT, p.wB = L.ptr(wT, f32, "wT"), L.ptr(wB, f32, "wB")
+    p.g_next, p.g_out, p.dS, p.y_prev = L.ptr(g_next, f32, "g_next"), L.ptr(g_out, f32, "g_out"), L.ptr(dS, f32, "dS"), L.ptr(y_prev, f32, "y_prev")
+    p.dy_bstride = bstride if bstride is not None else G * T
+    p.B, p.T, p.R, p.G, p.S, p.ksize, p.dilation = B, T, R, G, S, int(ksize), int(dilation)
+    L.check(L.lib().svsk_wavenet_dgrad_f32(C.byref(p), L.stream_ptr()), "wavenet_dgrad_f32")
+
+
+def wavenet_wgrad_splits(B, T, out_dim, R, G, S, cin, layers, ksize, target=2 * 148):
+    """Frame splits of svsk_wavenet_wgrad_f32: enough CTAs for about two waves on a B200, at least 8 chunks of 32 frames
+    per split."""
+    t = lambda M, N: -(-M // 64) * -(-N // 64)
+    tiles = layers * (t(G, ksize * R + cin + 1) + t(R, G // 2 + 1) + t(S, G // 2 + 1)) + t(out_dim, S + 1) + t(S, S + 1) + t(R, out_dim + 1)
+    chunks = B * -(-T // 32)
+    return max(1, min(-(-target // tiles), chunks // 8, 64))
+
+
+def wavenet_wgrad_f32(*, x_in, c, xs, ys, gs, dy, dS, skips, h1, dh1, glog, dilations, ksize, splits=1):
+    """svsk_wavenet_wgrad_f32 -> the gradient arena (wavenet_train_layout's second dict).  Shapes as in include/svsk.h;
+    dilations: int32 CUDA tensor [L]."""
+    B, out_dim, T = x_in.shape
+    cin = c.shape[1]
+    Ly, _, R, _ = xs.shape
+    G, S = ys.shape[2], dS.shape[1]
+    for name, t, shp in (("c", c, (B, cin, T)), ("xs", xs, (Ly, B, R, T)), ("ys", ys, (Ly, B, G, T)), ("gs", gs, (Ly + 1, B, R, T)),
+                         ("dy", dy, (B, Ly, G, T)), ("dS", dS, (B, S, T)), ("skips", skips, (B, S, T)), ("h1", h1, (B, S, T)),
+                         ("dh1", dh1, (B, S, T)), ("glog", glog, (B, out_dim, T)), ("dilations", dilations, (Ly,))):
+        _shape(f"wavenet_wgrad_f32: {name}", t, shp)
+    _, ngr = wavenet_train_sizes(out_dim, R, G, S, cin, Ly, ksize)
+    dev = x_in.device
+    dW = torch.empty(ngr, device=dev, dtype=f32)
+    ws = torch.empty(splits * ngr, device=dev, dtype=f32) if splits > 1 else None
+    p = L.WavenetWgradParams()
+    for name, t in (("x_in", x_in), ("c", c), ("xs", xs), ("ys", ys), ("gs", gs), ("dy", dy), ("dS", dS), ("skips", skips),
+                    ("h1", h1), ("dh1", dh1), ("glog", glog)):
+        setattr(p, name, L.ptr(t, f32, name).value)
+    p.dilations = L.ptr(dilations, torch.int32, "dilations").value
+    p.dW, p.ws = L.ptr(dW).value, L.ptr(ws).value
+    p.B, p.T, p.out_dim, p.R, p.G, p.S, p.cin, p.layers, p.ksize, p.splits = B, T, out_dim, R, G, S, cin, Ly, int(ksize), int(splits)
+    L.check(L.lib().svsk_wavenet_wgrad_f32(C.byref(p), L.stream_ptr()), "wavenet_wgrad_f32")
+    return dW
+
+
+def relu_mask_f32(x, m, out=None):
+    """svsk_relu_mask_f32: x where m > 0, else 0 (out may be x)."""
+    _shape("relu_mask_f32: m", m, x.shape)
+    out = torch.empty_like(x) if out is None else out
+    _shape("relu_mask_f32: out", out, x.shape)
+    L.check(L.lib().svsk_relu_mask_f32(L.ptr(x, f32, "x"), L.ptr(m, f32, "m"), L.ptr(out, f32, "out"), x.numel(), L.stream_ptr()),
+            "relu_mask_f32")
+    return out
 
 
 def usfgan_source(f0, *, hop, sample_rate, dense_factor=4, sine_amp=0.1, noise_amp=0.0, noise=None, sine_out=None,

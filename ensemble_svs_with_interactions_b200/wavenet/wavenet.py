@@ -45,11 +45,25 @@ class WaveNet(nn.Module):
         x = ops.conv1d_f32(skips, _wc(l1), l1.bias, in_relu=True)
         return ops.conv1d_f32(x, _wc(l3), l3.bias, in_relu=True)
 
-    @torch.no_grad()
     def forward(self, c, x, lengths=None):
         """c (B,T,in_dim) conditioning, x (B,T,out_dim) targets -> (B,T,out_dim)   (wavenet.py:60-87).
-        The network is launch-latency bound (138 MFLOP at the reference test's shape): the second call of a shape
-        captures the launches as one CUDA graph, later calls replay it."""
+
+        Differentiable only in training mode: when the module is in training mode, grad mode is on and c, x or a
+        parameter requires grad, the output has a grad_fn and ``backward()`` fills the gradients of the parameters
+        (weight_g / weight_v, or weight after remove_weight_norm_(), and the biases) and of c / x on libsvsk kernels
+        (wavenet/training.py).  Every other call, eval mode included even with grad mode on, runs the inference path
+        below and returns a tensor without grad_fn; that differs from a plain nn.Module, which records gradients in
+        eval mode too.  Both paths compute the same output bits."""
+        if self.training and torch.is_grad_enabled() and (
+                c.requires_grad or x.requires_grad or any(q.requires_grad for q in self.parameters())):
+            from .training import wavenet_forward_with_grad
+            return wavenet_forward_with_grad(self, c, x)
+        return self._forward_no_grad(c, x)
+
+    @torch.no_grad()
+    def _forward_no_grad(self, c, x):
+        """The inference path of forward.  The network is launch-latency bound (138 MFLOP at the reference test's
+        shape): the second call of a shape captures the launches as one CUDA graph, later calls replay it."""
         if not x.is_cuda:
             raise RuntimeError("WaveNet runs on CUDA (sm_100a) only: libsvsk has no CPU path")
         x = x.to(f32).transpose(1, 2).contiguous()

@@ -509,6 +509,7 @@ SVSK_API int svsk_wavenet_block_f32(const svsk_wavenet_block_params* p, void* st
 SVSK_API int svsk_wavenet_pack_f32(const float* wconv, const float* wc, const float* wskip, const float* wout, float* w1t,
                                    float* w2t, int R, int G, int S, int Cc, int ksize, void* stream);
 
+
 /* WaveNet autoregressive sampling, fp32 — replaces WaveNet.inference (nnsvs/wavenet/wavenet.py:89-149) for B tracks in
  * one launch.  Per track and step t < steps:
  *   x_0 = first_conv(onehot(y[t-1])) (the bias alone at t = 0); for each layer l (dilation 2^(l mod layers/stacks)):
@@ -553,6 +554,82 @@ typedef struct svsk_wavenet_ar_weights {
 /* Folds weight norm (w = g v / ||v|| per output row, as torch._weight_norm(v, g, 0)) and lays the weights out for
  * svsk_wavenet_ar_f32: wpack [pack_floats] and wcond [layers G][cin]. */
 SVSK_API int svsk_wavenet_ar_pack_f32(const svsk_wavenet_ar_weights* w, float* wpack, float* wcond, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * WaveNet training (WaveNet.forward under autograd, nnsvs/wavenet/wavenet.py:60-87), fp32 on the CUDA cores.
+ * L layers, residual R, gate G (G2 = G / 2), skip S, conditioning cin, out_dim classes, kernel k; Rp = R and G2p = G2
+ * rounded up to multiples of 4.  Shapes: exactly those svsk_wavenet_block_f32 accepts.
+ * ------------------------------------------------------------------------------------------------ */
+
+/* svsk_wavenet_block_f32 that also writes the gate pre-activations y [B][G][T] (y = conv + conv1x1c + b1, before the
+ * gate), which the backward needs.  x_out and skips are bit-identical to svsk_wavenet_block_f32's. */
+typedef struct svsk_wavenet_block_train_params {
+  svsk_wavenet_block_params blk;
+  float* y;
+} svsk_wavenet_block_train_params;
+SVSK_API int svsk_wavenet_block_train_f32(const svsk_wavenet_block_train_params* p, void* stream);
+
+/* Floats of the training weight pack (svsk_wavenet_train_pack_f32) and of the gradient arena (svsk_wavenet_wgrad_f32);
+ * SVSK_E_ARG for shapes svsk_wavenet_block_f32 rejects. */
+SVSK_API int svsk_wavenet_train_sizes(int out_dim, int R, int G, int S, int cin, int layers, int ksize, long long* pack_floats,
+                                      long long* grad_floats);
+/* Folds weight norm (w = g v / ||v|| per output row, the same arithmetic as torch._weight_norm(v, g, 0) on CUDA, so the
+ * forward matches the module's eval path bit for bit; g == NULL: w = v) of every weight of w (stacked as documented
+ * at svsk_wavenet_ar_weights; biases are not read) and writes, one launch, pack [pack_floats] =
+ *   w1t [L][k R + cin][G]  w2t [L][G2][S + R]      (svsk_wavenet_block_f32's layouts)
+ *   wT [L][k G][Rp]        wT[l][j G + co][ci] = conv_l[co][ci][j]             (transposed conv of the backward)
+ *   wB [L][R + S][G2p]     rows: conv1x1_out_l [R][G2] then conv1x1_skip_l [S][G2]
+ *   wcT [cin][L G]         wcT[cc][l G + co] = conv1x1c_l[co][cc]
+ *   first [R][out_dim], firstT [out_dim][R], last1 [S][S], last1T [S][S], last3 [out_dim][S], last3T [S][out_dim]
+ * Padding columns of wT and wB are zero. */
+SVSK_API int svsk_wavenet_train_pack_f32(const svsk_wavenet_ar_weights* w, float* pack, void* stream);
+
+/* One step of the backward through the residual blocks, from the last down: launch l (l = L .. 0) computes
+ *   g_l = g_{l+1} + sum_j conv_l[:, :, j]^T dy_l(t + (k-1-j) d_l)       (dL/dx_l; dy_in == NULL: l == L, g_l = 0)
+ * and, when y_prev != NULL (l >= 1), for block l-1
+ *   dz = conv1x1_out^T g_l + conv1x1_skip^T dS;  dy_{l-1} = [dz sig(b)(1 - tanh^2 a) | dz tanh(a) sig(b)(1 - sig(b))]
+ * with a, b the halves of y_prev.  Tensors fp32: dy_in, dy_out [B] x [G][T] with batch stride dy_bstride (the slices of a
+ * [B][L][G][T] buffer); g_next (NULL = 0), g_out [B][R][T]; dS [B][S][T] = dL/dskips (after the ReLU mask); y_prev
+ * [B][G][T]; wT = pack's wT[l], wB = pack's wB[l-1].  dilation is d_l. */
+typedef struct svsk_wavenet_dgrad_params {
+  const float* dy_in;
+  const float* wT;
+  const float* g_next;
+  float* g_out;
+  const float* dS;
+  const float* y_prev;
+  const float* wB;
+  float* dy_out;
+  long long dy_bstride;
+  int32_t B, T, R, G, S, ksize, dilation;
+} svsk_wavenet_dgrad_params;
+SVSK_API int svsk_wavenet_dgrad_f32(const svsk_wavenet_dgrad_params* p, void* stream);
+
+/* Gradients of every effective weight and bias, without atomics: each CTA reduces a 64 x 64 output tile over its share
+ * of the (b, t) frames in a fixed order; splits > 1 writes per-split partials to ws [splits][grad_floats] and a second
+ * launch sums them in split order, so results are bit-reproducible.  dW [grad_floats] receives, in this order:
+ *   conv [L][G][R][k], conv_b [L][G], cond [L][G][cin], skip [L][S][G2], skip_b [L][S], out [L][R][G2], out_b [L][R],
+ *   first [R][out_dim], first_b [R], last1 [S][S], last1_b [S], last3 [out_dim][S], last3_b [out_dim].
+ * Inputs (fp32): x_in [B][out_dim][T] (first_conv's input), c [B][cin][T], xs [L][B][R][T] (block inputs), ys
+ * [L][B][G][T], gs [L + 1][B][R][T] (dL/dx_l, g_L = 0), dy [B][L][G][T], dS, skips (the forward's skip sum), h1
+ * (last1's output before the ReLU), dh1 = dL/dh1 [B][S][T], glog = dL/dlogits [B][out_dim][T]; dilations: device int32
+ * [L]. */
+typedef struct svsk_wavenet_wgrad_params {
+  const float *x_in, *c, *xs, *ys, *gs, *dy, *dS, *skips, *h1, *dh1, *glog;
+  const int32_t* dilations;
+  float* dW;
+  float* ws;
+  int32_t B, T, out_dim, R, G, S, cin, layers, ksize, splits;
+} svsk_wavenet_wgrad_params;
+SVSK_API int svsk_wavenet_wgrad_f32(const svsk_wavenet_wgrad_params* p, void* stream);
+
+/* Weight-norm backward of the weights of w that have a gain (g != NULL), one launch: with n = ||v|| per row and dw the
+ * effective weight's gradient in dW (svsk_wavenet_wgrad_f32's layout), dg = <dw, v> / n and, in place, dw <- (g / n)
+ * (dw - dg v / n).  dg [first R][conv L G][cond L G][skip L S][out L R][last1 S][last3 out_dim]. */
+SVSK_API int svsk_wavenet_wnorm_grad_f32(const svsk_wavenet_ar_weights* w, float* dW, float* dg, void* stream);
+
+/* y[i] = m[i] > 0 ? x[i] : 0 (the ReLU derivative); y may alias x. */
+SVSK_API int svsk_relu_mask_f32(const float* x, const float* m, float* y, long long n, void* stream);
 
 /* Source signal and dilation factors of the uSFGAN front end from frame-level F0 (nnsvs/usfgan/utils/features.py:
  * SignalGenerator.sinusoid :145-164, dilated_factor :56-75; called per utterance by USFGANWrapper.inference,
