@@ -591,8 +591,11 @@ def wgrad_splits(B, tiles, budget=160):
 
 
 def ntc_to_nct_bf16(x, N=None, out=None, row0=0, shifts=(0,)):
-    """out[b, row0 + j * N + n, t] = x[b, t + shifts[j], n] (0 outside the track) for up to three shifts: x [B, T, ld] bf16
-    (first N columns), out [B, rows, Tp] bf16 (Tp = T rounded up to 8; a fresh `out` has exactly len(shifts) * N rows)."""
+    """out[b, row0 + j * N + n, t] = x[b, t + shifts[j], n] for every t < Tp, 0 where frame t + shifts[j] is outside
+    [0, T), for up to three shifts: x [B, T, ld] bf16 (first N columns), out [B, rows, Tp] bf16 (Tp = T rounded up to 8;
+    a fresh `out` has exactly len(shifts) * N rows).  The padding columns t in [T, Tp) follow the same rule, so they hold
+    x[t + shift] wherever that frame exists: they are not zero, and svsk_wgrad_bf16 never reads them.  The other rows of
+    `out` are left as they are."""
     B, T, ld = x.shape
     N = ld if N is None else N
     Tp = (T + 7) // 8 * 8
