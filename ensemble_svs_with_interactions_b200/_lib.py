@@ -207,7 +207,6 @@ _SIGNATURES = {
     "svsk_expand1_bf16": [_V, C.c_longlong, _V, _V, _V, C.c_int, C.c_int, C.c_int, _V],
     "svsk_diffnet_pack_block": [_V, _V, _V, _V, _V, _I, _I, _V],
     "svsk_wavenet_block_f32": [C.POINTER(WavenetBlockParams), _V],
-    "svsk_wavenet_pack_f32": [_V, _V, _V, _V, _V, _V, _I, _I, _I, _I, _I, _V],
     "svsk_wavenet_ar_f32": [C.POINTER(WavenetArParams), _V],
     "svsk_wavenet_ar_supported": [_I, _I, _I, _I, _I, _I, _I],
     "svsk_wavenet_ar_sizes": [_I, _I, _I, _I, _I, _I, _I, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)],

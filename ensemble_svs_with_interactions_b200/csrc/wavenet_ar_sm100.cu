@@ -15,57 +15,9 @@
 // frame 0 read as zeros, exactly what the zero-initialised ring buffer of conv.py:21-53 gives.
 #include <climits>
 
-#include "svsk_common.cuh"
+#include "wavenet_f32.cuh"
 
 namespace svsk {
-
-constexpr int kArThreads = 1024;
-constexpr int kArWarps = kArThreads / 32;
-constexpr int kArMaxLayers = 64;
-
-struct ArLayout {
-  long long first_w, first_b, layer0, layer_stride, w3, b3, w4, b4, total;
-  long long gw, gb, sw, sb;   // offsets inside one layer block
-  long long hist;             // floats of ring buffer per track
-  int smem;                   // bytes of dynamic shared memory
-};
-
-// Packed weights (floats): WfT [out][R] (first_conv, transposed: one class is one contiguous row), bf [R]; per layer
-// Wg [G][k R] (column j R + r = conv.weight[:, r, j]), bg [G], Wso [S + R][G/2] (rows: skip then out), bso [S + R];
-// then W3 [S][S], b3 [S], W4 [out][S], b4 [out].
-inline ArLayout ar_layout(int O, int R, int G, int S, int L, int stacks, int k) {
-  ArLayout a = {};
-  const long long Gh = G / 2, kR = (long long)k * R;
-  a.first_w = 0;
-  a.first_b = (long long)O * R;
-  a.layer0 = a.first_b + R;
-  a.gw = 0;
-  a.gb = G * kR;
-  a.sw = a.gb + G;
-  a.sb = a.sw + (S + R) * Gh;
-  a.layer_stride = a.sb + S + R;
-  a.w3 = a.layer0 + L * a.layer_stride;
-  a.b3 = a.w3 + (long long)S * S;
-  a.w4 = a.b3 + S;
-  a.b4 = a.w4 + (long long)O * S;
-  a.total = a.b4 + O;
-  const int per = L / stacks;
-  for (int l = 0; l < L; ++l) a.hist += ((long long)(k - 1) * (1LL << (l % per)) + 1) * R;
-  a.smem = (int)(((long long)L * kR + (long long)L * G + Gh + 2LL * S + 2LL * O) * sizeof(float) + 3LL * L * sizeof(int) +
-                 sizeof(int));
-  return a;
-}
-
-// The shapes the kernel's fixed register tiles cover (see the warp_rows instantiations below).
-inline bool ar_supported(int O, int R, int G, int S, int L, int stacks, int k) {
-  if (O < 1 || R < 1 || G < 2 || G % 2 || S < 1 || L < 1 || stacks < 1 || k < 1) return false;
-  if (L > kArMaxLayers || L % stacks || L / stacks > 16) return false;
-  // gate: k R <= 8 x 32 weights per lane, 2 pairs per warp; skip|out: K = G/2 <= 2 x 32, S + R <= 4 rows per warp;
-  // last1: S <= 2 x 32; last3: out_dim <= 8 rows per warp
-  if (k * R > 8 * 32 || G / 2 > 2 * 32 || S + R > 4 * kArWarps || S > 2 * 32 || O > 8 * kArWarps) return false;
-  const ArLayout a = ar_layout(O, R, G, S, L, stacks, k);
-  return a.smem <= 48 * 1024 && a.hist <= (1LL << 30) && a.total <= (1LL << 30);
-}
 
 __device__ __forceinline__ float warp_sum(float s) {
 #pragma unroll
@@ -277,32 +229,6 @@ __global__ void __launch_bounds__(kArThreads, 1) wavenet_ar_kernel(const svsk_wa
   }
 }
 
-// dst[layer * lstride + o * ostride + (j * inner + ci) * cstride] = v[layer][o][ci][j] * (g ? g[layer][o] / ||v[layer][o]|| : 1)
-// and bdst[layer * lstride + o] = bias[layer][o] (0 when bias is NULL; nothing when bdst is NULL).  One CTA per row o.
-__global__ void __launch_bounds__(128) wavenet_ar_fold_kernel(const float* __restrict__ v, const float* __restrict__ g,
-                                                              const float* __restrict__ bias, float* __restrict__ dst,
-                                                              float* __restrict__ bdst, int rows, int inner, int k,
-                                                              long long lstride, int ostride, int cstride) {
-  __shared__ float red[4];
-  const int row = blockIdx.x, layer = row / rows, o = row - layer * rows, n = inner * k;
-  const float* vr = v + (size_t)row * n;
-  float scale = 1.f;
-  if (g) {
-    float s = 0.f;
-    for (int i = threadIdx.x; i < n; i += 128) s = fmaf(vr[i], vr[i], s);
-    s = warp_sum(s);
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
-    __syncthreads();
-    scale = g[row] / sqrtf(red[0] + red[1] + red[2] + red[3]);
-  }
-  float* d = dst + layer * lstride + (size_t)o * ostride;
-  for (int i = threadIdx.x; i < n; i += 128) {
-    const int ci = i / k, j = i - ci * k;
-    d[(size_t)(j * inner + ci) * cstride] = vr[i] * scale;
-  }
-  if (bdst && threadIdx.x == 0) bdst[layer * lstride + o] = bias ? bias[row] : 0.f;
-}
-
 }  // namespace svsk
 
 using namespace svsk;
@@ -321,36 +247,6 @@ extern "C" int svsk_wavenet_ar_sizes(int out_dim, int R, int G, int S, int layer
   *pack_floats = a.total;
   *hist_floats = a.hist;
   return 0;
-}
-
-extern "C" int svsk_wavenet_ar_pack_f32(const svsk_wavenet_ar_weights* wp, float* wpack, float* wcond, void* stream) {
-  SVSK_REQUIRE(wp != nullptr && wpack && wcond, SVSK_E_ARG, "wavenet_ar_pack_f32: null argument");
-  const svsk_wavenet_ar_weights& w = *wp;
-  SVSK_REQUIRE(w.first_v && w.first_b && w.conv_v && w.cond_v && w.skip_v && w.skip_b && w.out_v && w.out_b && w.last1_v &&
-                   w.last1_b && w.last3_v && w.last3_b, SVSK_E_ARG, "wavenet_ar_pack_f32: null weight");
-  const int O = w.out_dim, R = w.R, G = w.G, Gh = w.G / 2, S = w.S, L = w.layers, k = w.ksize;
-  SVSK_REQUIRE(w.cin > 0 && ar_supported(O, R, G, S, L, w.stacks, k), SVSK_E_ARG,
-               "wavenet_ar_pack_f32: unsupported WaveNet (out %d, R %d, G %d, S %d, cin %d, layers %d, stacks %d, k %d)", O, R,
-               G, S, w.cin, L, w.stacks, k);
-  const ArLayout a = ar_layout(O, R, G, S, L, w.stacks, k);
-  cudaStream_t st = as_stream(stream);
-  const long long ls = a.layer_stride;
-  // first_conv [R][out][1] -> WfT [out][R]
-  wavenet_ar_fold_kernel<<<R, 128, 0, st>>>(w.first_v, w.first_g, w.first_b, wpack + a.first_w, wpack + a.first_b, R, O, 1, 0, 1, R);
-  // conv [L][G][R][k] -> Wg [G][k R], bg
-  wavenet_ar_fold_kernel<<<L * G, 128, 0, st>>>(w.conv_v, w.conv_g, w.conv_b, wpack + a.layer0 + a.gw, wpack + a.layer0 + a.gb,
-                                                G, R, k, ls, k * R, 1);
-  // conv1x1_skip [L][S][G/2], conv1x1_out [L][R][G/2] -> Wso rows 0 .. S-1 and S .. S+R-1
-  wavenet_ar_fold_kernel<<<L * S, 128, 0, st>>>(w.skip_v, w.skip_g, w.skip_b, wpack + a.layer0 + a.sw, wpack + a.layer0 + a.sb,
-                                                S, Gh, 1, ls, Gh, 1);
-  wavenet_ar_fold_kernel<<<L * R, 128, 0, st>>>(w.out_v, w.out_g, w.out_b, wpack + a.layer0 + a.sw + (long long)S * Gh,
-                                                wpack + a.layer0 + a.sb + S, R, Gh, 1, ls, Gh, 1);
-  // last_conv_layers.1 / .3
-  wavenet_ar_fold_kernel<<<S, 128, 0, st>>>(w.last1_v, w.last1_g, w.last1_b, wpack + a.w3, wpack + a.b3, S, S, 1, 0, S, 1);
-  wavenet_ar_fold_kernel<<<O, 128, 0, st>>>(w.last3_v, w.last3_g, w.last3_b, wpack + a.w4, wpack + a.b4, O, S, 1, 0, S, 1);
-  // conv1x1c [L][G][cin] -> wcond [L G][cin] (no bias)
-  wavenet_ar_fold_kernel<<<L * G, 128, 0, st>>>(w.cond_v, w.cond_g, nullptr, wcond, nullptr, L * G, w.cin, 1, 0, w.cin, 1);
-  return check_launch("wavenet_ar_pack_f32");
 }
 
 extern "C" int svsk_wavenet_ar_f32(const svsk_wavenet_ar_params* pp, void* stream) {

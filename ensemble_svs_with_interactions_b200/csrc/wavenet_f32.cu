@@ -107,37 +107,9 @@ __global__ void __launch_bounds__(256) wavenet_block_f32_kernel(const svsk_waven
   }
 }
 
-// w1t[(j * R + ci) * G + co] = conv.weight[co][ci][j];  w1t[(k R + cc) * G + co] = conv1x1c.weight[co][cc]
-// w2t[k * (S + R) + o] = o < S ? skip.weight[o][k] : out.weight[o - S][k]
-__global__ void wavenet_pack_kernel(const float* __restrict__ wconv, const float* __restrict__ wc, const float* __restrict__ wskip,
-                                    const float* __restrict__ wout, float* __restrict__ w1t, float* __restrict__ w2t, int R, int G,
-                                    int S, int Cc, int ksize) {
-  const int K1 = ksize * R + Cc, Gh = G / 2, O2 = S + R;
-  const int n1 = K1 * G, n2 = Gh * O2;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n1 + n2; i += gridDim.x * blockDim.x) {
-    if (i < n1) {
-      const int r = i / G, co = i % G;
-      if (r < ksize * R) { const int j = r / R, ci = r - j * R; w1t[i] = wconv[((size_t)co * R + ci) * ksize + j]; }
-      else w1t[i] = wc[(size_t)co * Cc + (r - ksize * R)];
-    } else {
-      const int q = i - n1, k = q / O2, o = q % O2;
-      w2t[q] = o < S ? wskip[(size_t)o * Gh + k] : wout[(size_t)(o - S) * Gh + k];
-    }
-  }
-}
-
 }  // namespace svsk
 
 using namespace svsk;
-
-extern "C" int svsk_wavenet_pack_f32(const float* wconv, const float* wc, const float* wskip, const float* wout, float* w1t,
-                                     float* w2t, int R, int G, int S, int Cc, int ksize, void* stream) {
-  SVSK_REQUIRE(wconv && wc && wskip && wout && w1t && w2t, SVSK_E_ARG, "wavenet_pack_f32: null");
-  SVSK_REQUIRE(R > 0 && G > 0 && G % 2 == 0 && S > 0 && Cc > 0 && ksize >= 1, SVSK_E_ARG, "wavenet_pack_f32: bad sizes");
-  const int n = (ksize * R + Cc) * G + (G / 2) * (S + R);
-  wavenet_pack_kernel<<<(n + 255) / 256, 256, 0, as_stream(stream)>>>(wconv, wc, wskip, wout, w1t, w2t, R, G, S, Cc, ksize);
-  return check_launch("wavenet_pack_f32");
-}
 
 // Checks shared by the inference and training entries; 0 and the dynamic shared memory in *smem, or SVSK_E_ARG.
 static int wavenet_block_check(const svsk_wavenet_block_params& p, size_t* smem_out) {

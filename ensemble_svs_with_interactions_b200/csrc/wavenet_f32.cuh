@@ -1,9 +1,58 @@
 // Frame tile and weight-streaming GEMM shared by the fused WaveNet block (wavenet_f32.cu) and its backward
-// (wavenet_train_sm100.cu).
+// (wavenet_train_sm100.cu); the sampler's weight layout, shared by the sampler (wavenet_ar_sm100.cu) and the weight-norm
+// fold that writes it (wavenet_train_sm100.cu).
 #pragma once
 #include "svsk_common.cuh"
 
 namespace svsk {
+
+constexpr int kArThreads = 1024;
+constexpr int kArWarps = kArThreads / 32;
+constexpr int kArMaxLayers = 64;
+
+struct ArLayout {
+  long long first_w, first_b, layer0, layer_stride, w3, b3, w4, b4, total;
+  long long gw, gb, sw, sb;   // offsets inside one layer block
+  long long hist;             // floats of ring buffer per track
+  int smem;                   // bytes of dynamic shared memory
+};
+
+// Packed weights (floats): WfT [out][R] (first_conv, transposed: one class is one contiguous row), bf [R]; per layer
+// Wg [G][k R] (column j R + r = conv.weight[:, r, j]), bg [G], Wso [S + R][G/2] (rows: skip then out), bso [S + R];
+// then W3 [S][S], b3 [S], W4 [out][S], b4 [out].
+inline ArLayout ar_layout(int O, int R, int G, int S, int L, int stacks, int k) {
+  ArLayout a = {};
+  const long long Gh = G / 2, kR = (long long)k * R;
+  a.first_w = 0;
+  a.first_b = (long long)O * R;
+  a.layer0 = a.first_b + R;
+  a.gw = 0;
+  a.gb = G * kR;
+  a.sw = a.gb + G;
+  a.sb = a.sw + (S + R) * Gh;
+  a.layer_stride = a.sb + S + R;
+  a.w3 = a.layer0 + L * a.layer_stride;
+  a.b3 = a.w3 + (long long)S * S;
+  a.w4 = a.b3 + S;
+  a.b4 = a.w4 + (long long)O * S;
+  a.total = a.b4 + O;
+  const int per = L / stacks;
+  for (int l = 0; l < L; ++l) a.hist += ((long long)(k - 1) * (1LL << (l % per)) + 1) * R;
+  a.smem = (int)(((long long)L * kR + (long long)L * G + Gh + 2LL * S + 2LL * O) * sizeof(float) + 3LL * L * sizeof(int) +
+                 sizeof(int));
+  return a;
+}
+
+// The shapes the sampler's fixed register tiles cover (see the warp_rows instantiations in wavenet_ar_sm100.cu).
+inline bool ar_supported(int O, int R, int G, int S, int L, int stacks, int k) {
+  if (O < 1 || R < 1 || G < 2 || G % 2 || S < 1 || L < 1 || stacks < 1 || k < 1) return false;
+  if (L > kArMaxLayers || L % stacks || L / stacks > 16) return false;
+  // gate: k R <= 8 x 32 weights per lane, 2 pairs per warp; skip|out: K = G/2 <= 2 x 32, S + R <= 4 rows per warp;
+  // last1: S <= 2 x 32; last3: out_dim <= 8 rows per warp
+  if (k * R > 8 * 32 || G / 2 > 2 * 32 || S + R > 4 * kArWarps || S > 2 * 32 || O > 8 * kArWarps) return false;
+  const ArLayout a = ar_layout(O, R, G, S, L, stacks, k);
+  return a.smem <= 48 * 1024 && a.hist <= (1LL << 30) && a.total <= (1LL << 30);
+}
 
 constexpr int kWnTT = 16;  // frames per CTA
 constexpr int kWnKC = 32;  // weight rows staged per chunk

@@ -7,6 +7,8 @@
 // plus svsk_conv1d_f32 for the transposed 1x1s of the head, of first_conv (dx) and of all conditioning convs at once (dc),
 // and svsk_relu_mask_f32 for the head's two ReLU derivatives.  Nothing uses atomics: every output element is written by
 // one thread, and every sum runs in a fixed order, so gradients are bit-reproducible.
+// The weight-norm fold here is the library's only one: the inference forward uses the same pack, and
+// svsk_wavenet_ar_pack_f32 runs it with the sampler's layout.
 #include "wavenet_f32.cuh"
 
 namespace svsk {
@@ -79,11 +81,17 @@ struct WnDst {
   float* base;            // NULL: unused; element (layer l, row ro, input channel ci, tap j) goes to
   long long ls, rs, cs, js;  // base[l ls + ro rs + ci cs + j js]
 };
+struct WnBias {
+  const float* src;       // NULL: zeros
+  float* dst;             // NULL: no copy; row r (layer l, row ro) writes dst[l ls + ro] = src[r]
+  long long ls;
+};
 struct WnGroup {
   const float* v;
   const float* g;         // NULL: no weight norm (w = v)
   int rows, rowsize, rpl, k;  // rows = layers * rpl; rowsize = cin * k (flat [ci][j] as in the conv weight)
   WnDst d[2];
+  WnBias b;               // the sampler's pack writes its biases in the same launch
   long long dw, dg;       // offsets in the gradient arena / the dg vector (svsk_wavenet_wnorm_grad_f32)
 };
 struct WnGroups {
@@ -145,6 +153,7 @@ __global__ void __launch_bounds__(kWnormBlock) wavenet_wnorm_fold_kernel(const W
     for (int d = 0; d < 2; ++d)
       if (q.d[d].base) q.d[d].base[l * q.d[d].ls + ro * q.d[d].rs + ci * q.d[d].cs + j * q.d[d].js] = w;
   }
+  if (q.b.dst && threadIdx.x == 0) q.b.dst[l * q.b.ls + ro] = q.b.src ? q.b.src[r] : 0.f;
 }
 
 __global__ void __launch_bounds__(kWnormBlock) wavenet_wnorm_grad_kernel(const WnGroups G, float* __restrict__ dW,
@@ -162,17 +171,21 @@ __global__ void __launch_bounds__(kWnormBlock) wavenet_wnorm_grad_kernel(const W
   for (int i = threadIdx.x; i < q.rowsize; i += kWnormBlock) dw[i] = scale * (dw[i] - dgr * (v[i] / nrm));
 }
 
+static void wn_add(WnGroups& G, const float* v, const float* g, long long rows, long long rowsize, long long rpl, long long k,
+                   WnDst d0, WnDst d1, WnBias b, long long dw, long long dg) {
+  WnGroup& q = G.g[G.n];
+  q.v = v; q.g = g; q.rows = (int)rows; q.rowsize = (int)rowsize; q.rpl = (int)rpl; q.k = (int)k;
+  q.d[0] = d0; q.d[1] = d1; q.b = b; q.dw = dw; q.dg = dg;
+  G.row0[G.n + 1] = G.row0[G.n] + (int)rows;
+  ++G.n;
+}
+
 // The seven weights of svsk_wavenet_ar_weights as fold / gradient groups.  pack == NULL: no destinations (gradient).
 static WnGroups wn_groups(const svsk_wavenet_ar_weights& w, const WnTrainDims& d, float* pack, bool only_normed) {
   WnGroups G{};
   auto add = [&](const float* v, const float* g, long long rows, long long rowsize, long long rpl, long long k, WnDst d0,
                  WnDst d1, long long dw, long long dg) {
-    if (only_normed && !g) return;
-    WnGroup& q = G.g[G.n];
-    q.v = v; q.g = g; q.rows = (int)rows; q.rowsize = (int)rowsize; q.rpl = (int)rpl; q.k = (int)k;
-    q.d[0] = d0; q.d[1] = d1; q.dw = dw; q.dg = dg;
-    G.row0[G.n + 1] = G.row0[G.n] + (int)rows;
-    ++G.n;
+    if (!only_normed || g) wn_add(G, v, g, rows, rowsize, rpl, k, d0, d1, {}, dw, dg);
   };
   auto P = [&](long long off) { return pack ? pack + off : nullptr; };
   const long long L = d.L, R = d.R, G_ = d.G, G2 = d.G2, S = d.S, k = d.k, out = d.out, cin = d.cin;
@@ -511,6 +524,37 @@ extern "C" int svsk_wavenet_train_pack_f32(const svsk_wavenet_ar_weights* w, flo
   const WnGroups G = wn_groups(*w, d, pack, false);
   wavenet_wnorm_fold_kernel<<<G.row0[G.n], kWnormBlock, 0, st>>>(G);
   return check_launch("wavenet_train_pack_f32");
+}
+
+// The sampler's pack (ArLayout, wavenet_f32.cuh): the same fold, so its weights are the forward's bits.
+extern "C" int svsk_wavenet_ar_pack_f32(const svsk_wavenet_ar_weights* wp, float* wpack, float* wcond, void* stream) {
+  SVSK_REQUIRE(wp != nullptr && wpack && wcond, SVSK_E_ARG, "wavenet_ar_pack_f32: null argument");
+  const svsk_wavenet_ar_weights& w = *wp;
+  SVSK_REQUIRE(w.first_v && w.first_b && w.conv_v && w.cond_v && w.skip_v && w.skip_b && w.out_v && w.out_b && w.last1_v &&
+                   w.last1_b && w.last3_v && w.last3_b, SVSK_E_ARG, "wavenet_ar_pack_f32: null weight");
+  const int O = w.out_dim, R = w.R, G = w.G, Gh = w.G / 2, S = w.S, L = w.layers, k = w.ksize, cin = w.cin;
+  SVSK_REQUIRE(cin > 0 && ar_supported(O, R, G, S, L, w.stacks, k), SVSK_E_ARG,
+               "wavenet_ar_pack_f32: unsupported WaveNet (out %d, R %d, G %d, S %d, cin %d, layers %d, stacks %d, k %d)", O, R,
+               G, S, cin, L, w.stacks, k);
+  const ArLayout a = ar_layout(O, R, G, S, L, w.stacks, k);
+  const long long ls = a.layer_stride;
+  float* lay = wpack + a.layer0;
+  WnGroups Q{};
+  // first_conv [R][out] -> WfT [out][R], bf
+  wn_add(Q, w.first_v, w.first_g, R, O, R, 1, {wpack + a.first_w, 0, 1, R, 0}, {}, {w.first_b, wpack + a.first_b, 0}, 0, 0);
+  // conv [L][G][R][k] -> Wg [G][k R] (column j R + r), bg
+  wn_add(Q, w.conv_v, w.conv_g, (long long)L * G, R * k, G, k, {lay + a.gw, ls, k * R, 1, R}, {}, {w.conv_b, lay + a.gb, ls}, 0, 0);
+  // conv1x1_skip [L][S][G/2], conv1x1_out [L][R][G/2] -> Wso rows 0 .. S-1 and S .. S+R-1, bso
+  wn_add(Q, w.skip_v, w.skip_g, (long long)L * S, Gh, S, 1, {lay + a.sw, ls, Gh, 1, 0}, {}, {w.skip_b, lay + a.sb, ls}, 0, 0);
+  wn_add(Q, w.out_v, w.out_g, (long long)L * R, Gh, R, 1, {lay + a.sw + (long long)S * Gh, ls, Gh, 1, 0}, {},
+         {w.out_b, lay + a.sb + S, ls}, 0, 0);
+  // last_conv_layers.1 / .3
+  wn_add(Q, w.last1_v, w.last1_g, S, S, S, 1, {wpack + a.w3, 0, S, 1, 0}, {}, {w.last1_b, wpack + a.b3, 0}, 0, 0);
+  wn_add(Q, w.last3_v, w.last3_g, O, S, O, 1, {wpack + a.w4, 0, S, 1, 0}, {}, {w.last3_b, wpack + a.b4, 0}, 0, 0);
+  // conv1x1c [L][G][cin] -> wcond [L G][cin] (no bias)
+  wn_add(Q, w.cond_v, w.cond_g, (long long)L * G, cin, G, 1, {wcond, (long long)G * cin, cin, 1, 0}, {}, {}, 0, 0);
+  wavenet_wnorm_fold_kernel<<<Q.row0[Q.n], kWnormBlock, 0, as_stream(stream)>>>(Q);
+  return check_launch("wavenet_ar_pack_f32");
 }
 
 extern "C" int svsk_wavenet_wnorm_grad_f32(const svsk_wavenet_ar_weights* w, float* dW, float* dg, void* stream) {

@@ -217,19 +217,6 @@ def diffnet_block_bf16(xb_in, xb_out, x32, skip32, cond, w1p, woutp, stepbias, b
     L.check(L.lib().svsk_diffnet_block3_bf16(C.byref(p), L.stream_ptr()), "diffnet_block_bf16")
 
 
-def wavenet_pack_f32(wconv, wc, wskip, wout):
-    """Effective (weight-norm folded) weights of one ResSkipBlock -> (w1t [k*R + Cc, G], w2t [G/2, S + R]) fp32."""
-    G, R, k = wconv.shape
-    Cc, S = wc.shape[1], wskip.shape[0]
-    dev = wconv.device
-    w1t = torch.empty((k * R + Cc, G), device=dev, dtype=f32)
-    w2t = torch.empty((G // 2, S + R), device=dev, dtype=f32)
-    L.check(L.lib().svsk_wavenet_pack_f32(L.ptr(wconv.contiguous(), f32), L.ptr(wc.contiguous(), f32), L.ptr(wskip.contiguous(), f32),
-                                          L.ptr(wout.contiguous(), f32), L.ptr(w1t), L.ptr(w2t), R, G, S, Cc, k, L.stream_ptr()),
-            "wavenet_pack_f32")
-    return w1t, w2t
-
-
 def wavenet_block_f32(x, c, w1t, b1, w2t, b2, skips, *, ksize, dilation, first, out=None):
     """One fused ResSkipBlock (svsk_wavenet_block_f32): x [B,R,T], c [B,Cc,T] -> new x; skips [B,S,T] set or accumulated."""
     B, R, T = x.shape

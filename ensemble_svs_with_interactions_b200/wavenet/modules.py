@@ -38,29 +38,21 @@ class ResSkipBlock(nn.Module):
         self.conv1x1_out = Conv1d1x1(gate_out_channels, residual_channels)
         self.conv1x1_skip = Conv1d1x1(gate_out_channels, skip_out_channels)
 
-    def _packed(self):
-        """Folded (weight norm) and transposed weights of the fused kernel, rebuilt when any parameter changes."""
-        key = tuple((q.data_ptr(), q._version) for q in self.parameters())
-        if getattr(self, "_pack_key", None) != key:
-            w1t, w2t = ops.wavenet_pack_f32(_w(self.conv).to(f32), _w(self.conv1x1c).to(f32)[:, :, 0],
-                                            _w(self.conv1x1_skip).to(f32)[:, :, 0], _w(self.conv1x1_out).to(f32)[:, :, 0])
-            b1 = None if self.conv.bias is None else self.conv.bias.detach().to(f32).contiguous()
-            b2 = torch.cat([self.conv1x1_skip.bias.detach(), self.conv1x1_out.bias.detach()]).to(f32).contiguous()
-            self._pack, self._pack_key = (w1t, b1, w2t, b2), key
-        return self._pack
-
-    def run(self, x, c, skips, first):
-        """x, c NCT fp32.  Returns the new x; accumulates the skip branch into ``skips``.  One launch
-        (svsk_wavenet_block_f32): "pad (k-1)d both sides then trim right" (modules.py:99-101) == taps at t-(k-1-j)d, zero
-        for t < 0; tanh on the first half of the gate channels, sigmoid on the second; x + res without a sqrt(1/2)."""
-        w1t, b1, w2t, b2 = self._packed()
-        return ops.wavenet_block_f32(x, c, w1t, b1, w2t, b2, skips, ksize=self.kernel_size, dilation=self.dilation, first=first)
-
     @torch.no_grad()
     def forward(self, x, c):
+        """x (B, R, T), c (B, cin, T) -> (x_out, skips) fp32, one launch (svsk_wavenet_block_f32): "pad (k-1)d both sides
+        then trim right" (modules.py:99-101) == taps at t-(k-1-j)d, zero for t < 0; tanh on the first half of the gate
+        channels, sigmoid on the second; x + res without a sqrt(1/2).  WaveNet runs its blocks from one pack of all layers
+        (wavenet/training.py); this lays out the same w1t / w2t for one block (include/svsk.h)."""
         x = x.to(f32).contiguous()
+        k, R = self.kernel_size, x.shape[1]
+        w1t = torch.cat([_w(self.conv).to(f32).permute(2, 1, 0).reshape(k * R, -1), _w(self.conv1x1c).to(f32)[:, :, 0].t()])
+        w2t = torch.cat([_w(self.conv1x1_skip)[:, :, 0], _w(self.conv1x1_out)[:, :, 0]]).to(f32).t().contiguous()
+        b1 = None if self.conv.bias is None else self.conv.bias.detach().to(f32).contiguous()
+        b2 = torch.cat([self.conv1x1_skip.bias.detach(), self.conv1x1_out.bias.detach()]).to(f32).contiguous()
         s = torch.empty((x.shape[0], self.conv1x1_skip.out_channels, x.shape[2]), device=x.device, dtype=f32)
-        return self.run(x, c.to(f32).contiguous(), s, True), s
+        x = ops.wavenet_block_f32(x, c.to(f32).contiguous(), w1t, b1, w2t, b2, s, ksize=k, dilation=self.dilation, first=True)
+        return x, s
 
     @torch.no_grad()
     def incremental_forward(self, x, c):

@@ -4,7 +4,7 @@
 The whole network is ONE ``torch.autograd.Function`` over the parameters stacked over the layers (a differentiable
 ``torch.stack``, so every ``nn.Parameter`` still receives its own ``.grad``):
 
-forward (the kernels of the eval path, so the output is the same bits)
+forward (_forward, which the inference path of WaveNet.forward runs too, so the output is the same bits)
     pack      = fold weight norm of every weight into the layouts below          svsk_wavenet_train_pack_f32, 1 launch
     x_0       = first_conv(x)                                                    svsk_conv1d_f32
     x_{l+1}, skips (+)=, y_l = block_l(x_l, c)                                   svsk_wavenet_block_train_f32, L launches
@@ -67,27 +67,40 @@ def _params(net):
 
 
 def _dims(net):
+    """(sizes as the ops wrappers take them, dilation of every block)."""
     blocks = net.main_conv_layers
     f0 = blocks[0]
-    return dict(out_dim=net.first_conv.in_channels, R=net.first_conv.out_channels, G=f0.conv.out_channels,
-                S=f0.conv1x1_skip.out_channels, cin=f0.conv1x1c.in_channels, layers=len(blocks), ksize=f0.kernel_size)
+    if len({f.kernel_size for f in blocks}) != 1:
+        raise RuntimeError("WaveNet on libsvsk: all blocks must share one kernel size")
+    return (dict(out_dim=net.first_conv.in_channels, R=net.first_conv.out_channels, G=f0.conv.out_channels,
+                 S=f0.conv1x1_skip.out_channels, cin=f0.conv1x1c.in_channels, layers=len(blocks), ksize=f0.kernel_size),
+            tuple(int(f.dilation) for f in blocks))
 
 
-def _forward(dims, dilations, c, x, w):
-    """Forward kernels: logits [B, out_dim, T] and what the backward keeps."""
-    L, k = dims["layers"], dims["ksize"]
+def _pack(dims, w):
+    """The weight pack of the forward (wavenet_train_layout's views) plus "b2", the blocks' [skip | out] biases."""
     pk = ops.wavenet_train_pack_f32({n: w[n] for n in w if not n.endswith("_b")}, **dims)
+    return dict(pk, b2=torch.cat([w["skip_b"], w["out_b"]], dim=1))
+
+
+def _forward(dims, dilations, pk, w, c, x, train):
+    """Forward kernels after the pack: logits [B, out_dim, T] and what the backward keeps.  train: the blocks also store
+    their gate pre-activations ys (svsk_wavenet_block_train_f32), else ys is None."""
+    L, k = dims["layers"], dims["ksize"]
     B, _, T = x.shape
     R, G, S = dims["R"], dims["G"], dims["S"]
     xs = torch.empty((L + 1, B, R, T), device=x.device, dtype=f32)
     ops.conv1d_f32(x, pk["first"], w["first_b"], out=xs[0])
     skips = torch.empty((B, S, T), device=x.device, dtype=f32)
-    ys = torch.empty((L, B, G, T), device=x.device, dtype=f32)
-    b2 = torch.cat([w["skip_b"], w["out_b"]], dim=1)
+    ys = torch.empty((L, B, G, T), device=x.device, dtype=f32) if train else None
     for l in range(L):
         b1 = None if w["conv_b"] is None else w["conv_b"][l]
-        ops.wavenet_block_train_f32(xs[l], c, pk["w1t"][l], b1, pk["w2t"][l], b2[l], skips, ys[l], ksize=k,
-                                    dilation=dilations[l], first=(l == 0), out=xs[l + 1])
+        blk = (xs[l], c, pk["w1t"][l], b1, pk["w2t"][l], pk["b2"][l], skips)
+        kw = dict(ksize=k, dilation=dilations[l], first=(l == 0), out=xs[l + 1])
+        if train:
+            ops.wavenet_block_train_f32(*blk, ys[l], **kw)
+        else:
+            ops.wavenet_block_f32(*blk, **kw)
     h1 = ops.conv1d_f32(skips, pk["last1"], w["last1_b"], in_relu=True)
     logits = ops.conv1d_f32(h1, pk["last3"], w["last3_b"], in_relu=True)
     return logits, (pk, xs, ys, skips, h1)
@@ -142,7 +155,7 @@ class _WaveNetFn(torch.autograd.Function):
         w = dict(zip(keys, params))
         ct = c.to(f32).transpose(1, 2).contiguous()
         xt = x.to(f32).transpose(1, 2).contiguous()
-        logits, saved = _forward(dims, dilations, ct, xt, w)
+        logits, saved = _forward(dims, dilations, _pack(dims, w), w, ct, xt, train=True)
         ctx.dims, ctx.dilations, ctx.keys = dims, dilations, keys
         ctx.c_dtype, ctx.x_dtype = c.dtype, x.dtype
         ctx.saved = saved               # kernel outputs only (not inputs / parameters): no version tracking needed
@@ -168,11 +181,7 @@ def wavenet_forward_with_grad(net, c, x):
     path's."""
     if not x.is_cuda or not c.is_cuda:
         raise RuntimeError(_CPU_ERROR)
-    dims = _dims(net)
-    blocks = net.main_conv_layers
-    if len({f.kernel_size for f in blocks}) != 1:
-        raise RuntimeError("WaveNet training path: all blocks must share one kernel size")
-    dilations = tuple(int(f.dilation) for f in blocks)
+    dims, dilations = _dims(net)
     items = _params(net)
     keys = tuple(k_ for k_, _ in items)
     return _WaveNetFn.apply(dims, dilations, keys, c, x, *[t for _, t in items])

@@ -5,17 +5,15 @@ from torch.nn import functional as F
 
 from .. import _lib as _L
 from .. import ops
-from .modules import Conv1d1x1, ResSkipBlock, _w
+from .modules import Conv1d1x1, ResSkipBlock
+from .training import _dims, _forward, _pack, _params, wavenet_forward_with_grad
 
 f32 = torch.float32
 
 
-def _wc(m):
-    """Effective (weight-norm folded) weight of a conv holder, cached until one of its parameters changes."""
-    key = tuple((q.data_ptr(), q._version) for q in m.parameters())
-    if getattr(m, "_w_key", None) != key:
-        m._w_cache, m._w_key = _w(m).to(f32).contiguous(), key
-    return m._w_cache
+def _weights(net):
+    """training._params, detached: the parameters stacked over the layers, as the inference packs read them."""
+    return {k: None if t is None else t.detach() for k, t in _params(net)}
 
 
 class WaveNet(nn.Module):
@@ -34,16 +32,15 @@ class WaveNet(nn.Module):
                                                Conv1d1x1(skip_out_channels, out_dim)])
         self.use_cuda_graph = True
 
-    def _forward_kernels(self, c, x):
-        """c (B,in_dim,T), x (B,out_dim,T) fp32 contiguous -> logits (B,out_dim,T): 3 + layers launches."""
-        x = ops.conv1d_f32(x, _wc(self.first_conv), self.first_conv.bias)
-        skip_ch = self.last_conv_layers[1].in_channels
-        skips = torch.empty((x.shape[0], skip_ch, x.shape[2]), device=x.device, dtype=f32)
-        for i, f in enumerate(self.main_conv_layers):
-            x = f.run(x, c, skips, i == 0)
-        l1, l3 = self.last_conv_layers[1], self.last_conv_layers[3]
-        x = ops.conv1d_f32(skips, _wc(l1), l1.bias, in_relu=True)
-        return ops.conv1d_f32(x, _wc(l3), l3.bias, in_relu=True)
+    def _packed(self):
+        """(sizes, dilations, weight pack, stacked parameters) of the inference forward, rebuilt when any parameter
+        changes: the leading arguments of training._forward."""
+        key = tuple((q.data_ptr(), q._version) for q in self.parameters())
+        if self.__dict__.get("_pack_key") != key:
+            (dims, dilations), w = _dims(self), _weights(self)
+            self.__dict__["_pack"] = (dims, dilations, _pack(dims, w), w)
+            self.__dict__["_pack_key"] = key
+        return self.__dict__["_pack"]
 
     def forward(self, c, x, lengths=None):
         """c (B,T,in_dim) conditioning, x (B,T,out_dim) targets -> (B,T,out_dim)   (wavenet.py:60-87).
@@ -56,14 +53,14 @@ class WaveNet(nn.Module):
         eval mode too.  Both paths compute the same output bits."""
         if self.training and torch.is_grad_enabled() and (
                 c.requires_grad or x.requires_grad or any(q.requires_grad for q in self.parameters())):
-            from .training import wavenet_forward_with_grad
             return wavenet_forward_with_grad(self, c, x)
         return self._forward_no_grad(c, x)
 
     @torch.no_grad()
     def _forward_no_grad(self, c, x):
         """The inference path of forward.  The network is launch-latency bound (138 MFLOP at the reference test's
-        shape): the second call of a shape captures the launches as one CUDA graph, later calls replay it."""
+        shape): the second call of a shape captures the launches as one CUDA graph, later calls replay it.  The kernels
+        are training._forward's (svsk_wavenet_block_f32 for the blocks) on a pack built once per parameter version."""
         if not x.is_cuda:
             raise RuntimeError("WaveNet runs on CUDA (sm_100a) only: libsvsk has no CPU path")
         x = x.to(f32).transpose(1, 2).contiguous()
@@ -83,17 +80,17 @@ class WaveNet(nn.Module):
                 s_c, s_x = c.clone(), x.clone()
                 side = torch.cuda.Stream()
                 side.wait_stream(torch.cuda.current_stream())
-                with torch.cuda.stream(side):           # warm-up outside capture: weight caches, allocator pools
-                    self._forward_kernels(s_c, s_x)
+                with torch.cuda.stream(side):           # warm-up outside capture: the weight pack, allocator pools
+                    _forward(*self._packed(), s_c, s_x, train=False)
                 torch.cuda.current_stream().wait_stream(side)
                 g = torch.cuda.CUDAGraph()
                 n0 = _L.launch_count
                 with torch.cuda.graph(g):
-                    out = self._forward_kernels(s_c, s_x)
+                    out = _forward(*self._packed(), s_c, s_x, train=False)[0]
                 ent = self._graphs[key] = (g, s_c, s_x, out, _L.launch_count - n0)
                 _L.launch_count = n0
         if ent is None:
-            return self._forward_kernels(c, x).transpose(1, 2)
+            return _forward(*self._packed(), c, x, train=False)[0].transpose(1, 2)
         g, s_c, s_x, out, n = ent
         s_c.copy_(c); s_x.copy_(x)
         g.replay()
@@ -116,29 +113,10 @@ class WaveNet(nn.Module):
         """Folded, laid-out weights of the device sampler, rebuilt when any parameter changes."""
         key = (cfg,) + tuple((q.data_ptr(), q._version) for q in self.parameters())
         if self.__dict__.get("_ar_key") != key:
-            def vg(mods):
-                if all(hasattr(m, "weight_g") for m in mods):
-                    return (torch.stack([m.weight_v.detach() for m in mods]).to(f32).contiguous(),
-                            torch.stack([m.weight_g.detach().reshape(-1) for m in mods]).to(f32).contiguous())
-                return torch.stack([_w(m) for m in mods]).to(f32).contiguous(), None
-
-            def bias(mods):
-                if any(m.bias is None for m in mods):
-                    return None
-                return torch.stack([m.bias.detach() for m in mods]).to(f32).contiguous()
-
-            blocks = self.main_conv_layers
-            w = {}
-            for name, mods in (("first", [self.first_conv]), ("conv", [f.conv for f in blocks]),
-                               ("cond", [f.conv1x1c for f in blocks]), ("skip", [f.conv1x1_skip for f in blocks]),
-                               ("out", [f.conv1x1_out for f in blocks]), ("last1", [self.last_conv_layers[1]]),
-                               ("last3", [self.last_conv_layers[3]])):
-                w[name + "_v"], w[name + "_g"] = vg(mods)
-                if name != "cond":
-                    w[name + "_b"] = bias(mods)
             out_dim, R, G, S, layers, stacks, k = cfg
             self.__dict__["_ar_pack"] = ops.wavenet_ar_pack_f32(
-                w, out_dim=out_dim, R=R, G=G, S=S, cin=blocks[0].conv1x1c.in_channels, layers=layers, stacks=stacks, ksize=k)
+                _weights(self), out_dim=out_dim, R=R, G=G, S=S, cin=self.main_conv_layers[0].conv1x1c.in_channels,
+                layers=layers, stacks=stacks, ksize=k)
             self.__dict__["_ar_key"] = key
         return self.__dict__["_ar_pack"]
 

@@ -492,8 +492,8 @@ SVSK_API int svsk_mdn_head_f32(const float* raw, float* log_pi, float* log_sigma
  *   y = causal_conv(x; ksize, dilation) + conv1x1c(c) + b1;  z = tanh(y[:G/2]) * sigmoid(y[G/2:])
  *   skips = (first ? 0 : skips) + conv1x1_skip(z) + b2[:S];  x_out = conv1x1_out(z) + b2[S:] + x
  * x, x_out [B][R][T], c [B][Cc][T], skips [B][S][T] fp32; x_out must not alias x.  w1t [ksize*R + Cc][G] and
- * w2t [G/2][S + R] come from svsk_wavenet_pack_f32 (effective, weight-norm-folded weights: conv [G][R][ksize],
- * conv1x1c [G][Cc], conv1x1_skip [S][G/2], conv1x1_out [R][G/2]); b1 [G] (may be NULL), b2 [S + R] = [skip | out]. */
+ * w2t [G/2][S + R] are the layer's slices w1t[l] and w2t[l] of svsk_wavenet_train_pack_f32's pack (effective,
+ * weight-norm-folded weights); b1 [G] (may be NULL), b2 [S + R] = [skip | out]. */
 typedef struct svsk_wavenet_block_params {
   const float* x;
   const float* c;
@@ -506,8 +506,6 @@ typedef struct svsk_wavenet_block_params {
   int32_t B, T, R, G, S, Cc, ksize, dilation, first;
 } svsk_wavenet_block_params;
 SVSK_API int svsk_wavenet_block_f32(const svsk_wavenet_block_params* p, void* stream);
-SVSK_API int svsk_wavenet_pack_f32(const float* wconv, const float* wc, const float* wskip, const float* wout, float* w1t,
-                                   float* w2t, int R, int G, int S, int Cc, int ksize, void* stream);
 
 
 /* WaveNet autoregressive sampling, fp32 — replaces WaveNet.inference (nnsvs/wavenet/wavenet.py:89-149) for B tracks in
@@ -551,8 +549,8 @@ typedef struct svsk_wavenet_ar_weights {
   const float *last3_v, *last3_g, *last3_b;
   int32_t out_dim, R, G, S, cin, layers, stacks, ksize;
 } svsk_wavenet_ar_weights;
-/* Folds weight norm (w = g v / ||v|| per output row, as torch._weight_norm(v, g, 0)) and lays the weights out for
- * svsk_wavenet_ar_f32: wpack [pack_floats] and wcond [layers G][cin]. */
+/* Folds weight norm with the fold of svsk_wavenet_train_pack_f32 (the same bits) and lays the weights out for
+ * svsk_wavenet_ar_f32, one launch: wpack [pack_floats] and wcond [layers G][cin]. */
 SVSK_API int svsk_wavenet_ar_pack_f32(const svsk_wavenet_ar_weights* w, float* wpack, float* wcond, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
@@ -576,7 +574,9 @@ SVSK_API int svsk_wavenet_train_sizes(int out_dim, int R, int G, int S, int cin,
 /* Folds weight norm (w = g v / ||v|| per output row, the same arithmetic as torch._weight_norm(v, g, 0) on CUDA, so the
  * forward matches the module's eval path bit for bit; g == NULL: w = v) of every weight of w (stacked as documented
  * at svsk_wavenet_ar_weights; biases are not read) and writes, one launch, pack [pack_floats] =
- *   w1t [L][k R + cin][G]  w2t [L][G2][S + R]      (svsk_wavenet_block_f32's layouts)
+ *   w1t [L][k R + cin][G]  w1t[l][j R + ci][co] = conv_l[co][ci][j], w1t[l][k R + cc][co] = conv1x1c_l[co][cc]
+ *   w2t [L][G2][S + R]     w2t[l][c2][o] = conv1x1_skip_l[o][c2] for o < S, conv1x1_out_l[o - S][c2] after
+ *                          (w1t[l] and w2t[l] are svsk_wavenet_block_f32's weights)
  *   wT [L][k G][Rp]        wT[l][j G + co][ci] = conv_l[co][ci][j]             (transposed conv of the backward)
  *   wB [L][R + S][G2p]     rows: conv1x1_out_l [R][G2] then conv1x1_skip_l [S][G2]
  *   wcT [cin][L G]         wcT[cc][l G + co] = conv1x1c_l[co][cc]

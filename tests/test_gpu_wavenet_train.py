@@ -1,6 +1,7 @@
 """WaveNet training on the device (wavenet/training.py): gradients of WaveNet.forward against float64 autograd through
 the oracle (oracle.wavenet_forward is built from differentiable torch ops, weight norm included), the forward against
-the eval path bit for bit, determinism, and a short SGD run against the same run driven by oracle gradients."""
+the eval path bit for bit, the weight packs against torch's weight-norm fold bit for bit, ResSkipBlock on its own,
+determinism, and a short SGD run against the same run driven by oracle gradients."""
 import pytest
 import torch
 import torch.nn.functional as F
@@ -124,6 +125,63 @@ def test_training_forward_equals_eval_forward(name):
     y_eval = m(c, x)
     assert y_eval.grad_fn is None and not y_eval.requires_grad          # eval mode with grad enabled: today's path
     assert torch.equal(y_train.detach(), y_eval)
+
+
+def _fold(mod):
+    """torch's weight-norm fold on CUDA; the weight itself after remove_weight_norm_()."""
+    if hasattr(mod, "weight_g"):
+        return torch._weight_norm(mod.weight_v, mod.weight_g, 0).detach()
+    return mod.weight.detach()
+
+
+@pytest.mark.parametrize("weight_norm", [True, False])
+@pytest.mark.parametrize("name", ["golden", "test_shape", "default", "k2"])
+def test_packs_equal_torch_weight_norm(name, weight_norm):
+    """The one fold of the library gives torch._weight_norm's bits, in the forward's pack and in the sampler's."""
+    m, _ = _model(name)
+    if not weight_norm:
+        m.remove_weight_norm_()
+    blocks, l1, l3 = m.main_conv_layers, m.last_conv_layers[1], m.last_conv_layers[3]
+    _, _, pk, _ = m._packed()
+    for l, f in enumerate(blocks):
+        k, R = f.kernel_size, f.conv.in_channels
+        w1t = torch.cat([_fold(f.conv).permute(2, 1, 0).reshape(k * R, -1), _fold(f.conv1x1c)[:, :, 0].t()])
+        w2t = torch.cat([_fold(f.conv1x1_skip), _fold(f.conv1x1_out)])[:, :, 0].t()
+        assert torch.equal(pk["w1t"][l], w1t) and torch.equal(pk["w2t"][l], w2t), l
+    for key, mod in (("first", m.first_conv), ("last1", l1), ("last3", l3)):
+        assert torch.equal(pk[key], _fold(mod)), key
+    # the sampler's ArLayout (include/svsk.h, svsk_wavenet_ar_f32): WfT, bf; per layer Wg, bg, Wso, bso; W3, b3, W4, b4
+    conf = m._ar_config()
+    assert conf is not None
+    wpack, wcond = m._ar_packed(conf)
+    bias = lambda mod: mod.bias.detach() if mod.bias is not None else torch.zeros(mod.out_channels, device=DEV)
+    parts = [_fold(m.first_conv)[:, :, 0].t(), bias(m.first_conv)]
+    for f in blocks:
+        G = f.conv.out_channels
+        parts += [_fold(f.conv).permute(0, 2, 1).reshape(G, -1), bias(f.conv),
+                  torch.cat([_fold(f.conv1x1_skip), _fold(f.conv1x1_out)]), torch.cat([bias(f.conv1x1_skip), bias(f.conv1x1_out)])]
+    parts += [_fold(l1), bias(l1), _fold(l3), bias(l3)]
+    assert torch.equal(wpack, torch.cat([p.flatten() for p in parts]))
+    assert torch.equal(wcond, torch.cat([_fold(f.conv1x1c) for f in blocks]))
+
+
+@pytest.mark.parametrize("weight_norm", [True, False])
+@pytest.mark.parametrize("name", ["golden", "test_shape", "default", "k2"])
+def test_res_skip_block_standalone_matches_oracle(name, weight_norm):
+    """ResSkipBlock.forward on its own (WaveNet runs its blocks from the shared pack) against oracle.wavenet_block."""
+    m, cfg = _model(name)
+    if not weight_norm:
+        m.remove_weight_norm_()
+    sd = {k: v.detach().cpu().double() for k, v in m.state_dict().items()}
+    gen = torch.Generator().manual_seed(5)
+    x = torch.randn(2, m.first_conv.out_channels, 300, generator=gen)
+    c = torch.randn(2, cfg["in_dim"], 300, generator=gen)
+    worst = {"rel": (0.0, ""), "abs": (0.0, "")}
+    for i, f in enumerate(m.main_conv_layers):
+        xo, s = f(x.to(DEV), c.to(DEV))
+        rx, rs = O.wavenet_block(sd, i, x.double(), c.double(), f.dilation)
+        _compare(f"block {i} x_out", xo.cpu().double(), rx, worst)
+        _compare(f"block {i} skips", s.cpu().double(), rs, worst)
 
 
 def test_no_grad_in_training_mode_takes_the_inference_path():
