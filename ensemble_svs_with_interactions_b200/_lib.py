@@ -80,6 +80,22 @@ class LstmParams(C.Structure):
     ]
 
 
+class LstmBwdParams(C.Structure):
+    _fields_ = [
+        ("dh", C.c_void_p), ("gates", C.c_void_p), ("cell", C.c_void_p), ("w_hh", C.c_void_p), ("lengths", C.c_void_p),
+        ("dpre", C.c_void_p), ("B", C.c_int32), ("T", C.c_int32), ("H", C.c_int32), ("ndir", C.c_int32),
+    ]
+
+
+class WgradF32Params(C.Structure):
+    _fields_ = [
+        ("dy", C.c_void_p), ("x", C.c_void_p), ("dw", C.c_void_p), ("db", C.c_void_p), ("ws", C.c_void_p),
+        ("dy_batch_stride", C.c_int64), ("x_batch_stride", C.c_int64),
+        ("B", C.c_int32), ("N", C.c_int32), ("K", C.c_int32), ("T", C.c_int32), ("ksize", C.c_int32), ("origin", C.c_int32),
+        ("pad_mode", C.c_int32), ("splits", C.c_int32),
+    ]
+
+
 class TapGemmBf16Params(C.Structure):
     _fields_ = [
         ("x", C.c_void_p), ("wp", C.c_void_p), ("bias", C.c_void_p), ("y_bf16", C.c_void_p), ("y_f32", C.c_void_p),
@@ -244,6 +260,11 @@ _SIGNATURES = {
     "svsk_bn_batch_stats_f32": [_V, _I, _I, _I, _V, _V, _V, _V, _F, _V],
     "svsk_bn_apply_f32": [_V, _V, _V, _V, _V, _V, _F, _I, _I, _I, _I, _V],
     "svsk_encoder_front": [_V, _V, _V, C.c_longlong, _I, _I, _I, _I, _I, _V],
+    "svsk_lstm_train_f32": [C.POINTER(LstmParams), _V, _V, _V],
+    "svsk_lstm_bwd_f32": [C.POINTER(LstmBwdParams), _V],
+    "svsk_wgrad_f32": [C.POINTER(WgradF32Params), _V],
+    "svsk_bn_relu_bwd_f32": [_V, _V, _V, _V, _V, _V, _F, _V, _V, _V, _I, _I, _I, _V],
+    "svsk_reflect_fold_f32": [_V, _V, _V, _I, _I, _I, _I, _I, _V],
     "svsk_filtfilt_f32": [_V, _V, _V, _V, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double), _I, _I, _I, _I, _I, _I, _V],
     "svsk_variance_scaling_f32": [_V, _V, _V, _V, _V, _I, _I, _I, _I, _V],
     "svsk_scale_features_f32": [_V, _V, _V, _V, _I, C.c_longlong, _I, _V],

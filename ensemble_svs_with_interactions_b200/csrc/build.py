@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = ["svsk_api.cu", "simt_f32.cu", "tma_util.cu", "diffnet_pack.cu", "diffnet_block3_sm100.cu", "diffnet_stack_sm100.cu", "diffnet_stack_duo_sm100.cu",
            "diffnet_step_sm100.cu", "diffnet_train_sm100.cu", "linear_sm100.cu", "usfgan_block_sm100.cu", "usfgan_block_fr_sm100.cu", "conv1d_sm100.cu", "usfgan_front.cu",
            "lstm_sm100.cu", "encoder_sm100.cu", "postproc.cu", "wavenet_f32.cu",
-           "wavenet_ar_sm100.cu", "wavenet_train_sm100.cu"]
+           "wavenet_ar_sm100.cu", "wavenet_train_sm100.cu", "lstm_train_sm100.cu", "encoder_train_sm100.cu"]
 LIB = os.path.join(HERE, "libsvsk.so")
 # micro-benchmarks behind tools/ubench_*.py: their own library, NOT part of the product libsvsk.so
 TOOLS = os.path.join(HERE, "..", "..", "tools")

@@ -18,15 +18,11 @@
 //    units to all CTAs of the cluster as 16-byte st.async messages that complete a transaction barrier in the
 //    receiver — no __syncthreads and no cluster-wide barrier inside the loop;
 //  * the gate pre-activations of step t+3 are fetched while step t computes (register ring, loop unrolled by four).
-#include <cuda_bf16.h>
 #include <cstdlib>
 
-#include "sm100_ptx.cuh"
-#include "svsk_common.cuh"
+#include "lstm_sm100.cuh"
 
 namespace svsk {
-
-constexpr int kLstmMaxThreads = 256;
 
 struct LstmArgs {
   const float* pre;
@@ -34,35 +30,18 @@ struct LstmArgs {
   const int32_t* lengths;
   float* h_f32;
   __nv_bfloat16* h_bf16;
+  float* gates;           // kTrain: [B][ndir*4H][T] activated gates i, f, g, o of every frame < length
+  float* cell;            // kTrain: [B][ndir*H][T] cell state c_t
   long long pre_sb, pre_st, pre_sr, hf_sb, hf_st, hf_sr, hb_sb, hb_st;
   int B, T, H, ndir;
   int NC, U, L;           // CTAs per cluster, units per CTA, real elements per column segment (H / CS)
   unsigned* dbg;          // SVSK_LSTM_TIMELINE: clock stamps of one step (CTA 0, thread 0)
 };
 
-__device__ __forceinline__ void st_async_v4(uint32_t cluster_addr, float a, float b, float c, float d, uint32_t cluster_mbar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.f32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(cluster_addr),
-               "f"(a), "f"(b), "f"(c), "f"(d), "r"(cluster_mbar)
-               : "memory");
-}
-
-// Gate activations on the critical path of every step: ex2.approx / rcp.approx forms, absolute error ~1e-6 (the fp32
-// parity tolerance is 2e-4), a third of the dependent-instruction chain of expf / tanhf.
-__device__ __forceinline__ float ex2_fast(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ float rcp_fast(float x) {
-  float y;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ float sigmoid_fast(float x) { return rcp_fast(1.f + ex2_fast(-1.4426950408889634f * x)); }
-__device__ __forceinline__ float tanh_fast(float x) { return fmaf(-2.f, rcp_fast(1.f + ex2_fast(2.8853900817779268f * x)), 1.f); }
-
-// CS column segments per unit (lanes unit*CS .. unit*CS+CS-1), KSEG = padded segment length.
-template <int CS, int KSEG>
+// CS column segments per unit (lanes unit*CS .. unit*CS+CS-1), KSEG = padded segment length.  kTrain: the input-gate lane
+// of each unit also stores the four activated gates and c_t of every frame (what svsk_lstm_bwd_f32 needs); the arithmetic
+// is the same instruction for instruction, so h is bit-identical to the inference kernel's.
+template <int CS, int KSEG, bool kTrain>
 __global__ void __launch_bounds__(kLstmMaxThreads, 1) lstm_recurrence_kernel(const LstmArgs a) {
   constexpr int kPitch = KSEG + 4;  // neighbouring segments start 4 banks apart: the CS broadcasts of a warp do not collide
   constexpr int NG = CS >= 4 ? 1 : 4 / CS;  // gates a lane owns after the reduction
@@ -216,6 +195,14 @@ __global__ void __launch_bounds__(kLstmMaxThreads, 1) lstm_recurrence_kernel(con
         const int frame = frame_of(t);
         if (a.h_f32) a.h_f32[(size_t)b * a.hf_sb + (size_t)frame * a.hf_st + (size_t)col * a.hf_sr] = h;
         if (a.h_bf16) a.h_bf16[(size_t)b * a.hb_sb + (size_t)frame * a.hb_st + col] = __float2bfloat16_rn(h);
+        if constexpr (kTrain) {
+          float* gp = a.gates + ((size_t)b * a.ndir * 4 + (size_t)d * 4) * H * a.T + (size_t)unit * a.T + frame;
+          gp[0] = gi;
+          gp[(size_t)H * a.T] = gf;
+          gp[(size_t)2 * H * a.T] = gg;
+          gp[(size_t)3 * H * a.T] = go;
+          a.cell[((size_t)b * a.ndir * H + col) * a.T + frame] = cell;
+        }
       }
     }
   }
@@ -225,47 +212,27 @@ __global__ void __launch_bounds__(kLstmMaxThreads, 1) lstm_recurrence_kernel(con
     const int frame = len + i / U, zc = d * H + c * U + i % U;
     if (a.h_f32) a.h_f32[(size_t)b * a.hf_sb + (size_t)frame * a.hf_st + (size_t)zc * a.hf_sr] = 0.f;
     if (a.h_bf16) a.h_bf16[(size_t)b * a.hb_sb + (size_t)frame * a.hb_st + zc] = __float2bfloat16_rn(0.f);
+    if constexpr (kTrain) {
+      for (int g = 0; g < 4; ++g) a.gates[((size_t)b * a.ndir * 4 * H + (size_t)d * 4 * H + g * H + c * U + i % U) * a.T + frame] = 0.f;
+      a.cell[((size_t)b * a.ndir * H + zc) * a.T + frame] = 0.f;
+    }
   }
   ptx::cluster_sync_all();  // nobody leaves while a peer may still address its shared memory
 }
 
-template <int CS, int KSEG>
+template <int CS, int KSEG, bool kTrain>
 static int launch_lstm(const LstmArgs& a, int threads, cudaStream_t st) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(a.B * a.ndir * a.NC));
-  cfg.blockDim = dim3((unsigned)threads);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = (unsigned)a.NC;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, lstm_recurrence_kernel<CS, KSEG>, a);
-  if (e != cudaSuccess) return fail((int)e, "lstm_f32: launch: %s", cudaGetErrorString(e));
-  return 0;
+  return launch_cluster(lstm_recurrence_kernel<CS, KSEG, kTrain>, a, a.B * a.ndir * a.NC, a.NC, threads, st, "lstm_f32");
 }
 
-// H -> (CTAs per cluster, units per CTA, column segments per unit, segment length); false when H has no layout here.
-static bool lstm_layout(int H, int* NC, int* U, int* CS, int* L) {
-  if (H < 4 || H > 256 || H % 4) return false;
-  int cs = 1;
-  while (H / cs > 32 || H % cs) {
-    cs *= 2;
-    if (cs > 8) return false;
-  }
-  if (H % (4 * cs)) return false;  // segments hold whole quads of units (16-byte messages)
-  for (int nc = 1; nc <= 8; nc *= 2) {
-    if (H % (4 * nc) || H / nc > 32) continue;
-    *NC = nc;
-    *U = H / nc;
-    *CS = cs;
-    *L = H / cs;
-    return true;
-  }
-  return false;
+template <bool kTrain>
+static int launch_lstm_any(const LstmArgs& a, int CS, int threads, cudaStream_t st) {
+  if (CS == 8) return launch_lstm<8, 32, kTrain>(a, threads, st);
+  if (CS == 4) return launch_lstm<4, 32, kTrain>(a, threads, st);
+  if (CS == 2) return launch_lstm<2, 32, kTrain>(a, threads, st);
+  if (a.L <= 8) return launch_lstm<1, 8, kTrain>(a, threads, st);
+  if (a.L <= 16) return launch_lstm<1, 16, kTrain>(a, threads, st);
+  return launch_lstm<1, 32, kTrain>(a, threads, st);
 }
 
 }  // namespace svsk
@@ -277,35 +244,37 @@ extern "C" int svsk_lstm_supported(int H) {
   return lstm_layout(H, &NC, &U, &CS, &L) ? 1 : 0;
 }
 
-extern "C" int svsk_lstm_f32(const svsk_lstm_params* pp, void* stream) {
-  SVSK_REQUIRE(pp != nullptr, SVSK_E_ARG, "lstm_f32: null params");
+// Argument checks shared by both entries, then the kernel arguments; 0 or an SVSK_E_* code (nothing launched).
+static int lstm_args(const svsk_lstm_params* pp, const char* what, LstmArgs* a, int* CS, int* threads) {
+  SVSK_REQUIRE(pp != nullptr, SVSK_E_ARG, "%s: null params", what);
   const svsk_lstm_params& p = *pp;
-  SVSK_REQUIRE(p.pre && p.w_hh && (p.h_f32 || p.h_bf16), SVSK_E_ARG, "lstm_f32: null tensor");
-  SVSK_REQUIRE(p.B > 0 && p.T > 0 && (p.ndir == 1 || p.ndir == 2), SVSK_E_ARG, "lstm_f32: B=%d T=%d ndir=%d", p.B, p.T, p.ndir);
-  LstmArgs a = {};
-  int CS = 1;
-  SVSK_REQUIRE(lstm_layout(p.H, &a.NC, &a.U, &CS, &a.L), SVSK_E_ARG,
-               "lstm_f32: hidden size %d has no cluster layout (need H <= 256 and H %% (4 * 2^k) == 0 with H / 2^k <= 32, k <= 3)", p.H);
+  SVSK_REQUIRE(p.pre && p.w_hh && (p.h_f32 || p.h_bf16), SVSK_E_ARG, "%s: null tensor", what);
+  SVSK_REQUIRE(p.B > 0 && p.T > 0 && (p.ndir == 1 || p.ndir == 2), SVSK_E_ARG, "%s: B=%d T=%d ndir=%d", what, p.B, p.T, p.ndir);
+  *a = LstmArgs{};
+  SVSK_REQUIRE(lstm_layout(p.H, &a->NC, &a->U, CS, &a->L), SVSK_E_ARG,
+               "%s: hidden size %d has no cluster layout (need H <= 256 and H %% (4 * 2^k) == 0 with H / 2^k <= 32, k <= 3)", what, p.H);
+  a->pre = p.pre; a->w_hh = p.w_hh; a->lengths = p.lengths; a->h_f32 = p.h_f32; a->h_bf16 = reinterpret_cast<__nv_bfloat16*>(p.h_bf16);
+  a->pre_sb = p.pre_stride_b; a->pre_st = p.pre_stride_t; a->pre_sr = p.pre_stride_r;
+  a->hf_sb = p.hf_stride_b; a->hf_st = p.hf_stride_t; a->hf_sr = p.hf_stride_c;
+  a->hb_sb = p.hb_stride_b; a->hb_st = p.hb_stride_t;
+  a->B = p.B; a->T = p.T; a->H = p.H; a->ndir = p.ndir;
+  *threads = (a->U * *CS + 31) & ~31;
+  SVSK_REQUIRE(*threads <= kLstmMaxThreads, SVSK_E_ARG, "%s: %d threads", what, *threads);
+  return 0;
+}
+
+extern "C" int svsk_lstm_f32(const svsk_lstm_params* pp, void* stream) {
+  LstmArgs a;
+  int CS = 1, threads = 0;
+  if (int rc = lstm_args(pp, "lstm_f32", &a, &CS, &threads)) return rc;
+  const svsk_lstm_params& p = *pp;
   if (int rc = require_sm100()) return rc;
-  a.pre = p.pre; a.w_hh = p.w_hh; a.lengths = p.lengths; a.h_f32 = p.h_f32; a.h_bf16 = reinterpret_cast<__nv_bfloat16*>(p.h_bf16);
-  a.pre_sb = p.pre_stride_b; a.pre_st = p.pre_stride_t; a.pre_sr = p.pre_stride_r;
-  a.hf_sb = p.hf_stride_b; a.hf_st = p.hf_stride_t; a.hf_sr = p.hf_stride_c;
-  a.hb_sb = p.hb_stride_b; a.hb_st = p.hb_stride_t;
-  a.B = p.B; a.T = p.T; a.H = p.H; a.ndir = p.ndir;
   static unsigned* dbg_buf = nullptr;
   const bool timeline = getenv("SVSK_LSTM_TIMELINE") != nullptr;
   if (timeline && !dbg_buf) cudaMalloc(&dbg_buf, 64);
   a.dbg = timeline ? dbg_buf : nullptr;
-  const int threads = (a.U * CS + 31) & ~31;
-  SVSK_REQUIRE(threads <= kLstmMaxThreads, SVSK_E_ARG, "lstm_f32: %d threads", threads);
   cudaStream_t st = as_stream(stream);
-  int rc;
-  if (CS == 8) rc = launch_lstm<8, 32>(a, threads, st);
-  else if (CS == 4) rc = launch_lstm<4, 32>(a, threads, st);
-  else if (CS == 2) rc = launch_lstm<2, 32>(a, threads, st);
-  else if (a.L <= 8) rc = launch_lstm<1, 8>(a, threads, st);
-  else if (a.L <= 16) rc = launch_lstm<1, 16>(a, threads, st);
-  else rc = launch_lstm<1, 32>(a, threads, st);
+  int rc = launch_lstm_any<false>(a, CS, threads, st);
   if (timeline && rc == 0) {  // debugging aid: cycles from the top of step 65 to {wait done, dot done, h done, sent}
     unsigned h[8];
     cudaStreamSynchronize(st);
@@ -313,4 +282,15 @@ extern "C" int svsk_lstm_f32(const svsk_lstm_params* pp, void* stream) {
     fprintf(stderr, "lstm timeline H=%d NC=%d: wait %u dot %u h %u sent %u\n", p.H, a.NC, h[1] - h[0], h[2] - h[0], h[3] - h[0], h[4] - h[0]);
   }
   return rc;
+}
+
+extern "C" int svsk_lstm_train_f32(const svsk_lstm_params* pp, float* gates, float* cell, void* stream) {
+  LstmArgs a;
+  int CS = 1, threads = 0;
+  if (int rc = lstm_args(pp, "lstm_train_f32", &a, &CS, &threads)) return rc;
+  SVSK_REQUIRE(gates && cell, SVSK_E_ARG, "lstm_train_f32: null gates / cell");
+  if (int rc = require_sm100()) return rc;
+  a.gates = gates;
+  a.cell = cell;
+  return launch_lstm_any<true>(a, CS, threads, as_stream(stream));
 }

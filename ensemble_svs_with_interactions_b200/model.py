@@ -19,7 +19,13 @@ Linear: ``forward`` returns (log_pi, log_sigma, mu) [B, T, G, D], ``inference`` 
 component (svsk_mdn_head_f32).  Training mode (module.train()): the FORWARD is built for dropout = 0 — what the diffusion
 recipe's encoders use — i.e. BatchNorm1d with the batch statistics of the padded batch and the running-buffer update
 (svsk_bn_batch_stats_f32 / svsk_bn_apply_f32; fp32 kernels whatever ``precision`` says, since the statistics are taken
-on the convolution's own output); there are no backward kernels for the encoder, so a call that needs gradients raises.
+on the convolution's own output).
+
+``backward_kernels=True`` makes the module trainable on the device: in training mode with grad enabled, when ``x``,
+``spk_embs`` or a parameter requires grad, ``forward`` is one autograd Function (encoder_training.py) and
+``loss.backward()`` fills every parameter's ``.grad`` (and those of ``x`` / ``spk_embs``); output and BatchNorm buffers are
+those of the no-grad training forward, bit for bit.  Eval mode and ``torch.no_grad()`` record no graph, as for WaveNet.
+With the default ``backward_kernels=False`` a call that needs gradients raises (the MDN head has no backward either way).
 """
 from __future__ import annotations
 
@@ -28,7 +34,7 @@ from typing import Optional
 import torch
 from torch import nn
 
-from . import ops
+from . import encoder_training, ops
 from .base import BaseModel, PredictionType
 
 __all__ = ["FFConvLSTM", "MultiSpeakerFFConvLSTM", "MDNLayer", "init_weights"]
@@ -179,7 +185,7 @@ class FFConvLSTM(BaseModel):
 
     def __init__(self, in_dim, ff_hidden_dim=2048, conv_hidden_dim=1024, lstm_hidden_dim=256, out_dim=67, dropout=0.0,
                  num_lstm_layers=2, bidirectional=True, init_type="none", use_mdn=False, dim_wise=True, num_gaussians=4,
-                 in_ph_start_idx: int = 1, in_ph_end_idx: int = 50, embed_dim=None, precision="auto"):
+                 in_ph_start_idx: int = 1, in_ph_end_idx: int = 50, embed_dim=None, precision="auto", backward_kernels=False):
         super().__init__()
         self.in_dim, self.out_dim = in_dim, out_dim
         self.num_gaussians = num_gaussians
@@ -188,6 +194,7 @@ class FFConvLSTM(BaseModel):
         self.embed_dim = embed_dim
         self.use_mdn = use_mdn
         self.precision = precision
+        self.backward_kernels = bool(backward_kernels)
         self.ff_hidden_dim, self.conv_hidden_dim, self.lstm_hidden_dim = ff_hidden_dim, conv_hidden_dim, lstm_hidden_dim
         self._padded_hidden = None
 
@@ -248,14 +255,26 @@ class FFConvLSTM(BaseModel):
         return self._plan
 
     # ------------------------------------------------------------------ forward
-    def _check(self, x, lengths):
+    def _records_grad(self, x, spk_embs):
+        """True when forward runs as the autograd Function: backward_kernels, training mode, grad enabled and something
+        that requires grad."""
+        return (self.backward_kernels and self.training and torch.is_grad_enabled()
+                and (x.requires_grad or (spk_embs is not None and spk_embs.requires_grad)
+                     or any(p.requires_grad for p in self.parameters())))
+
+    def _check(self, x, lengths, spk_embs=None):
         if self.training:
             if self.lstm.dropout > 0 and self.lstm.num_layers > 1:
                 raise RuntimeError("FFConvLSTM: the training-mode forward is built for dropout = 0 only (the diffusion recipe's "
                                    f"encoders); got dropout = {self.lstm.dropout}.  Call .eval() for inference")
-            if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
-                raise RuntimeError("FFConvLSTM has no backward kernels: the training-mode forward (BatchNorm batch statistics, "
-                                   "running-buffer update) runs under torch.no_grad() or with frozen parameters only")
+            if not self.backward_kernels:
+                if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+                    raise RuntimeError("FFConvLSTM has no backward kernels: the training-mode forward (BatchNorm batch statistics, "
+                                       "running-buffer update) runs under torch.no_grad() or with frozen parameters only; "
+                                       "construct with backward_kernels=True to train it on the device")
+            elif self.use_mdn and self._records_grad(x, spk_embs):
+                raise RuntimeError("FFConvLSTM(backward_kernels=True): the MDN head (use_mdn=True) has no backward kernels; "
+                                   "train it with use_mdn=False or run the training forward under torch.no_grad()")
         if not x.is_cuda:
             raise RuntimeError("FFConvLSTM: input must be a CUDA tensor (libsvsk has no CPU path)")
         if x.dim() != 3 or x.shape[-1] != self.in_dim:
@@ -283,18 +302,26 @@ class FFConvLSTM(BaseModel):
         if self.training:
             # BatchNorm1d with batch statistics (model.py:839-852 under module.train()): the fp32 kernels, the convolutions'
             # own weights (nothing folded), the running buffers updated in place -> the cached eval plan is stale afterwards
-            key = tuple((p.data_ptr(), p._version) for p in self.parameters())
-            if self.__dict__.get("_plan_train_key") != key:
-                self.__dict__["_plan_train"], self.__dict__["_plan_train_key"] = _Plan(self, "fp32"), key
+            plan = self._train_plan()
             with torch.no_grad():
-                out = self._forward_fp32(x, lens_dev, spk_embs, self.__dict__["_plan_train"], train=True)
+                out = self._forward_fp32(x, lens_dev, spk_embs, plan, train=True)
             self._plan = None
             return out[:, :max(lens)]
         plan = self.plan()
         out = self._forward_fp32(x, lens_dev, spk_embs, plan) if plan.precision == "fp32" else self._forward_bf16(x, lens_dev, spk_embs, plan)
         return out[:, :max(lens)]
 
+    def _train_plan(self) -> _Plan:
+        """fp32 weights of the training forward, rebuilt when a parameter changes."""
+        key = tuple((p.data_ptr(), p._version) for p in self.parameters())
+        if self.__dict__.get("_plan_train_key") != key:
+            self.__dict__["_plan_train"], self.__dict__["_plan_train_key"] = _Plan(self, "fp32"), key
+        return self.__dict__["_plan_train"]
+
     def forward(self, x, lengths=None, y=None, spk_embs=None):
+        if self._records_grad(x, spk_embs):
+            lens = self._check(x, lengths, spk_embs)
+            return encoder_training.ffconvlstm_forward_with_grad(self, x, lens, spk_embs)
         raw = self._raw(x, lengths, spk_embs)
         if self.use_mdn:     # (log_pi, log_sigma, mu), each [B, T, G, D]  (mdn.py:45-74)
             return ops.mdn_head_f32(raw.contiguous(), self.num_gaussians, self.out_dim)[0]
@@ -307,36 +334,55 @@ class FFConvLSTM(BaseModel):
             return mu, sigma
         return self(x, lengths, spk_embs=spk_embs)
 
-    def _forward_fp32(self, x, lens_dev, spk, plan, train=False):
+    def _forward_fp32(self, x, lens_dev, spk, plan, train=False, keep=None):
+        """keep (training only): a dict that receives what encoder_training's backward needs; the BatchNorm is then applied
+        out of place and the recurrences also store their gates and cells — the same kernels and the same output bits."""
         B, T, _ = x.shape
         H = plan.Hp
         if self.embed_dim is not None:
             xf = torch.empty((B * T, self.in_dim), device=x.device, dtype=torch.float32)
             ops.encoder_front(x.view(B * T, self.in_dim), self.in_ph_start_idx, self.num_vocab, y_f32=xf)
             h = ops.ntc_to_nct_f32(xf.view(B, T, self.in_dim), self.in_dim)
+            if keep is not None:
+                keep["front_in"] = h
             h = ops.conv1d_f32(h, plan.front[0][0], plan.front[0][1])
         else:
             h = ops.ntc_to_nct_f32(x, self.in_dim)
         if spk is not None:
             h = ops.lincomb_f32([h, ops.ntc_to_nct_f32(spk, spk.shape[-1])], [1.0, 1.0])
+        ff = [h]
         for w, b in plan.ff:
             h = ops.conv1d_f32(h, w, b, act=ops.ACT_RELU)
+            ff.append(h)
+        if keep is not None:
+            keep.update(ff=ff, conv=[], lstm=[])
         for k, (w, b) in enumerate(plan.conv):
             if train:
                 conv, bn = self.conv[4 * k + 1], self.conv[4 * k + 2]
                 if bn.momentum is None or not bn.track_running_stats:
                     raise RuntimeError("FFConvLSTM: BatchNorm1d(momentum=None / track_running_stats=False) is not built")
+                a_in = h
                 h = ops.conv1d_f32(h, conv.weight.detach().float().contiguous(), conv.bias.detach().float().contiguous(),
                                    pad_mode=ops.PAD_REFLECT)
-                ops.batchnorm_train_f32(h, bn.weight.detach().float().contiguous(), bn.bias.detach().float().contiguous(),
-                                        bn.running_mean, bn.running_var, eps=bn.eps, momentum=bn.momentum, relu=True)
+                z = h
+                stats = None if keep is None else (torch.empty_like(h[0, :, 0]), torch.empty_like(h[0, :, 0]))
+                h = ops.batchnorm_train_f32(z, bn.weight.detach().float().contiguous(), bn.bias.detach().float().contiguous(),
+                                            bn.running_mean, bn.running_var, eps=bn.eps, momentum=bn.momentum, relu=True,
+                                            out=None if keep is None else torch.empty_like(z), stats=stats)
                 bn.num_batches_tracked += 1
+                if keep is not None:
+                    keep["conv"].append((z, stats, h, a_in))
             else:
                 h = ops.conv1d_f32(h, w, b, pad_mode=ops.PAD_REFLECT, act=ops.ACT_RELU)
         for w_ih, b, w_hh in plan.lstm:
             pre = ops.conv1d_f32(h, w_ih, b)                                   # [B, 8H, T]
-            h = torch.empty((B, 2 * H, T), device=x.device, dtype=torch.float32)
-            ops.lstm_f32(pre, w_hh, lens_dev, H, pre_layout="nct", h_f32=h)
+            h_in, h = h, torch.empty((B, 2 * H, T), device=x.device, dtype=torch.float32)
+            if keep is None:
+                ops.lstm_f32(pre, w_hh, lens_dev, H, pre_layout="nct", h_f32=h)
+            else:
+                gates, cell = torch.empty_like(pre), torch.empty_like(h)
+                ops.lstm_train_f32(pre, w_hh, lens_dev, H, h_f32=h, gates=gates, cell=cell)
+                keep["lstm"].append((h_in, h, gates, cell))
         y = ops.conv1d_f32(h, plan.fc[0], plan.fc[1])                          # [B, n_out, T]
         return ops.nct_to_ntc(y, want_bf16=False, want_f32=True)[1]
 
@@ -389,9 +435,11 @@ class MultiSpeakerFFConvLSTM(FFConvLSTM):
 
     def __init__(self, in_dim, speaker_embedding, ff_hidden_dim=2048, conv_hidden_dim=1024, lstm_hidden_dim=256, out_dim=67,
                  dropout=0.0, num_lstm_layers=2, bidirectional=True, init_type="none", use_mdn=False, dim_wise=True,
-                 num_gaussians=4, in_ph_start_idx: int = 1, in_ph_end_idx: int = 50, embed_dim=None, precision="auto"):
+                 num_gaussians=4, in_ph_start_idx: int = 1, in_ph_end_idx: int = 50, embed_dim=None, precision="auto",
+                 backward_kernels=False):
         super().__init__(in_dim, ff_hidden_dim, conv_hidden_dim, lstm_hidden_dim, out_dim, dropout, num_lstm_layers, bidirectional,
-                         init_type, use_mdn, dim_wise, num_gaussians, in_ph_start_idx, in_ph_end_idx, embed_dim, precision)
+                         init_type, use_mdn, dim_wise, num_gaussians, in_ph_start_idx, in_ph_end_idx, embed_dim, precision,
+                         backward_kernels)
         self.speaker_embedding = speaker_embedding
 
     def forward(self, x, spks, lengths=None, y=None):

@@ -967,17 +967,135 @@ def encoder_front(x, onehot_start, onehot_len, *, y_f32=None, y_bf16=None):
                                        0 if y_bf16 is None else y_bf16.shape[1], L.stream_ptr()), "encoder_front")
 
 
-def batchnorm_train_f32(x, gamma, beta, running_mean, running_var, *, eps, momentum, relu=True):
-    """nn.BatchNorm1d in training mode (+ ReLU) on x [B, C, T] fp32, in place: batch statistics over all B*T positions,
-    running buffers updated as torch does (svsk_bn_batch_stats_f32 + svsk_bn_apply_f32).  Returns x."""
+def batchnorm_train_f32(x, gamma, beta, running_mean, running_var, *, eps, momentum, relu=True, out=None, stats=None):
+    """nn.BatchNorm1d in training mode (+ ReLU) on x [B, C, T] fp32: batch statistics over all B*T positions, running
+    buffers updated as torch does (svsk_bn_batch_stats_f32 + svsk_bn_apply_f32).  In place unless ``out`` [B, C, T] is
+    given (x is then kept, as the backward needs it); ``stats``: (mean, var) [C] tensors that receive the batch
+    statistics.  Returns the output."""
     B, Cc, T = x.shape
-    mean = torch.empty((Cc,), device=x.device, dtype=f32)
-    var = torch.empty((Cc,), device=x.device, dtype=f32)
+    if out is None:
+        out = x
+    _shape("batchnorm_train_f32: out", out, x.shape)
+    if stats is None:
+        stats = (torch.empty((Cc,), device=x.device, dtype=f32), torch.empty((Cc,), device=x.device, dtype=f32))
+    mean, var = stats
+    _shape("batchnorm_train_f32: mean", mean, (Cc,))
+    _shape("batchnorm_train_f32: var", var, (Cc,))
     L.check(L.lib().svsk_bn_batch_stats_f32(L.ptr(x, f32, "x"), B, Cc, T, L.ptr(mean), L.ptr(var), L.ptr(running_mean, f32),
                                             L.ptr(running_var, f32), float(momentum), L.stream_ptr()), "bn_batch_stats_f32")
-    L.check(L.lib().svsk_bn_apply_f32(L.ptr(x, f32, "x"), L.ptr(x), L.ptr(mean), L.ptr(var), L.ptr(gamma, f32), L.ptr(beta, f32),
-                                      float(eps), int(relu), B, Cc, T, L.stream_ptr()), "bn_apply_f32")
-    return x
+    L.check(L.lib().svsk_bn_apply_f32(L.ptr(x, f32, "x"), L.ptr(out, f32, "out"), L.ptr(mean), L.ptr(var), L.ptr(gamma, f32),
+                                      L.ptr(beta, f32), float(eps), int(relu), B, Cc, T, L.stream_ptr()), "bn_apply_f32")
+    return out
+
+
+# ---- FFConvLSTM encoder training (include/svsk.h, "FFConvLSTM encoder training") ------------------------------------
+def lstm_train_f32(pre, w_hh, lengths, H, *, h_f32, gates, cell):
+    """svsk_lstm_train_f32: lstm_f32 with pre [B, ndir*4H, T] ("nct") and h_f32 [B, ndir*H, T] that also writes the
+    activated gates [B, ndir*4H, T] and the cell states [B, ndir*H, T] the backward needs."""
+    ndir = w_hh.shape[0]
+    B, R, T = pre.shape
+    _shape("lstm_train_f32: w_hh", w_hh, (ndir, 4 * H, H))
+    _shape("lstm_train_f32: pre", pre, (B, ndir * 4 * H, T))
+    _shape("lstm_train_f32: h_f32", h_f32, (B, ndir * H, T))
+    _shape("lstm_train_f32: gates", gates, (B, ndir * 4 * H, T))
+    _shape("lstm_train_f32: cell", cell, (B, ndir * H, T))
+    p = L.LstmParams()
+    p.pre, p.w_hh, p.lengths = L.ptr(pre, f32, "pre"), L.ptr(w_hh, f32, "w_hh"), L.ptr(lengths, torch.int32, "lengths")
+    p.pre_stride_b, p.pre_stride_t, p.pre_stride_r = R * T, 1, T
+    p.h_f32 = L.ptr(h_f32, f32, "h_f32")
+    p.hf_stride_b, p.hf_stride_t, p.hf_stride_c = ndir * H * T, 1, T
+    p.B, p.T, p.H, p.ndir = B, T, H, ndir
+    L.check(L.lib().svsk_lstm_train_f32(C.byref(p), L.ptr(gates, f32, "gates"), L.ptr(cell, f32, "cell"), L.stream_ptr()),
+            "lstm_train_f32")
+
+
+def lstm_bwd_f32(dh, gates, cell, w_hh, lengths, H, out=None):
+    """svsk_lstm_bwd_f32: dL/dpre [B, ndir*4H, T] from dL/dh [B, ndir*H, T] and lstm_train_f32's gates / cell."""
+    ndir = w_hh.shape[0]
+    B, _, T = dh.shape
+    _shape("lstm_bwd_f32: w_hh", w_hh, (ndir, 4 * H, H))
+    _shape("lstm_bwd_f32: dh", dh, (B, ndir * H, T))
+    _shape("lstm_bwd_f32: gates", gates, (B, ndir * 4 * H, T))
+    _shape("lstm_bwd_f32: cell", cell, (B, ndir * H, T))
+    if lengths is not None:
+        _shape("lstm_bwd_f32: lengths", lengths, (B,))
+    out = torch.empty((B, ndir * 4 * H, T), device=dh.device, dtype=f32) if out is None else out
+    _shape("lstm_bwd_f32: out", out, (B, ndir * 4 * H, T))
+    p = L.LstmBwdParams()
+    p.dh, p.gates, p.cell = L.ptr(dh, f32, "dh"), L.ptr(gates, f32, "gates"), L.ptr(cell, f32, "cell")
+    p.w_hh, p.lengths, p.dpre = L.ptr(w_hh, f32, "w_hh"), L.ptr(lengths, torch.int32, "lengths"), L.ptr(out, f32, "out")
+    p.B, p.T, p.H, p.ndir = B, T, H, ndir
+    L.check(L.lib().svsk_lstm_bwd_f32(C.byref(p), L.stream_ptr()), "lstm_bwd_f32")
+    return out
+
+
+def _frames_view(name, t):
+    """Batch stride of a [B, C, T] fp32 CUDA tensor whose rows are T contiguous frames (a channel slice is fine)."""
+    if t.dim() != 3 or t.stride(2) != 1 or t.stride(1) != t.shape[2]:
+        raise ValueError(f"{name} must be [B, C, T] with rows of T contiguous frames, got shape {list(t.shape)} strides {t.stride()}")
+    if not t.is_cuda or t.dtype != f32:
+        raise RuntimeError(f"{name} must be a CUDA fp32 tensor: libsvsk has no CPU path")
+    return t.stride(0)
+
+
+def wgrad_f32_splits(B, T, N, ncols, target=2 * 148):
+    """Frame splits of svsk_wgrad_f32: about two waves of CTAs on a B200, at least 4 chunks of 32 frames per split."""
+    tiles = -(-N // 64) * -(-ncols // 64)
+    return max(1, min(-(-target // tiles), (B * -(-T // 32)) // 4, 64))
+
+
+def wgrad_f32(dy, x, *, ksize=1, origin=0, pad_mode=PAD_ZEROS, bias=True, dw=None):
+    """svsk_wgrad_f32: dw [N, K, ksize] = sum_b sum_t dy[b, n, t] x[b, k, t + j - origin] (zero / reflect padded) and,
+    with ``bias``, db [N] = sum dy.  dy [B, N, T], x [B, K, T] (channel slices of larger tensors allowed).  -> (dw, db)."""
+    B, N, T = dy.shape
+    if x.dim() != 3 or x.shape[0] != B or x.shape[2] != T:
+        raise ValueError(f"wgrad_f32: x must be [{B}, K, {T}], got {list(x.shape)}")
+    K = x.shape[1]
+    dsb, xsb = _frames_view("wgrad_f32: dy", dy), _frames_view("wgrad_f32: x", x)
+    dw = torch.empty((N, K, ksize), device=dy.device, dtype=f32) if dw is None else dw
+    _shape("wgrad_f32: dw", dw, (N, K, ksize))
+    db = torch.empty((N,), device=dy.device, dtype=f32) if bias else None
+    ncols = K * ksize + int(bias)
+    splits = wgrad_f32_splits(B, T, N, ncols)
+    ws = torch.empty((splits, N, ncols), device=dy.device, dtype=f32) if splits > 1 else None
+    p = L.WgradF32Params()
+    p.dy, p.x = C.c_void_p(dy.data_ptr()), C.c_void_p(x.data_ptr())
+    p.dw, p.db, p.ws = L.ptr(dw, f32, "dw"), L.ptr(db), L.ptr(ws)
+    p.dy_batch_stride, p.x_batch_stride = dsb, xsb
+    p.B, p.N, p.K, p.T, p.ksize, p.origin, p.pad_mode, p.splits = B, N, K, T, int(ksize), int(origin), int(pad_mode), splits
+    L.check(L.lib().svsk_wgrad_f32(C.byref(p), L.stream_ptr()), "wgrad_f32")
+    return dw, db
+
+
+def bn_relu_bwd_f32(dy, y, x, mean, var, gamma, *, eps, out=None):
+    """svsk_bn_relu_bwd_f32: BatchNorm1d (batch statistics) + ReLU backward on [B, C, T] -> (dx, dgamma, dbeta).
+    y: the forward's ReLU output, x: the BatchNorm input, mean / var: its batch statistics; out may be dy."""
+    B, Cc, T = dy.shape
+    for name, t in (("y", y), ("x", x)):
+        _shape(f"bn_relu_bwd_f32: {name}", t, (B, Cc, T))
+    for name, t in (("mean", mean), ("var", var), ("gamma", gamma)):
+        _shape(f"bn_relu_bwd_f32: {name}", t, (Cc,))
+    out = torch.empty_like(dy) if out is None else out
+    _shape("bn_relu_bwd_f32: out", out, (B, Cc, T))
+    dgamma = torch.empty((Cc,), device=dy.device, dtype=f32)
+    dbeta = torch.empty((Cc,), device=dy.device, dtype=f32)
+    L.check(L.lib().svsk_bn_relu_bwd_f32(L.ptr(dy, f32, "dy"), L.ptr(y, f32, "y"), L.ptr(x, f32, "x"), L.ptr(mean, f32, "mean"),
+                                         L.ptr(var, f32, "var"), L.ptr(gamma, f32, "gamma"), float(eps), L.ptr(out, f32, "out"),
+                                         L.ptr(dgamma), L.ptr(dbeta), B, Cc, T, L.stream_ptr()), "bn_relu_bwd_f32")
+    return out, dgamma, dbeta
+
+
+def reflect_fold_f32(dx, dy, w):
+    """svsk_reflect_fold_f32, in place on dx [B, Cin, T]: adds the ReflectionPad1d rows of the Conv1d w [Cout, Cin, k]
+    (pad = (k - 1) / 2) whose output gradient is dy [B, Cout, T].  Returns dx."""
+    B, Cin, T = dx.shape
+    Cout, Cin_w, k = w.shape
+    if Cin_w != Cin or k % 2 == 0:
+        raise ValueError(f"reflect_fold_f32: w must be [Cout, {Cin}, odd k], got {list(w.shape)}")
+    _shape("reflect_fold_f32: dy", dy, (B, Cout, T))
+    L.check(L.lib().svsk_reflect_fold_f32(L.ptr(dx, f32, "dx"), L.ptr(dy, f32, "dy"), L.ptr(w, f32, "w"), B, Cin, Cout, T,
+                                          (k - 1) // 2, L.stream_ptr()), "reflect_fold_f32")
+    return dx
 
 
 # ---- acoustic post-processing (include/svsk.h, "acoustic post-processing on the device") ----------------------------

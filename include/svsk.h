@@ -459,6 +459,66 @@ SVSK_API int svsk_bn_apply_f32(const float* x, float* y, const float* mean, cons
 SVSK_API int svsk_encoder_front(const float* x, float* y_f32, void* y_bf16, long long rows, int in_dim, int onehot_start,
                                 int onehot_len, int ldy_f, int ldy_b, void* stream);
 
+/* ---- FFConvLSTM encoder training (backward of model.py:893-922 with dropout = 0), fp32 on the CUDA cores ---------- */
+
+/* svsk_lstm_f32 that also keeps what the backward needs: gates [B][ndir*4H][T] (the activated i, f, g, o of every frame
+ * < lengths[b], torch row order within a direction: gates[b][(dir*4 + g)*H + u][t]) and cell [B][ndir*H][T] (c_t).
+ * Frames >= lengths[b] hold zeros.  Same checks as svsk_lstm_f32; h is bit-identical to svsk_lstm_f32's. */
+SVSK_API int svsk_lstm_train_f32(const svsk_lstm_params* p, float* gates, float* cell, void* stream);
+
+/* Backward of the recurrence (torch.nn.LSTM's backward through pack_padded_sequence, model.py:917-919), in each
+ * direction's own scan order reversed (the reverse direction starts at lengths[b] - 1):
+ *   dh = dh_ext[t] + W_hh^T da_{t+1} ; dc = dc_{t+1} f_{t+1} + dh o (1 - tanh^2 c_t)
+ *   dpre[t] = da_t = [dc g i(1-i), dc c_{t-1} f(1-f), dc i (1-g^2), dh tanh(c_t) o(1-o)]
+ * dpre = dL/d(W_ih x + b_ih + b_hh) [B][ndir*4H][T], zero for frames >= lengths[b] (dh_ext there is not read).
+ * dh_ext [B][ndir*H][T]; gates / cell from svsk_lstm_train_f32; w_hh [ndir][4H][H]; lengths [B] or NULL (= T).
+ * H as svsk_lstm_supported.  One thread-block cluster per (track, direction), W_hh^T in registers. */
+typedef struct svsk_lstm_bwd_params {
+  const float* dh;
+  const float* gates;
+  const float* cell;
+  const float* w_hh;
+  const int32_t* lengths;
+  float* dpre;
+  int32_t B, T, H, ndir;
+} svsk_lstm_bwd_params;
+SVSK_API int svsk_lstm_bwd_f32(const svsk_lstm_bwd_params* p, void* stream);
+
+/* Weight (and bias) gradient of a Conv1d / Linear, also of W_hh with a one-frame shift:
+ *   dw[n][k][j] = sum_b sum_t dy[b][n][t] * x[b][k][src(t + j - origin)] ;  db[n] = sum_b sum_t dy[b][n][t]
+ * dy at dy[b*dy_batch_stride + n*T + t], x at x[b*x_batch_stride + k*T + u]; src: pad_mode SVSK_PAD_ZEROS (0 outside
+ * [0, T)) or SVSK_PAD_REFLECT (ReflectionPad1d, needs 0 <= origin < ksize and a reach below T).  Uses: the Linears
+ * (ksize 1, origin 0), the ReflectionPad1d(3) + Conv1d(k=7) layers (origin 3, reflect), the LSTM input projections, and
+ * W_hh as da^T against h of the previous step (origin 1 forward, -1 reverse: h[lengths[b]] = 0 is read).  db may be NULL.
+ * 64 x 64 output tiles reduced over 32-frame chunks in a fixed order; splits > 1 splits the chunks and needs ws
+ * [splits][N][K*ksize + (db != NULL)], summed in split order by a second launch.  No atomics: bit-reproducible. */
+typedef struct svsk_wgrad_f32_params {
+  const float* dy;
+  const float* x;
+  float* dw;                /* [N][K][ksize] */
+  float* db;                /* [N] or NULL */
+  float* ws;
+  int64_t dy_batch_stride, x_batch_stride;
+  int32_t B, N, K, T, ksize, origin, pad_mode, splits;
+} svsk_wgrad_f32_params;
+SVSK_API int svsk_wgrad_f32(const svsk_wgrad_f32_params* p, void* stream);
+
+/* BatchNorm1d (batch statistics, model.py:839-852 under module.train()) + ReLU backward over all B*T positions of a
+ * channel, padded frames included: with xhat = (x - mean) / sqrtf(var + eps) (x the BatchNorm input, mean / var the
+ * forward's svsk_bn_batch_stats_f32 outputs) and y the forward's ReLU output,
+ *   dz = dy [y > 0] ; dbeta = sum dz ; dgamma = sum dz xhat ; dx = gamma / sqrt(var + eps) (dz - (dbeta + xhat dgamma) / (B T))
+ * All [B][C][T] fp32; dx may be dy. */
+SVSK_API int svsk_bn_relu_bwd_f32(const float* dy, const float* y, const float* x, const float* mean, const float* var,
+                                  const float* gamma, float eps, float* dx, float* dgamma, float* dbeta, int B, int C, int T,
+                                  void* stream);
+
+/* nn.ReflectionPad1d(pad) backward in front of a Conv1d(w [Cout][Cin][2 pad + 1]): dx [B][Cin][T] holds the gradient of
+ * the padded input's centre rows (svsk_conv1d_f32 of dy with the flipped, transposed weights); this adds the padded rows
+ * dXp[p] = sum_j w[:, ci, j]^T dy[p - j] into the frames they reflect: rows 0 .. pad-1 into frames pad .. 1, rows
+ * T+pad .. T+2pad-1 into frames T-2 .. T-1-pad.  dy [B][Cout][T]; 1 <= pad <= 4, T > pad. */
+SVSK_API int svsk_reflect_fold_f32(float* dx, const float* dy, const float* w, int B, int Cin, int Cout, int T, int pad,
+                                   void* stream);
+
 /* ---- acoustic post-processing on the device (SURVEY.md §8(f) row 3) ----------------------------------------------- */
 
 /* nnsvs.dsp.lowpass_filter over whole batches (dsp.py:10-33; gen.py:1500-1513 calls it per feature dimension):
