@@ -11,7 +11,6 @@
 // sequence end: those tiles are filled row by row by four gather warps (cp.async).  Two TMEM accumulators let the epilogue
 // (8 warps: bias, ReLU / sigmoid, bf16, swizzled smem, one TMA store per lane quarter) of tile n overlap the MMAs of n+1.
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "sm100_ptx.cuh"
 #include "svsk_common.cuh"
@@ -340,7 +339,7 @@ extern "C" int svsk_conv1d_bf16(const svsk_conv1d_bf16_params* pp, void* stream)
   const int fixed = wbytes + 2 * out_chunks * kCTile + 256 * 4 + (int)sizeof(ConvBarriers) + 1024;
   // window mode: all taps of a tile out of one (128 + span)-row load per channel block
   const int span = (p.ksize - 1) * p.dilation;
-  const int window = (p.ksize > 1 && span <= kCMaxSpan && !getenv("SVSK_CONV1D_NO_WINDOW")) ? 1 : 0;
+  const int window = (p.ksize > 1 && span <= kCMaxSpan) ? 1 : 0;
   const int win_rows = window ? (128 + span + 7) / 8 * 8 : 128;
   const int stage_bytes = win_rows * 128;
   int nstages = (232448 - fixed) / stage_bytes;

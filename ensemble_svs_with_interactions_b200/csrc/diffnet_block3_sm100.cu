@@ -23,7 +23,6 @@
 //   C: for block j:     Wout[block j][kb], kb < C/64          (A operand = G tile kb)
 // Warps: 0 = TMA producer (both CTAs), 1 = MMA issuer (leader CTA) / forwarder (peer) + TMEM alloc, 2..9 = epilogue.
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "sm100_ptx.cuh"
 #include "svsk_common.cuh"
@@ -45,8 +44,6 @@ struct Diffnet3Args {
   const float* stepbias;
   const float* bout;
   int B, T, C, H, dilation, sb_stride, init_skip, write_x, nentries;
-  unsigned long long* dbg;
-  int dbg_flags;  // profiling ablations: 4 = skip MMAs, 8 = skip TMA loads after the first ring fill
 };
 
 struct __align__(8) Diffnet3Barriers {
@@ -87,9 +84,6 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
   const int b = blockIdx.y;
   const int t_cta0 = (blockIdx.x >> 1) * 256 + (int)rank * 128;  // first frame of this CTA's 128 TMEM lanes
   const int w_row0 = (int)rank * 128;                             // this CTA's half of a 256-row weight block
-  unsigned long long* dbg = a.dbg ? a.dbg + (size_t)(blockIdx.y * gridDim.x + blockIdx.x) * 32 : nullptr;
-#define SVSK_STAMP(i) do { if (dbg) dbg[i] = clock64(); } while (0)
-  if (threadIdx.x == 0) SVSK_STAMP(0);
 
   const int n_a = HB * NB;                       // phase-A ring entries
   const int n_total = n_a + NB * 3 * CB + NB * KB2;
@@ -128,7 +122,6 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
     }
     // Programmatic dependent launch: activations (conditioner tiles, then x = the previous layer's output) from here.
     asm volatile("griddepcontrol.wait;" ::: "memory");
-    SVSK_STAMP(21);
     for (int hb = 0; hb < HB; ++hb) {
       ptx::mbar_arrive_expect_tx(&bars->cd_full[hb], k3Tile);
       ptx::tma_load_3d(g_smem + hb * k3Tile, &tm_cond, &bars->cd_full[hb], hb * 64, t_cta0, b);
@@ -153,17 +146,9 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
     if (lane == 0) {
       int s = pre_issued % a.nentries;
       uint32_t ph = (pre_issued == a.nentries) ? 1u : 0u;
-      long long acc_pe = 0;
       for (int e = pre_issued; e < n_total; ++e) {
-        const long long c_0 = dbg ? clock64() : 0ll;
         ptx::mbar_wait(&bars->empty[s], ph ^ 1);
-        if (dbg) acc_pe += clock64() - c_0;
         uint8_t* dst = ring + s * k3Tile;
-        if (a.dbg_flags & 8) {  // profiling: no loads after the first ring fill
-          ptx::mbar_arrive(&bars->full[s]);
-          if (++s == a.nentries) { s = 0; ph ^= 1; }
-          continue;
-        }
         ptx::mbar_arrive_expect_tx(&bars->full[s], k3Tile);
         if (e < n_a) {
           ptx::tma_load_2d(dst, &tm_w1, &bars->full[s], (3 * CB + e / NB) * 64, (e % NB) * 256 + w_row0);
@@ -176,8 +161,6 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
         }
         if (++s == a.nentries) { s = 0; ph ^= 1; }
       }
-      SVSK_STAMP(1);
-      if (dbg) dbg[16] = acc_pe;  // producer: cycles waiting for free ring entries
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer: one thread of the leader CTA
@@ -185,34 +168,26 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
       const uint32_t idesc = ptx::umma_idesc_bf16_f32(256, 256);
       const uint32_t ring_lo = ptx::umma_desc_lo(ptx::smem_u32(ring)), g_lo = ptx::umma_desc_lo(ptx::smem_u32(g_smem));
       const uint32_t xw_lo = ptx::umma_desc_lo(ptx::smem_u32(xw_smem));
-      const bool mma_on = !(a.dbg_flags & 4);
       int s = 0;
       uint32_t ph = 0;
       bool ready = false;  // the barrier of ring entry (s, ph) was already seen complete by the previous group's probe
-      long long acc_wf = 0;
       // An mbarrier wait whose result is needed at once stalls this thread ~160 cycles even on a long-completed phase
       // (tools/ubench_umma.py): every MMA group therefore probes the NEXT entry's barrier while its MMAs are issued.
-#define SVSK_WAIT_ENTRY()                                        \
-  do {                                                           \
-    if (!ready) {                                                \
-      const long long c_0 = dbg ? clock64() : 0ll;               \
-      ptx::mbar_wait(&bars->full[s], ph);                        \
-      if (dbg) acc_wf += clock64() - c_0;                        \
-    }                                                            \
-    ready = false;                                               \
-    ptx::tc_fence_after();                                       \
+#define SVSK_WAIT_ENTRY()                       \
+  do {                                          \
+    if (!ready) ptx::mbar_wait(&bars->full[s], ph); \
+    ready = false;                              \
+    ptx::tc_fence_after();                      \
   } while (0)
 #define SVSK_NEXT_ENTRY() do { if (++s == a.nentries) { s = 0; ph ^= 1; } } while (0)
 #define SVSK_ISSUE4(dcol, alo, blo, acc0)                                                                          \
   do {                                                                                                             \
     const int sn = (s + 1 == a.nentries) ? 0 : s + 1;                                                              \
-    if (mma_on) ready = ptx::umma2_bf16_x4_probe(tmem + (dcol), alo, blo, idesc, acc0, 4, &bars->full[sn], sn ? ph : ph ^ 1); \
+    ready = ptx::umma2_bf16_x4_probe(tmem + (dcol), alo, blo, idesc, acc0, 4, &bars->full[sn], sn ? ph : ph ^ 1); \
   } while (0)
       // ---- phase A: conditioner k-blocks out of the (future) G buffer, both output blocks per tile
-      SVSK_STAMP(22);
       for (int hb = 0; hb < HB; ++hb) {
         ptx::mbar_wait(&bars->cd_full[hb], 0);
-        if (hb == 0) SVSK_STAMP(23);
         const uint32_t a_lo = g_lo + hb * (k3Tile >> 4);
         for (int j = 0; j < NB; ++j) {
           SVSK_WAIT_ENTRY();
@@ -221,11 +196,9 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
           SVSK_NEXT_ENTRY();
         }
       }
-      SVSK_STAMP(19);
       // ---- phase B: the three taps out of the resident window
       ptx::mbar_wait(&bars->xw_full, 0);
       ptx::tc_fence_after();
-      SVSK_STAMP(20);
       for (int j = 0; j < NB; ++j) {
         for (int jt = 0; jt < 3; ++jt) {
           const uint32_t row_lo = xw_lo + (uint32_t)(k3Halo + (jt - 1) * a.dilation) * (128u >> 4);
@@ -237,13 +210,10 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
           }
         }
         ptx::umma_commit2_mc(&bars->d1_full[j], 3);
-        SVSK_STAMP(2 + j);
       }
-      if (dbg) dbg[17] = acc_wf;  // GEMM1: blocking waits for ring entries (probe misses)
       // ---- phase C: GEMM2
       ptx::mbar_wait(&bars->g_ready, 0);
       ptx::tc_fence_after();
-      SVSK_STAMP(4);
       for (int j = 0; j < NB; ++j) {
         for (int kb = 0; kb < KB2; ++kb) {
           SVSK_WAIT_ENTRY();
@@ -252,7 +222,6 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
           SVSK_NEXT_ENTRY();
         }
         ptx::umma_commit2_mc(&bars->d2_full[j], 3);
-        SVSK_STAMP(5 + j);
       }
 #undef SVSK_WAIT_ENTRY
 #undef SVSK_NEXT_ENTRY
@@ -284,7 +253,6 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
     const uint32_t tlane = (uint32_t)(q * 32) << 16;
     const bool has_l = (t - a.dilation) >= 0, has_r = (t + a.dilation) < T;
     const bool warp_edge = __any_sync(0xffffffffu, !has_l || !has_r);  // warp-uniform: the bias correction is a branch
-    const bool stamp = (warp == 2 && lane == 0);
 
     // per-column biases -> smem (off the path to the first MMA): sb_full = centre + left + right tap terms, what an
     // interior frame gets.  The step-bias rows may come from the preceding kernel: wait for it first.
@@ -305,7 +273,6 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
     for (int j = 0; j < NB; ++j) {
       ptx::mbar_wait(&bars->d1_full[j], 0);
       ptx::tc_fence_after();
-      if (stamp) SVSK_STAMP(7 + 2 * j);
       uint32_t rgb[2][16], rfb[2][16];
       ptx::tmem_ld16(tmem + tlane + j * 256 + 16 * sub, rgb[0]);
       ptx::tmem_ld16(tmem + tlane + j * 256 + 128 + 16 * sub, rfb[0]);
@@ -357,13 +324,11 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
         ptx::st_shared_v4(gk + ptx::sw128_offset((uint32_t)row, ch16 + 1), ptx::pack_bf16(z[8], z[9]),
                           ptx::pack_bf16(z[10], z[11]), ptx::pack_bf16(z[12], z[13]), ptx::pack_bf16(z[14], z[15]));
       }
-      if (stamp) SVSK_STAMP(8 + 2 * j);
     }
     ptx::tc_fence_before();
     ptx::fence_proxy_async_smem();  // G (generic-proxy stores) -> visible to the tensor cores' async proxy
     if (rank == 0) ptx::mbar_arrive(&bars->g_ready);
     else ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(&bars->g_ready), 0));
-    if (stamp) SVSK_STAMP(11);
 
     // ---- epilogue 2: residual -> in place over the window's centre rows -> TMA store ; skip -> fp32 slabs -> TMA
     //      reduce-add (or plain store on the first layer)
@@ -373,7 +338,6 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
     for (int j = 0; j < NB; ++j) {
       ptx::mbar_wait(&bars->d2_full[j], 0);
       ptx::tc_fence_after();
-      if (stamp) SVSK_STAMP(12 + j);
       const int res_cols = min(max(C - j * 256, 0), 256);  // residual columns in this 256-column block
       if (res_cols > 0 && a.write_x) {
         ptx::mbar_wait(&bars->xw_full, 0);  // (long since complete) makes the TMA-written window visible to this thread
@@ -450,15 +414,12 @@ diffnet_block3_kernel(const __grid_constant__ CUtensorMap tm_xw, const __grid_co
       }
     }
     if (elected) ptx::bulk_wait_read_all();  // smem may be released; global visibility comes with grid completion
-    if (stamp) SVSK_STAMP(14);
   }
 
   ptx::tc_fence_before();
   __syncthreads();
   ptx::cluster_sync_all();  // the peer's smem / TMEM are in use by the leader's MMAs until here
   if (warp == 1) ptx::tmem_dealloc2(tmem, k3TmemCols);
-  if (threadIdx.x == 0) SVSK_STAMP(15);
-#undef SVSK_STAMP
 }
 
 }  // namespace svsk
@@ -544,10 +505,6 @@ extern "C" int svsk_diffnet_block3_bf16(const svsk_diffnet_block_params* pp, voi
   a.init_skip = p.init_skip;
   a.write_x = p.write_x;
   a.nentries = nentries;
-  a.dbg = nullptr;
-  a.dbg_flags = 0;
-  if (const char* e = getenv("SVSK_DIFFNET_TIMELINE")) a.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
-  if (const char* e = getenv("SVSK_DIFFNET_ABLATE")) a.dbg_flags = atoi(e);
 
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(2 * ceil_div(p.T, 256), p.B);
@@ -562,7 +519,7 @@ extern "C" int svsk_diffnet_block3_bf16(const svsk_diffnet_block_params* pp, voi
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = getenv("SVSK_NO_PDL") ? 1 : 2;
+  cfg.numAttrs = 2;
   cudaError_t e = cudaLaunchKernelEx(&cfg, diffnet_block3_kernel, tm_xw, tm_cond, tm_w1, tm_wout, tm_xout, tm_skip, a);
   if (e != cudaSuccess) return fail((int)e, "diffnet_block3_bf16: launch: %s", cudaGetErrorString(e));
   return check_launch("diffnet_block3_bf16");

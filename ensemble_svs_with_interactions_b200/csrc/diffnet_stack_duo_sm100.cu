@@ -51,9 +51,7 @@ struct DuoArgs {
   int* flags;             // [B * tiles_per_track] layers published per 128-frame tile; zero at launch
   int B, T, H, L, sb_batch_stride, sb_layer_stride, init_skip, nentries, tiles_per_track;
   int dilation[kDMaxLayers];
-  unsigned long long* dbg;  // SVSK_DIFFNET_TIMELINE: [CTA][64] clock64 stamps of layer kDStampLayer (32 per slot), leader CTAs
 };
-constexpr int kDStampLayer = 4;
 
 struct __align__(8) DuoSlotBarriers {
   uint64_t cd_full[2];   // conditioner tile hb of this layer landed (leader: in both CTAs)
@@ -90,9 +88,9 @@ __device__ __forceinline__ void duo_st_release_gpu(int* p, int v) {
 }
 __device__ __forceinline__ void duo_fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 
-// kHB = H / 64 (1 or 2) and kProf (clock64 stamps) are compile-time: the single-thread roles pay for every run-time loop
-// bound and branch (diffnet_stack_sm100.cu, DESIGN §4 item 17).
-template <int kHB, bool kProf>
+// kHB = H / 64 (1 or 2) is compile-time: the single-thread roles pay for every run-time loop bound and branch
+// (diffnet_stack_sm100.cu, DESIGN §4 item 17).
+template <int kHB>
 __global__ void __launch_bounds__(kDThreads, 1)
 diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_constant__ CUtensorMap tm_e0,
                          const __grid_constant__ CUtensorMap tm_e1, const __grid_constant__ CUtensorMap tm_cond,
@@ -123,9 +121,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
   const int vp0 = pair, vp1 = pair + npairs;
   const bool live1 = vp1 * 256 < T;  // (slot 0 is always live: the grid has ceil(n256 / 2) pairs per track)
   const int n_slots = live1 ? 2 : 1;
-  unsigned long long* dbg = (kProf && a.dbg) ? a.dbg + (size_t)(blockIdx.y * gridDim.x + blockIdx.x) * 64 : nullptr;
-#define DUO_STAMP(l_, u_, i_) do { if (kProf && dbg && (l_) == kDStampLayer) dbg[(u_) * 32 + (i_)] = clock64(); } while (0)
-  if (kProf && dbg && threadIdx.x == 0) dbg[63] = clock64();
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tm_xw0);
@@ -211,7 +206,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
         const CUtensorMap* tm_e = pp ? &tm_e1 : &tm_e0;
         // publish the first / last 8 rows of layer l-1's output (the epilogue has written them in place)
         ptx::mbar_wait(&sb->xe_ready, pp);
-        DUO_STAMP(l, u, 0);   // layer l-1's centre rows written (activation producer)
         for (int cb = 0; cb < kDCB; ++cb) {
           uint8_t* centre = xw_smem + cb * kDWinBytes + kDHalo * 128;
           ptx::tma_store_3d(tm_e, centre, cb * 64, t_cta0, b);
@@ -219,10 +213,8 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
         }
         ptx::bulk_commit_group();
         ptx::bulk_wait_all();  // the stores are complete (not merely read out of shared memory)
-        DUO_STAMP(l, u, 1);   // edge rows stored
         duo_fence_proxy_async_global();
         duo_st_release_gpu(a.flags + tile_idx, l);
-        DUO_STAMP(l, u, 2);   // flag published
         // halo rows of layer l's input: the neighbours' edge rows of layer l-1's output
         for (uint32_t spin = 0;; ++spin) {  // both flags per round trip, relaxed; one acquire fence at the end
           const int fl = has_left ? duo_ld_relaxed_gpu(a.flags + tile_idx - 1) : l;
@@ -230,10 +222,8 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
           if (fl >= l && fr >= l) break;
           if (spin > (1u << 21)) __trap();
         }
-        DUO_STAMP(l, u, 3);   // neighbours' flags seen
         asm volatile("fence.acq_rel.gpu;" ::: "memory");
         duo_fence_proxy_async_global();
-        DUO_STAMP(l, u, 4);   // fences done, halo loads issued next
         // (Measured and not kept: fetching the 4 KB of halo rows with ld.global.cg by the whole warp + st.shared instead of
         // TMA, which saves the second fence — 141.8 vs 135.4 us per launch: an L2 round trip under this load is ~2 k cycles
         // whoever issues it.)
@@ -245,7 +235,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
         }
         // conditioner tiles of layer l, once the G buffer is free again
         ptx::mbar_wait(&sb->gc_free, pp);
-        DUO_STAMP(l, u, 5);   // G buffer free: conditioner tiles requested
         for (int hb = 0; hb < HB; ++hb) {
           ptx::mbar_arrive_expect_tx(&sb->cd_full[hb], kDTile);
           ptx::tma_load_3d(g_smem + hb * kDTile, &tm_cond, &sb->cd_full[hb], hb * 64, t_cta0, b);
@@ -291,7 +280,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
             ptx::mbar_wait(&sb->d2_drained, pp);  // ... and the accumulator read out (residual and skip halves)
           }
           ptx::tc_fence_after();
-          DUO_STAMP(l, u, 8);   // MMA thread: centre rows + accumulator ready
           for (int cb = 0; cb < kDCB; ++cb) {
             DUO_WAIT_ENTRY();
             DUO_ISSUE4(tb, xw_lo + cb * (kDWinBytes >> 4) + kDHalo * 8, cb != 0);
@@ -300,7 +288,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
             ptx::mbar_wait(&sb->xw_full, pl);
             ptx::tc_fence_after();
           }
-          DUO_STAMP(l, u, 9);   // MMA thread: halo rows landed
           for (int jt = 0; jt < 3; jt += 2) {
             const uint32_t row_lo = xw_lo + (uint32_t)(kDHalo + (jt - 1) * d) * 8u;
             for (int cb = 0; cb < kDCB; ++cb) {
@@ -315,7 +302,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
             DUO_ISSUE4(tb, g_lo + hb * (kDTile >> 4), 1);
           }
           ptx::umma_commit2_mc(&sb->d1_full, pair_mask);
-          DUO_STAMP(l, u, 10);  // MMA thread: GEMM1 issued
         }
         for (int u = 0; u < n_slots; ++u) {  // ---- GEMM2 of slot u
           DuoSlotBarriers* sb = &bars->s[u];
@@ -323,13 +309,11 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
           const uint32_t tb = (uint32_t)u * 256u;
           ptx::mbar_wait(&sb->g_ready, pl);
           ptx::tc_fence_after();
-          DUO_STAMP(l, u, 11);  // MMA thread: G ready
           for (int kb = 0; kb < kDKB2; ++kb) {
             DUO_WAIT_ENTRY();
             DUO_ISSUE4(tb, g_lo + kb * (kDTile >> 4), kb != 0);
           }
           ptx::umma_commit2_mc(&sb->d2_full, pair_mask);
-          DUO_STAMP(l, u, 12);  // MMA thread: GEMM2 issued
         }
       }
 #undef DUO_WAIT_ENTRY
@@ -414,7 +398,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
         // ---- epilogue 1: gating -> G  (accumulator columns [0,128) gate, [128,256) filter)
         ptx::mbar_wait(&sb->d1_full, pl);
         ptx::tc_fence_after();
-        if (et == 0) DUO_STAMP(l, u, 16);  // epilogue: D1 complete
         {
           uint32_t rgb[2][16], rfb[2][16];
           ptx::tmem_ld16(tcol + 16 * sub, rgb[0]);
@@ -470,13 +453,11 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
         ptx::tc_fence_before();
         ptx::fence_proxy_async_smem();  // G (generic-proxy stores) -> visible to the tensor cores' async proxy
         ptx::mbar_arrive_cluster(gr_leader);
-        if (et == 0) DUO_STAMP(l, u, 17);  // epilogue: gated (this thread)
 
         // ---- epilogue 2: residual (columns [0,128)) -> in place over the window's centre rows (the next layer's centre
         //      tap); skip (columns [128,256)) -> fp32 slabs in the G buffer -> TMA reduce-add (plain store on layer 0)
         ptx::mbar_wait(&sb->d2_full, pl);
         ptx::tc_fence_after();
-        if (et == 0) DUO_STAMP(l, u, 18);  // epilogue: D2 complete
         if (!last) {
           if (l == 0) ptx::mbar_wait(&sb->xw_full, 0);  // (long complete) makes the TMA-written window visible here
           uint32_t rr[2][16];
@@ -510,7 +491,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
           ptx::fence_proxy_async_smem();
           ptx::mbar_arrive_cluster(xc_leader);  // the next layer's centre tap is waiting for this
           ptx::mbar_arrive(&sb->xe_ready);
-          if (et == 0) DUO_STAMP(l, u, 19);  // epilogue: residual written (this thread)
         }
         // skip: 4 slabs of 32 columns (one 128-byte fp32 row per frame); the kDW warps of a lane quarter alternate slabs,
         // each stages its 32 rows of a slab in its own 4 KB piece of a G tile and issues its own TMA reduce-add
@@ -555,7 +535,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
             ptx::mbar_arrive(&sb->gc_free);
           }
         }
-        if (et == 0) DUO_STAMP(l, u, 20);  // epilogue: skip slabs handed to the TMA unit
         ptx::tc_fence_before();
         ptx::mbar_arrive_cluster(dr_leader);
         // the bias arrays are rewritten at the top of the next layer: every epilogue thread of the slot must be done with them
@@ -568,8 +547,6 @@ diffnet_stack_duo_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __gri
   __syncthreads();
   ptx::cluster_sync_all();  // the peer's smem / TMEM are in use by the leader's MMAs until here
   if (warp == 1) ptx::tmem_dealloc2(tmem, 512);
-  if (kProf && dbg && threadIdx.x == 0) dbg[62] = clock64();
-#undef DUO_STAMP
 }
 
 static int duo_smem(int H, int* nentries_out) {
@@ -583,9 +560,8 @@ static int duo_smem(int H, int* nentries_out) {
 
 using DuoKernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap,
                              DuoArgs);
-static DuoKernelFn duo_kernel_variant(int hb, bool prof) {
-  if (hb == 1) return prof ? diffnet_stack_duo_kernel<1, true> : diffnet_stack_duo_kernel<1, false>;
-  return prof ? diffnet_stack_duo_kernel<2, true> : diffnet_stack_duo_kernel<2, false>;
+static DuoKernelFn duo_kernel_variant(int hb) {
+  return hb == 1 ? diffnet_stack_duo_kernel<1> : diffnet_stack_duo_kernel<2>;
 }
 
 bool diffnet_stack_duo_applies(int C, int H) {
@@ -600,8 +576,8 @@ static int duo_prepare(int* nentries, int* smem_bytes) {
   static bool attr_set[64] = {false};
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
     cudaError_t e = cudaSuccess;
-    for (int v = 0; v < 4 && e == cudaSuccess; ++v)
-      e = cudaFuncSetAttribute(duo_kernel_variant(1 + (v & 1), (v & 2) != 0), cudaFuncAttributeMaxDynamicSharedMemorySize, kDSmemLimit);
+    for (int hb = 1; hb <= 2 && e == cudaSuccess; ++hb)
+      e = cudaFuncSetAttribute(duo_kernel_variant(hb), cudaFuncAttributeMaxDynamicSharedMemorySize, kDSmemLimit);
     if (e != cudaSuccess) return fail((int)e, "diffnet_stack_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
   }
@@ -620,11 +596,11 @@ static void duo_launch_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* attr
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   // cooperative: the grid starts only when ALL its CTAs can be resident at once — the neighbour hand-shakes need it.
-  // A track that is a single CTA pair has no neighbour: plain launch (keeps small calls replayable by ncu).
+  // A track that is a single CTA pair has no neighbour: plain launch.
   attr[1].id = cudaLaunchAttributeCooperative;
   attr[1].val.cooperative = 1;
   cfg->attrs = attr;
-  cfg->numAttrs = (n256 <= 2 || getenv("SVSK_STACK_NO_COOPERATIVE")) ? 1 : 2;
+  cfg->numAttrs = n256 <= 2 ? 1 : 2;
 }
 
 // 1 / 0: all CTA pairs of B tracks x T frames fit the device at once / do not
@@ -635,7 +611,7 @@ int diffnet_stack_duo_fits(int B, int T) {
   cudaLaunchAttribute attr[2];
   duo_launch_config(&cfg, attr, B, T, smem_bytes, nullptr);
   int max_clusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&max_clusters, duo_kernel_variant(2, false), &cfg) != cudaSuccess) {
+  if (cudaOccupancyMaxActiveClusters(&max_clusters, duo_kernel_variant(2), &cfg) != cudaSuccess) {
     cudaGetLastError();
     return 0;
   }
@@ -650,7 +626,7 @@ int diffnet_stack_duo_launch(const svsk_diffnet_stack_params& p, void* stream) {
   cudaLaunchAttribute attr[2];
   duo_launch_config(&cfg, attr, p.B, p.T, smem_bytes, stream);
   int max_clusters = 0;
-  cudaError_t oe = cudaOccupancyMaxActiveClusters(&max_clusters, duo_kernel_variant(2, false), &cfg);
+  cudaError_t oe = cudaOccupancyMaxActiveClusters(&max_clusters, duo_kernel_variant(2), &cfg);
   if (oe != cudaSuccess) return fail((int)oe, "diffnet_stack_bf16: cudaOccupancyMaxActiveClusters: %s", cudaGetErrorString(oe));
   const int n_clusters = (int)(cfg.gridDim.x / 2) * p.B;
   SVSK_REQUIRE(n_clusters <= max_clusters, SVSK_E_ARG,
@@ -701,12 +677,10 @@ int diffnet_stack_duo_launch(const svsk_diffnet_stack_params& p, void* stream) {
   a.nentries = nentries;
   a.tiles_per_track = 2 * ceil_div(p.T, 256);
   for (int l = 0; l < kDMaxLayers; ++l) a.dilation[l] = l < p.L ? p.dilation[l] : 1;
-  a.dbg = nullptr;
-  if (const char* e = getenv("SVSK_DIFFNET_TIMELINE")) a.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
 
   cudaError_t e = cudaMemsetAsync(p.flags, 0, sizeof(int) * (size_t)p.B * a.tiles_per_track, as_stream(stream));
   if (e != cudaSuccess) return fail((int)e, "diffnet_stack_bf16: flag reset: %s", cudaGetErrorString(e));
-  e = cudaLaunchKernelEx(&cfg, duo_kernel_variant(p.H / 64, a.dbg != nullptr), tm_xw0, tm_e0, tm_e1, tm_cond, tm_w1, tm_wout, tm_skip, a);
+  e = cudaLaunchKernelEx(&cfg, duo_kernel_variant(p.H / 64), tm_xw0, tm_e0, tm_e1, tm_cond, tm_w1, tm_wout, tm_skip, a);
   if (e != cudaSuccess) return fail((int)e, "diffnet_stack_bf16: launch: %s", cudaGetErrorString(e));
   return check_launch("diffnet_stack_bf16 (two tiles per CTA pair)");
 }

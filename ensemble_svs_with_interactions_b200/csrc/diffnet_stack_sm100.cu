@@ -86,12 +86,12 @@ struct DiffnetStackArgs {
   int* flags;             // [B * tiles_per_track] layers published per tile; zero at launch
   int dsmem_halo;         // 1: one cluster per track, halo rows through distributed shared memory; 0: through global memory
   int B, T, C, H, L, sb_batch_stride, sb_layer_stride, init_skip, nentries, tiles_per_track;
-  // C = 128 only (one 256-column output block): the accumulator alternates between the two halves of TMEM from layer to
+  // C = 128 (one 256-column output block): the accumulator alternates between the two halves of TMEM from layer to
   // layer, so that a layer's GEMM1 does not wait for the previous layer's skip columns to be read out (they share the
   // block with the residual columns: ~5 k of a 19.4 k-cycle layer, profiles/r02j_stack_c128_timeline.log), and the
   // conditioner tiles — the same for every layer — stay in their own shared-memory tiles instead of being reloaded into
   // the G buffer once the skip epilogue has released it (3.8 k cycles into the layer).
-  int pingpong, cond_resident;
+  int cond_resident;
   // Measured in round 2 and removed (it was a run-time switch inside the single-thread roles' loops, see the template
   // parameters of the kernel): the conditioner k-blocks issued BEFORE block 0's side taps in global-memory halo mode, on the
   // idea that the halo rows land ~9.5 k cycles after the previous residual epilogue there and the conditioner MMAs need
@@ -108,7 +108,6 @@ struct DiffnetStackArgs {
   // cluster-wide multicast: 366 us with half the ring misses but 8x the L2 reads.  Their run-time switches cost the
   // single-thread roles more than any of them gained.
   int dilation[kSMaxLayers];
-  unsigned long long* dbg;
 };
 
 struct __align__(8) DiffnetStackBarriers {
@@ -173,9 +172,9 @@ __device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) 
 // kUseP: the conditioner projection is precomputed (DiffnetStackArgs::use_p) — a compile-time switch, so that the instantiation without it
 // keeps the register allocation it had before the projection's prefetch registers existed (168 registers are the cap at
 // 352 threads; a handful of spilled loop invariants cost the MMA-issuing thread 5 % of the launch).
-// kDsmem (one cluster per track, halo rows through distributed shared memory) and kProf (clock64 stamps for tools/bench_stack.py)
-// are compile-time for the same reason: the single-thread roles pay for every run-time branch in their loops.
-template <bool kUseP, bool kDsmem, bool kProf, int kC>
+// kDsmem (one cluster per track, halo rows through distributed shared memory) is compile-time for the same reason: the
+// single-thread roles pay for every run-time branch in their loops.
+template <bool kUseP, bool kDsmem, int kC>
 __global__ void __launch_bounds__(kSThreads, 1)
 diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_constant__ CUtensorMap tm_e0,
                      const __grid_constant__ CUtensorMap tm_e1, const __grid_constant__ CUtensorMap tm_cond,
@@ -227,10 +226,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
   const int w_row0 = (int)rank * 128;                             // this CTA's half of a 256-row weight block
   const int n_layer = NB * (3 * CB + HB) + NB * KB2;              // ring entries per layer
   const int n_total = L * n_layer;
-  unsigned long long* dbg = (kProf && a.dbg) ? a.dbg + (size_t)(blockIdx.y * gridDim.x + blockIdx.x) * 32 : nullptr;
-#define SVSK_STAMP(i) do { if (kProf && dbg) dbg[i] = clock64(); } while (0)
-  if (threadIdx.x == 0) SVSK_STAMP(0);
-
   int pre_issued = 0;  // weight producer: entries issued before the CTA-wide sync
 
   if (warp == 0 && lane == 0) {
@@ -348,7 +343,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
         }
         // publish the first / last 8 rows of layer l-1's output (the epilogue has written them in place)
         ptx::mbar_wait(&bars->xe_ready, pp);
-        if (l == 1) SVSK_STAMP(9);
         for (int cb = 0; cb < CB; ++cb) {
           uint8_t* centre = xw_smem + cb * kSWinBytes + kSHalo * 128;
           ptx::tma_store_3d(tm_e, centre, cb * 64, t_cta0, b);
@@ -356,10 +350,8 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
         }
         ptx::bulk_commit_group();
         ptx::bulk_wait_all();  // the stores are complete (not merely read out of shared memory)
-        if (l == 1) SVSK_STAMP(10);
         fence_proxy_async_global();
         st_release_gpu(a.flags + tile_idx, l);
-        if (l == 1) SVSK_STAMP(11);
         // halo rows of layer l's input: the neighbours' edge rows of layer l-1's output
         for (uint32_t spin = 0;; ++spin) {  // both flags per round trip, relaxed; one acquire fence at the end
           const int fl = has_left ? ld_relaxed_gpu(a.flags + tile_idx - 1) : l;
@@ -368,7 +360,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
           if (spin > (1u << 21)) __trap();
         }
         asm volatile("fence.acq_rel.gpu;" ::: "memory");
-        if (l == 1) SVSK_STAMP(12);
         fence_proxy_async_global();
         ptx::mbar_arrive_expect_tx(&bars->xw_full, 2 * CB * kSHaloBytes);
         for (int cb = 0; cb < CB; ++cb) {
@@ -376,11 +367,9 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
           ptx::tma_load_3d(tile, tm_e, &bars->xw_full, cb * 64, t_cta0 - kSHalo, b);
           ptx::tma_load_3d(tile + (kSHalo + 128) * 128, tm_e, &bars->xw_full, cb * 64, t_cta0 + 128, b);
         }
-        if (l == 1) SVSK_STAMP(13);
         // conditioner tiles of layer l, once the G buffer is free again
         if ((kC == 128 && a.cond_resident) && !kUseP) continue;
         ptx::mbar_wait(&bars->gc_free, pp);
-        if (l == 1) SVSK_STAMP(14);
         for (int hb = 0; hb < HB; ++hb) {
           ptx::mbar_arrive_expect_tx(&bars->cd_full[hb], kSTile);
           ptx::tma_load_3d(g_smem + hb * kSTile, &tm_cond, &bars->cd_full[hb], hb * 64, t_cta0, b);
@@ -400,16 +389,11 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
       // CTAs that write halo rows this pair's GEMM1 reads: the pair itself and the outer neighbour on either side
       const uint16_t halo_mask = (uint16_t)(pair_mask | (lead > 0 ? 1u << (lead - 1) : 0u) | (lead + 2 < csize ? 1u << (lead + 2) : 0u));
       bool ready = false;  // the barrier of ring entry (s, ph) was already seen complete by the previous group's probe
-      long long acc_wait = 0, n_miss = 0;
       // An mbarrier wait whose result is needed at once stalls this thread ~160 cycles even on a long-completed phase
       // (tools/ubench_umma.py): every MMA group therefore probes the NEXT entry's barrier while its MMAs are issued.
 #define SVSK_WAIT_ENTRY()                                 \
   do {                                                    \
-    if (!ready) {                                         \
-      const long long c_0 = (kProf && dbg) ? clock64() : 0ll; \
-      SVSK_STACK_ISSUER_WAIT(&bars->full[s], ph);         \
-      if (kProf && dbg) { acc_wait += clock64() - c_0; ++n_miss; } \
-    }                                                     \
+    if (!ready) SVSK_STACK_ISSUER_WAIT(&bars->full[s], ph); \
     ready = false;                                        \
     ptx::tc_fence_after();                                \
   } while (0)
@@ -424,24 +408,20 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
       for (int l = 0; l < L; ++l) {
         const uint32_t pl = (uint32_t)l & 1u, pp = pl ^ 1u;
         const int d = a.dilation[l];
-        const uint32_t tb = (kC == 128 && a.pingpong) ? pl * 256u : 0u;  // TMEM column base of this layer's accumulator block(s)
+        const uint32_t tb = kC == 128 ? pl * 256u : 0u;  // TMEM column base of this layer's accumulator block(s)
         // ---- centre tap, block 0
         if (l == 0) {
           ptx::mbar_wait(&bars->xw_full, 0);
         } else {
           ptx::mbar_wait(&bars->xc_ready, pp);      // centre rows rewritten in place by the previous layer's epilogue
-          if (l == 2) SVSK_STAMP(27);
           // and the accumulator block read out: by the previous layer — or, alternating halves, by the one before it
           // (barrier pl completes once every two layers)
-          if (!(kC == 128 && a.pingpong)) ptx::mbar_wait(&bars->d2_drained[0], pp);
+          if (kC != 128) ptx::mbar_wait(&bars->d2_drained[0], pp);
           else if (l >= 2) ptx::mbar_wait(&bars->d2_drained[pl], (uint32_t)((l - 2) >> 1) & 1u);
         }
         ptx::tc_fence_after();
-        if (l == 1) SVSK_STAMP(2);
-        if (l == 2) SVSK_STAMP(18);
         for (int cb = 0; cb < CB; ++cb) {
           SVSK_WAIT_ENTRY();
-          if (l == 2 && cb == 0) SVSK_STAMP(19);
           SVSK_ISSUE4(0, xw_lo + cb * (kSWinBytes >> 4) + kSHalo * 8, ring_lo + s * (kSTile >> 4), cb != 0);
         }
         {
@@ -452,7 +432,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
               else ptx::mbar_wait(&bars->xw_full, pl);
               ptx::tc_fence_after();
             }
-            if (l == 1) SVSK_STAMP(3);
             for (int jt = 0; jt < 3; jt += 2) {
               const uint32_t row_lo = xw_lo + (uint32_t)(kSHalo + (jt - 1) * d) * 8u;
               for (int cb = 0; cb < CB; ++cb) {
@@ -467,7 +446,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
               if (l == 0 || !(kC == 128 && a.cond_resident)) ptx::mbar_wait(&bars->cd_full[hb], pl);
               if (hb == 0 && l != 0 && NB > 1) ptx::mbar_wait(&bars->d2_drained[1], pp);
               ptx::tc_fence_after();
-              if (l == 1 && hb == 0) SVSK_STAMP(4);
               const uint32_t a_lo = cond_lo + hb * (kSTile >> 4);
               for (int j = 0; j < NB; ++j) {
                 SVSK_WAIT_ENTRY();
@@ -477,7 +455,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
           }
         }
         ptx::umma_commit2_mc(&bars->d1_full[0], pair_mask);
-        if (l == 1) SVSK_STAMP(5);
         // ---- all taps, blocks 1..
         for (int j = 1; j < NB; ++j) {
           if (HB == 0 && l != 0) {  // no conditioner k-blocks ahead of these: the block's first MMAs overwrite the accumulator
@@ -495,7 +472,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
         }
         // GEMM1 of this layer has read the window for the last time: the neighbouring tiles may overwrite its halo rows
         if (kDsmem) ptx::umma_commit2_mc(&bars->halo_free, halo_mask);
-        if (l == 1) SVSK_STAMP(6);
         // ---- GEMM2: G tiles of gating block 0 first (its k-blocks of output block 0 run while block 1 is still gated)
         ptx::mbar_wait(&bars->g_ready[0], pl);
         ptx::tc_fence_after();
@@ -504,16 +480,13 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
             if (NB > 1 && j == 0 && kb == KB2 / 2) {  // G tiles KB2/2.. come from gating block 1
               ptx::mbar_wait(&bars->g_ready[1], pl);
               ptx::tc_fence_after();
-              if (l == 1) SVSK_STAMP(7);
             }
             SVSK_WAIT_ENTRY();
             SVSK_ISSUE4(j * 256, g_lo + kb * (kSTile >> 4), ring_lo + s * (kSTile >> 4), kb != 0);
           }
           ptx::umma_commit2_mc(&bars->d2_full[j], pair_mask);
         }
-        if (l == 1) SVSK_STAMP(8);
       }
-      if (kProf && dbg) { dbg[16] = acc_wait; dbg[17] = n_miss; }  // blocking waits for ring entries: cycles, count
 #undef SVSK_WAIT_ENTRY
 #undef SVSK_NEXT_ENTRY
 #undef SVSK_ISSUE4
@@ -569,7 +542,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
     const int t = t_cta0 + row;
     const uint32_t tlane = (uint32_t)(q * 32) << 16;
     const bool in_seq = t < T;
-    const bool elected = (warp == 2 && lane == 0);
     const uint32_t xc_leader = ptx::mapa(ptx::smem_u32(&bars->xc_ready), lead);
     const uint32_t gr_leader = ptx::mapa(ptx::smem_u32(&bars->g_ready[0]), lead);
     const uint32_t dr_leader = ptx::mapa(ptx::smem_u32(&bars->d2_drained[0]), lead);
@@ -587,10 +559,11 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
     constexpr int kChunks = 8 / kSW;  // 16-column chunks per thread and gating block
     static_assert(kChunks % 2 == 0, "the two prefetch slots alternate per chunk across blocks");
 
+    uint32_t acc_col = 0;  // C = 128: TMEM column of this layer's accumulator, alternating halves
     for (int l = 0; l < L; ++l) {
       const uint32_t pl = (uint32_t)l & 1u;
       const int d = a.dilation[l];
-      const uint32_t tcol = tmem + tlane + ((kC == 128 && a.pingpong) ? pl * 256u : 0u);   // this thread's lane, this layer's accumulator
+      const uint32_t tcol = tmem + tlane + acc_col;   // this thread's lane, this layer's accumulator
       const bool has_l = (t - d) >= 0, has_r = (t + d) < T;
       // A track's first / last d frames lack a tap's bias term.  Warp-uniform, so that the correction is a BRANCH around the
       // rare case: written per element (if (!has_l) ...) it compiled to 64 predicated-off loads + 64 adds per 16-column
@@ -624,7 +597,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
       for (int j = 0; j < NB; ++j) {
         ptx::mbar_wait(&bars->d1_full[j], pl);
         ptx::tc_fence_after();
-        if (l == 1 && elected) SVSK_STAMP(20 + 2 * j);   // 20 / 22: gating of block 0 / 1 starts
         uint32_t rgb[2][16], rfb[2][16];
         ptx::tmem_ld16(tcol + j * 256 + 16 * sub, rgb[0]);
         ptx::tmem_ld16(tcol + j * 256 + 128 + 16 * sub, rfb[0]);
@@ -703,7 +675,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
         ptx::tc_fence_before();
         ptx::fence_proxy_async_smem();  // G (generic-proxy stores) -> visible to the tensor cores' async proxy
         ptx::mbar_arrive_cluster(gr_leader + (uint32_t)j * 8u);
-        if (l == 1 && elected) SVSK_STAMP(21 + 2 * j);   // 21 / 23: ... and ends (this thread)
       }
 
       // ---- epilogue 2: residual -> in place over the window's centre rows (the next layer's centre tap) ;
@@ -711,13 +682,11 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
       for (int j = 0; j < NB; ++j) {
         ptx::mbar_wait(&bars->d2_full[j], pl);
         ptx::tc_fence_after();
-        if (l == 1 && elected) SVSK_STAMP(24 + 2 * j);  // 24: D2[0] complete, 26: D2[1] complete
         const int res_cols = min(max(C - j * 256, 0), 256);  // residual columns in this 256-column block
         bool drained_said = false;
         if (res_cols > 0 && !last) {
           if (l == 0) ptx::mbar_wait(&bars->xw_full, 0);  // (long complete) makes the TMA-written window visible here
           if (send_left || send_right) ptx::mbar_wait(&bars->halo_free, pl);  // the neighbour's GEMM1 of this layer is done
-          if (l == 1 && warp == 4 && lane == 0) SVSK_STAMP(28);               // an edge thread (row 0) starts its residual part
           const int n_res = res_cols / (16 * kSW);
           uint32_t rr[2][16];
           ptx::tmem_ld16(tcol + j * 256 + 16 * sub, rr[0]);
@@ -763,7 +732,7 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
             ptx::fence_proxy_async_smem();
             ptx::mbar_arrive_cluster(xc_leader);  // first: the next layer's centre tap is waiting for this
             ptx::mbar_arrive(&bars->xe_ready);
-            if (res_cols == 256 && !(kC == 128 && a.pingpong)) {
+            if (res_cols == 256 && kC != 128) {
               // ... and for this: the block holds no skip columns, so this thread has read all of it out of TMEM.  Said
               // BEFORE the edge threads' cluster-scope fence below (MEMBAR.ALL.GPU + L1 invalidate, ~3 k cycles in 4 of the
               // 8 epilogue warps), during which the next layer's first MMA used to wait on a condition long true:
@@ -778,9 +747,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
             }
           }
         }
-        if (l == 1 && elected && j == 0) SVSK_STAMP(25);  // residual half written
-        if (l == 1 && warp == 4 && lane == 0 && j == 0) SVSK_STAMP(9);              // ... by an edge thread (row 0; DSMEM mode)
-        if (l == 1 && warp == kSActWarp - 1 && lane == 31 && j == 0) SVSK_STAMP(10);   // ... by the last epilogue warp
         // skip part: columns [res_cols, 256) of this block in slabs of 32 (one 128-byte fp32 row per frame).  Each warp
         // owns whole slabs (the two warps of a lane quarter alternate) and its 32 rows of them: it stages them in a
         // private 2 x 4 KB piece of the G buffer and issues its own TMA reduce-add — no CTA-wide barrier, no shared
@@ -823,21 +789,19 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
               ptx::bulk_commit_group();
             }
           }
-          if (l == 1 && elected) SVSK_STAMP(29);
           if (lane == 0) {
             ptx::bulk_wait_read_all();  // this warp's slabs are read: the G buffer may take the next conditioner tiles
             ptx::mbar_arrive(&bars->gc_free);
           }
-          if (l == 1 && elected) SVSK_STAMP(30);
         }
         if (!drained_said) {
           ptx::tc_fence_before();
-          ptx::mbar_arrive_cluster(dr_leader + ((kC == 128 && a.pingpong) ? pl : (uint32_t)j) * 8u);
+          ptx::mbar_arrive_cluster(dr_leader + (kC == 128 ? pl : (uint32_t)j) * 8u);
         }
       }
       // the bias arrays are rewritten at the top of the next layer: every epilogue thread must be done reading them
       ptx::named_bar_sync(1, kSEpi);
-      if (l == 1 && elected) SVSK_STAMP(31);             // all epilogue threads of this CTA are through layer 1
+      if (kC == 128) acc_col ^= 256u;
     }
   }
 
@@ -845,8 +809,6 @@ diffnet_stack_kernel(const __grid_constant__ CUtensorMap tm_xw0, const __grid_co
   __syncthreads();
   ptx::cluster_sync_all();  // the peer's smem / TMEM are in use by the leader's MMAs until here
   if (warp == 1) ptx::tmem_dealloc2(tmem, kSTmemCols);
-  if (threadIdx.x == 0) SVSK_STAMP(15);
-#undef SVSK_STAMP
 }
 
 }  // namespace svsk
@@ -855,17 +817,13 @@ using namespace svsk;
 
 using StackKernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap,
                                DiffnetStackArgs);
-static StackKernelFn stack_kernel_variant(bool use_p, bool dsmem, bool prof, int C) {
-  static const StackKernelFn table[16] = {
-      diffnet_stack_kernel<false, false, false, 256>, diffnet_stack_kernel<true, false, false, 256>,
-      diffnet_stack_kernel<false, true, false, 256>,  diffnet_stack_kernel<true, true, false, 256>,
-      diffnet_stack_kernel<false, false, true, 256>,  diffnet_stack_kernel<true, false, true, 256>,
-      diffnet_stack_kernel<false, true, true, 256>,   diffnet_stack_kernel<true, true, true, 256>,
-      diffnet_stack_kernel<false, false, false, 128>, diffnet_stack_kernel<true, false, false, 128>,
-      diffnet_stack_kernel<false, true, false, 128>,  diffnet_stack_kernel<true, true, false, 128>,
-      diffnet_stack_kernel<false, false, true, 128>,  diffnet_stack_kernel<true, false, true, 128>,
-      diffnet_stack_kernel<false, true, true, 128>,   diffnet_stack_kernel<true, true, true, 128>};
-  return table[(use_p ? 1 : 0) | (dsmem ? 2 : 0) | (prof ? 4 : 0) | (C == 128 ? 8 : 0)];
+static StackKernelFn stack_kernel_variant(bool use_p, bool dsmem, int C) {
+  static const StackKernelFn table[8] = {
+      diffnet_stack_kernel<false, false, 256>, diffnet_stack_kernel<true, false, 256>,
+      diffnet_stack_kernel<false, true, 256>,  diffnet_stack_kernel<true, true, 256>,
+      diffnet_stack_kernel<false, false, 128>, diffnet_stack_kernel<true, false, 128>,
+      diffnet_stack_kernel<false, true, 128>,  diffnet_stack_kernel<true, true, 128>};
+  return table[(use_p ? 1 : 0) | (dsmem ? 2 : 0) | (C == 128 ? 4 : 0)];
 }
 
 namespace svsk {  // diffnet_stack_duo_sm100.cu: C = 128 with two tiles per CTA pair
@@ -894,7 +852,7 @@ static int stack_smem(int C, int H, int* nentries_out, int* cond_resident_out = 
   int fixed = CB * kSWinBytes + gc_tiles * kSTile + 4 * 2 * C * (int)sizeof(float) + (int)sizeof(DiffnetStackBarriers) + 1024;
   // C = 128: resident conditioner tiles if that still leaves a ring of 5 (the depth the C = 256 kernel runs with)
   int resident = 0;
-  if (C == 128 && HB > 0 && !getenv("SVSK_STACK_NO_PINGPONG") && (kSSmemLimit - fixed - HB * kSTile) / kSTile >= 5) {
+  if (C == 128 && HB > 0 && (kSSmemLimit - fixed - HB * kSTile) / kSTile >= 5) {
     resident = 1;
     fixed += HB * kSTile;
   }
@@ -917,8 +875,8 @@ static int stack_prepare(int C, int H, int* nentries, int* smem_bytes, int* cond
   static bool attr_set[64] = {false};
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
     cudaError_t e = cudaSuccess;
-    for (int v = 0; v < 16 && e == cudaSuccess; ++v) {
-      StackKernelFn fn = stack_kernel_variant(v & 1, v & 2, v & 4, (v & 8) ? 128 : 256);
+    for (int v = 0; v < 8 && e == cudaSuccess; ++v) {
+      StackKernelFn fn = stack_kernel_variant(v & 1, v & 2, (v & 4) ? 128 : 256);
       e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, kSSmemLimit);
       if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
     }
@@ -932,7 +890,7 @@ static int stack_prepare(int C, int H, int* nentries, int* smem_bytes, int* cond
 // size is the next power of two (extra CTAs work on frames past the end: zeros in, nothing out).  Otherwise CTA pairs.
 static int stack_cluster_size(int T) {
   const int tiles = 2 * ceil_div(T, 256);
-  if (tiles > 16 || getenv("SVSK_STACK_NO_DSMEM")) return 2;
+  if (tiles > 16) return 2;
   int c = 2;
   while (c < tiles) c *= 2;
   return c;
@@ -953,12 +911,11 @@ static void stack_launch_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at
   // neighbour hand-shakes need even when other work shares the device
   // One cluster per track (DSMEM mode) has no hand-shake across clusters — the cluster launch itself co-schedules the
   // CTAs that talk to each other — so it needs no such guarantee (and no per-tile counters to reset): a plain cluster
-  // launch measures 0.9 % faster per sampling pass (same-box A/B against SVSK_STACK_COOPERATIVE=1: 41.70 vs 42.07 ms).  (A programmatic-dependent-launch edge between the stack and the
+  // launch measures 0.9 % faster per sampling pass (same-box A/B against a cooperative launch: 41.70 vs 42.07 ms).  (A programmatic-dependent-launch edge between the stack and the
   // step kernel was measured as well: no gain — the early CTAs of the next kernel only fragment the cluster placement.)
-  // A track that is a single CTA pair (T <= 256) has no neighbour at all: same plain launch (which also keeps small
-  // calls such as __graft_entry__.smoke() replayable by ncu, whose kernel replay cannot re-launch a cooperative grid).
+  // A track that is a single CTA pair (T <= 256) has no neighbour at all: same plain launch.
   const bool single_pair = ceil_div(T, 256) == 1;
-  if ((csize > 2 || single_pair) && !getenv("SVSK_STACK_COOPERATIVE")) {
+  if (csize > 2 || single_pair) {
     cfg->attrs = attr;
     cfg->numAttrs = 1;
     return;
@@ -966,7 +923,7 @@ static void stack_launch_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at
   attr[1].id = cudaLaunchAttributeCooperative;
   attr[1].val.cooperative = 1;
   cfg->attrs = attr;
-  cfg->numAttrs = getenv("SVSK_STACK_NO_COOPERATIVE") ? 1 : 2;
+  cfg->numAttrs = 2;
 }
 
 static int stack_one_tile_fits(int B, int T, int C, int H) {
@@ -976,7 +933,7 @@ static int stack_one_tile_fits(int B, int T, int C, int H) {
   cudaLaunchAttribute attr[2];
   stack_launch_config(&cfg, attr, B, T, smem_bytes, nullptr);
   int max_clusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&max_clusters, stack_kernel_variant(false, false, false, C), &cfg) != cudaSuccess) {
+  if (cudaOccupancyMaxActiveClusters(&max_clusters, stack_kernel_variant(false, false, C), &cfg) != cudaSuccess) {
     cudaGetLastError();
     return 0;
   }
@@ -1070,7 +1027,7 @@ extern "C" int svsk_diffnet_stack_bf16(const svsk_diffnet_stack_params* pp, void
   cudaLaunchAttribute attr[2];
   stack_launch_config(&cfg, attr, p.B, p.T, smem_bytes, stream);
   int max_clusters = 0;
-  cudaError_t oe = cudaOccupancyMaxActiveClusters(&max_clusters, stack_kernel_variant(false, false, false, p.C), &cfg);
+  cudaError_t oe = cudaOccupancyMaxActiveClusters(&max_clusters, stack_kernel_variant(false, false, p.C), &cfg);
   if (oe != cudaSuccess) return fail((int)oe, "diffnet_stack_bf16: cudaOccupancyMaxActiveClusters: %s", cudaGetErrorString(oe));
   const int n_clusters = (int)(cfg.gridDim.x / attr[0].val.clusterDim.x) * p.B;
   SVSK_REQUIRE(n_clusters <= max_clusters, SVSK_E_ARG,
@@ -1128,22 +1085,19 @@ extern "C" int svsk_diffnet_stack_bf16(const svsk_diffnet_stack_params* pp, void
   a.sb_layer_stride = p.stepbias_layer_stride;
   a.init_skip = p.init_skip;
   a.nentries = nentries;
-  a.pingpong = (p.C == 128 && !getenv("SVSK_STACK_NO_PINGPONG")) ? 1 : 0;
   a.cond_resident = cond_resident;
   a.use_p = use_p ? 1 : 0;
   a.pfilt = static_cast<const uint4*>(p.pcond_filt);
   a.tiles_per_track = 2 * ceil_div(p.T, 256);
   for (int l = 0; l < kSMaxLayers; ++l) a.dilation[l] = l < p.L ? p.dilation[l] : 1;
-  a.dbg = nullptr;
-  if (const char* e = getenv("SVSK_DIFFNET_TIMELINE")) a.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
 
   cudaError_t e = cudaSuccess;
-  if (!a.dsmem_halo || getenv("SVSK_STACK_COOPERATIVE")) {  // the per-tile layer counters are only used when edge rows travel through global memory
+  if (!a.dsmem_halo) {  // the per-tile layer counters are only used when edge rows travel through global memory
     e = cudaMemsetAsync(p.flags, 0, sizeof(int) * (size_t)p.B * a.tiles_per_track, as_stream(stream));
     if (e != cudaSuccess) return fail((int)e, "diffnet_stack_bf16: flag reset: %s", cudaGetErrorString(e));
   }
-  e = cudaLaunchKernelEx(&cfg, stack_kernel_variant(use_p, a.dsmem_halo != 0, a.dbg != nullptr, p.C), tm_xw0, tm_e0, tm_e1, tm_cond, tm_w1,
-                         tm_wout, tm_skip, a);
+  e = cudaLaunchKernelEx(&cfg, stack_kernel_variant(use_p, a.dsmem_halo != 0, p.C), tm_xw0, tm_e0, tm_e1, tm_cond, tm_w1, tm_wout,
+                         tm_skip, a);
   if (e != cudaSuccess) return fail((int)e, "diffnet_stack_bf16: launch: %s", cudaGetErrorString(e));
   return check_launch("diffnet_stack_bf16");
 }

@@ -12,7 +12,6 @@
 // The weight region holds Wskip first (C/64 tiles of C rows), then Wout (C/64 tiles of Mp rows) and Win (ceil(Mp/64)
 // tiles of C rows), TMA-loaded as soon as GEMM-a has completed.
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "sm100_ptx.cuh"
 #include "svsk_common.cuh"
@@ -33,7 +32,6 @@ struct DiffnetStepArgs {
   const float *sra, *srm1, *c1, *c2, *plv;
   float skip_scale;
   int B, T, C, Mp, clip, head;
-  unsigned* dbg;  // SVSK_STEP_TIMELINE: clock stamps of CTA (0, 0), thread 0
 };
 
 struct __align__(8) DiffnetStepBarriers {
@@ -65,8 +63,6 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.y, t0 = blockIdx.x * 128;
-#define STEP_STAMP(i) do { if (a.dbg && threadIdx.x == 0 && blockIdx.x == 1 && blockIdx.y == 0) a.dbg[i] = (unsigned)clock(); } while (0)
-  STEP_STAMP(0);
 
   if (threadIdx.x == 0) {
     ptx::prefetch_tmap(&tm_wskip);
@@ -85,7 +81,6 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
     ptx::tmem_relinquish();
   }
 
-  STEP_STAMP(1);
   // ---- A = bf16(skip32 * scale): 16 bytes (8 channels) per thread and step, rows past the end of the track = 0.
   //      Eight steps' loads are in flight together (the loop is bound by the latency of its 128 KB of fp32 reads).
   {
@@ -123,7 +118,6 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
   ptx::tc_fence_after();
   const uint32_t tmem = bars->tmem_base;
   const uint32_t tm_a = tmem, tm_b = tmem + 256;  // D_a / D_c: columns [0, C) ; D_b: columns [256, 256 + Mp)
-  STEP_STAMP(2);
 
   // ---- GEMM-a
   if (threadIdx.x == 0) {
@@ -138,7 +132,6 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
   }
   ptx::mbar_wait(&bars->mma_done[0], 0);
   ptx::tc_fence_after();
-  STEP_STAMP(3);
   if (threadIdx.x == 0) {  // Wskip is dead: bring in the other two weight matrices while H is being written
     ptx::mbar_arrive_expect_tx(&bars->w_full[1], CB * Mp * 128 + (a.head ? MB * ws_tile : 0));
     for (int kb = 0; kb < CB; ++kb) ptx::tma_load_2d(wout_s + kb * kStepTile, &tm_wout, &bars->w_full[1], kb * 64, 0);
@@ -174,11 +167,9 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
   ptx::tc_fence_after();
 
   // ---- GEMM-b
-  STEP_STAMP(4);
   if (threadIdx.x == 0) {
     ptx::mbar_wait(&bars->w_full[1], 0);
     ptx::tc_fence_after();
-    STEP_STAMP(5);
     const uint32_t idesc = ptx::umma_idesc_bf16_f32(128, (uint32_t)Mp);
     const uint32_t h_lo = ptx::umma_desc_lo(ptx::smem_u32(ah)), w_lo = ptx::umma_desc_lo(ptx::smem_u32(wout_s));
     for (int kb = 0; kb < CB; ++kb)
@@ -204,7 +195,6 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
   }
   ptx::mbar_wait(&bars->mma_done[1], 0);
   ptx::tc_fence_after();
-  STEP_STAMP(6);
 
   // ---- eps = D_b + b_out ; DDPM update of x in place ; X = bf16(x) over H
   {
@@ -262,7 +252,6 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
     __syncthreads();
     ptx::tc_fence_after();
 
-    STEP_STAMP(7);
     // ---- GEMM-c (K = Mp: whole 16-column steps only, the weight tile's columns past Mp are TMA zero fill)
     if (threadIdx.x == 0) {
       const uint32_t idesc = ptx::umma_idesc_bf16_f32(128, (uint32_t)C);
@@ -276,7 +265,6 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
     }
     ptx::mbar_wait(&bars->mma_done[2], 0);
     ptx::tc_fence_after();
-    STEP_STAMP(8);
 
     // ---- xb = bf16(relu(D_c + b_in)) over X, then one TMA store per 64-channel tile (rows past the end are clipped)
     for (int c0 = 16 * half; c0 < C; c0 += 32) {
@@ -301,9 +289,7 @@ diffnet_step_kernel(const __grid_constant__ CUtensorMap tm_wskip, const __grid_c
     if (threadIdx.x == 0) {
       for (int cb = 0; cb < CB; ++cb) ptx::tma_store_3d(&tm_xout, ah + cb * kStepTile, cb * 64, t0, b);
       ptx::bulk_commit_group();
-      STEP_STAMP(9);
       ptx::bulk_wait_read_all();
-      STEP_STAMP(10);
     }
   } else {
     ptx::tc_fence_before();
@@ -379,23 +365,11 @@ extern "C" int svsk_diffnet_step_bf16(const svsk_diffnet_step_params* pp, void* 
   a.c1 = p.posterior_mean_coef1; a.c2 = p.posterior_mean_coef2; a.plv = p.posterior_log_variance_clipped;
   a.skip_scale = p.skip_scale;
   a.B = p.B; a.T = p.T; a.C = p.C; a.Mp = p.Mp; a.clip = p.clip_denoised; a.head = p.xb_out ? 1 : 0;
-  static unsigned* dbg_buf = nullptr;
-  const bool timeline = getenv("SVSK_STEP_TIMELINE") != nullptr;
-  if (timeline && !dbg_buf) cudaMalloc(&dbg_buf, 64);
-  a.dbg = timeline ? dbg_buf : nullptr;
   if (p.C == 128)
     diffnet_step_kernel<128><<<dim3(ceil_div(p.T, 128), p.B), kStepThreads, smem_bytes, as_stream(stream)>>>(tm_wskip, tm_wout, tm_win,
                                                                                                               tm_xout, a);
   else
     diffnet_step_kernel<256><<<dim3(ceil_div(p.T, 128), p.B), kStepThreads, smem_bytes, as_stream(stream)>>>(tm_wskip, tm_wout, tm_win,
                                                                                                               tm_xout, a);
-  if (timeline) {  // debugging aid: cycles since the kernel's first instruction at each phase boundary of one CTA
-    unsigned h[16];
-    cudaStreamSynchronize(as_stream(stream));
-    cudaMemcpy(h, dbg_buf, 64, cudaMemcpyDeviceToHost);
-    fprintf(stderr, "step timeline: prologue %u | A written %u | GEMM-a done %u | H written %u | Wout/Win landed %u | GEMM-b done %u | X written %u | "
-            "GEMM-c done %u | store issued %u | store read %u\n", h[1] - h[0], h[2] - h[0], h[3] - h[0], h[4] - h[0], h[5] - h[0], h[6] - h[0],
-            h[7] - h[0], h[8] - h[0], h[9] - h[0], h[10] - h[0]);
-  }
   return check_launch("diffnet_step_bf16");
 }

@@ -18,8 +18,6 @@
 //    units to all CTAs of the cluster as 16-byte st.async messages that complete a transaction barrier in the
 //    receiver — no __syncthreads and no cluster-wide barrier inside the loop;
 //  * the gate pre-activations of step t+3 are fetched while step t computes (register ring, loop unrolled by four).
-#include <cstdlib>
-
 #include "lstm_sm100.cuh"
 
 namespace svsk {
@@ -35,7 +33,6 @@ struct LstmArgs {
   long long pre_sb, pre_st, pre_sr, hf_sb, hf_st, hf_sr, hb_sb, hb_st;
   int B, T, H, ndir;
   int NC, U, L;           // CTAs per cluster, units per CTA, real elements per column segment (H / CS)
-  unsigned* dbg;          // SVSK_LSTM_TIMELINE: clock stamps of one step (CTA 0, thread 0)
 };
 
 // CS column segments per unit (lanes unit*CS .. unit*CS+CS-1), KSEG = padded segment length.  kTrain: the input-gate lane
@@ -120,12 +117,9 @@ __global__ void __launch_bounds__(kLstmMaxThreads, 1) lstm_recurrence_kernel(con
       const int t = t0 + j;
       if (t >= len) break;
       const int cur = j & 1, nxt = cur ^ 1;
-      const bool stamp = a.dbg && blockIdx.x == 0 && tid == 0 && t == 65;
-      if (stamp) a.dbg[0] = (unsigned)clock();
       if (tid == 0 && t + 1 < len) ptx::mbar_arrive_expect_tx(&hbar[nxt], (uint32_t)H * 4u);
       if (gate_thread && t + 3 < len) fetch(t + 3, q[(j + 3) & 3]);
       if (t > 0) ptx::mbar_wait(&hbar[cur], ((t - 1) >> 1) & 1);   // h_{t-1} complete in hbuf[cur]
-      if (stamp) a.dbg[1] = (unsigned)clock();
 
       const float* hs = &hbuf[cur][k * kPitch];
       float acc[4][2];
@@ -144,7 +138,6 @@ __global__ void __launch_bounds__(kLstmMaxThreads, 1) lstm_recurrence_kernel(con
         }
       }
       float s0 = acc[0][0] + acc[0][1], s1 = acc[1][0] + acc[1][1], s2 = acc[2][0] + acc[2][1], s3 = acc[3][0] + acc[3][1];
-      if (stamp) a.dbg[2] = (unsigned)clock() + (s0 == 123.f);
 
       // transposing reduction over the unit's CS lanes, then activation of the gate(s) this lane ends up with
       float gi, gf, gg, go;
@@ -182,7 +175,6 @@ __global__ void __launch_bounds__(kLstmMaxThreads, 1) lstm_recurrence_kernel(con
       }
       cell = fmaf(gf, cell, gi * gg);                                 // meaningful on the input-gate lane of each unit
       const float h = go * tanh_fast(cell);
-      if (stamp) a.dbg[3] = (unsigned)clock() + (h == 123.f);
       // four consecutive units' h -> one 16-byte message per (quad, destination CTA)
       const float m0 = __shfl_sync(0xffffffffu, h, (4 * mq + 0) * CS);
       const float m1 = __shfl_sync(0xffffffffu, h, (4 * mq + 1) * CS);
@@ -190,7 +182,6 @@ __global__ void __launch_bounds__(kLstmMaxThreads, 1) lstm_recurrence_kernel(con
       const float m3 = __shfl_sync(0xffffffffu, h, (4 * mq + 3) * CS);
       if (sender && t + 1 < len)
         st_async_v4(mdata0 + (uint32_t)(nxt * CS * kPitch) * 4u, m0, m1, m2, m3, mbar0 + (uint32_t)nxt * 8u);
-      if (stamp) a.dbg[4] = (unsigned)clock();
       if (cell_thread) {
         const int frame = frame_of(t);
         if (a.h_f32) a.h_f32[(size_t)b * a.hf_sb + (size_t)frame * a.hf_st + (size_t)col * a.hf_sr] = h;
@@ -267,21 +258,8 @@ extern "C" int svsk_lstm_f32(const svsk_lstm_params* pp, void* stream) {
   LstmArgs a;
   int CS = 1, threads = 0;
   if (int rc = lstm_args(pp, "lstm_f32", &a, &CS, &threads)) return rc;
-  const svsk_lstm_params& p = *pp;
   if (int rc = require_sm100()) return rc;
-  static unsigned* dbg_buf = nullptr;
-  const bool timeline = getenv("SVSK_LSTM_TIMELINE") != nullptr;
-  if (timeline && !dbg_buf) cudaMalloc(&dbg_buf, 64);
-  a.dbg = timeline ? dbg_buf : nullptr;
-  cudaStream_t st = as_stream(stream);
-  int rc = launch_lstm_any<false>(a, CS, threads, st);
-  if (timeline && rc == 0) {  // debugging aid: cycles from the top of step 65 to {wait done, dot done, h done, sent}
-    unsigned h[8];
-    cudaStreamSynchronize(st);
-    cudaMemcpy(h, dbg_buf, 32, cudaMemcpyDeviceToHost);
-    fprintf(stderr, "lstm timeline H=%d NC=%d: wait %u dot %u h %u sent %u\n", p.H, a.NC, h[1] - h[0], h[2] - h[0], h[3] - h[0], h[4] - h[0]);
-  }
-  return rc;
+  return launch_lstm_any<false>(a, CS, threads, as_stream(stream));
 }
 
 extern "C" int svsk_lstm_train_f32(const svsk_lstm_params* pp, float* gates, float* cell, void* stream) {

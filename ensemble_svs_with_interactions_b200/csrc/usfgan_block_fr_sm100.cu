@@ -37,7 +37,6 @@
 // TMEM: two D1 (2 x 128 columns, one per epilogue group) and four D2 (4 x 64, two per group: the residual's identity
 // MMAs of the group's next tile are issued while the current one is still being read) = 512 columns.
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "sm100_ptx.cuh"
 #include "svsk_common.cuh"
@@ -64,9 +63,6 @@ struct UsfganFrArgs {
   int B, T, dilation, adaptive, tiles_per_row, total_tiles;
   float out_scale;
   int out_relu;
-  unsigned long long* dbg;  // profiling only: [grid][16] accumulated clock64 deltas per role
-  int dbg_flags;            // profiling only: 1 = skip epilogue math/stores, 2 = no MUFU, 4 = skip MMAs, 8 = no global
-                            // stores, 16 = no TMEM loads, 64 = no TMA boxes for the gathered taps
 };
 
 struct __align__(8) UsfganFrBarriers {
@@ -99,7 +95,7 @@ __device__ __forceinline__ bool fr_tile_needs_gather(int t0, int T, int d, int a
 constexpr int kFWinRows = 128 + 16;
 constexpr int kFWinBytes = kFWinRows * 128;  // 18 KB: the tap0 tile of the stage + the first 2 KB of its centre tile
 
-template <bool kProf, bool kWindow>
+template <bool kWindow>
 __global__ void __launch_bounds__(kFThreads, 1)
 usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w1,
                        const __grid_constant__ CUtensorMap tm_wout, const __grid_constant__ CUtensorMap tm_xout,
@@ -117,7 +113,6 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int T = a.T;
-  const int flags = kProf ? a.dbg_flags : 0;
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tm_x);
@@ -161,15 +156,12 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
       ptx::mbar_arrive_expect_tx(&bars->w_full, 3 * kFTile + 8192);
       for (int kb = 0; kb < 3; ++kb) ptx::tma_load_2d(w1_s + kb * kFTile, &tm_w1, &bars->w_full, kb * 64, 0);
       ptx::tma_load_2d(wout_s, &tm_wout, &bars->w_full, 0, 0);
-      long long acc_p = 0;
       int n = 0;
       for (int tile = blockIdx.x; tile < a.total_tiles; tile += gridDim.x, ++n) {
         const int b = tile / a.tiles_per_row, t0 = (tile - b * a.tiles_per_row) * 128;
         const bool gather = fr_tile_needs_gather(t0, T, a.dilation, a.adaptive);
         const int st = n & 1;
-        const long long c_0 = (kProf ? clock64() : 0ll);
         ptx::mbar_wait(&bars->empty[st], ((n >> 1) & 1) ^ 1);
-        acc_p += (kProf ? clock64() : 0ll) - c_0;
         uint8_t* slot = stages + st * kFStage;
         if (kWindow && !gather) {
           ptx::mbar_arrive_expect_tx(&bars->full[st], kFWinBytes);
@@ -183,7 +175,6 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
           }
         }
       }
-      if (kProf && a.dbg) a.dbg[blockIdx.x * 16 + 0] = acc_p;  // producer: cycles waiting for a free stage
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ GEMM1 issuer
@@ -198,25 +189,19 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
       // The barriers of tile n+1 are probed while the MMAs of tile n are issued (ptx::umma_bf16_x4_probe): no phase can
       // complete twice in between, because the stage's next producer waits for this thread's commit.
       bool full_ready = false, g_ready = false;
-      long long acc_full = 0, acc_g = 0, acc_mma = 0, acc_total = (kProf ? clock64() : 0ll);
       const uint32_t wo_lo = ptx::umma_desc_lo(ptx::smem_u32(wout_s)), g_lo = ptx::umma_desc_lo(ptx::smem_u32(gbuf));
       // GEMM2 of this CTA's m-th tile: D2 += G . Wout^T onto the residual the identity MMAs left there
       auto issue_gemm2 = [&](int m) {
         const int pm = m & 1, j = pm * 2 + ((m >> 1) & 1);  // D2 accumulator: two per epilogue group, alternating
-        if (!(flags & 4)) {
-          const uint32_t gl = g_lo + pm * (kFTile >> 4);
+        const uint32_t gl = g_lo + pm * (kFTile >> 4);
 #pragma unroll
-          for (int k4 = 0; k4 < 4; ++k4) ptx::umma_bf16_lo(tmem + 256 + j * 64, gl + 2 * k4, wo_lo + 2 * k4, idesc2, 1);
-          ptx::umma_commit(&bars->d2_full[j]);
-        } else {
-          ptx::mbar_arrive(&bars->d2_full[j]);
-        }
+        for (int k4 = 0; k4 < 4; ++k4) ptx::umma_bf16_lo(tmem + 256 + j * 64, gl + 2 * k4, wo_lo + 2 * k4, idesc2, 1);
+        ptx::umma_commit(&bars->d2_full[j]);
       };
       int n = 0;
       int tt = (int)blockIdx.x % a.tiles_per_row;  // tile index within its track (kWindow: which operand layout the stage holds)
       for (int tile = blockIdx.x; tile < a.total_tiles; tile += gridDim.x, ++n) {
         const int p = n & 1;
-        long long c_0 = (kProf ? clock64() : 0ll);
         // D1[p] is free once the epilogue has gated tile n - 2 out of it — the same event makes G[p] of tile n - 2 ready
         // for GEMM2, which is therefore issued HERE, ahead of this tile's GEMM1.  With a thread of its own for GEMM2 both
         // woke on the same barrier, and whenever GEMM1's 17 MMAs won the race the epilogue group waited for four N = 64
@@ -228,13 +213,9 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
           ptx::tc_fence_after();
           issue_gemm2(n - 2);
         }
-        long long c_1 = (kProf ? clock64() : 0ll);
-        acc_g += c_1 - c_0;
         if (!full_ready) ptx::mbar_wait(&bars->full[p], (n >> 1) & 1);
         ptx::fence_proxy_async_smem();  // the gather warps' cp.async writes -> tensor-core (async proxy) reads
         ptx::tc_fence_after();
-        c_0 = (kProf ? clock64() : 0ll);
-        acc_full += c_0 - c_1;
         const uint32_t s_lo = st_lo + p * (kFStage >> 4);
         // operand rows: three tiles of the stage, or (window) three row offsets of one tile
         uint32_t a_t0 = s_lo, a_c = s_lo + kT16, a_t2 = s_lo + 2 * kT16;
@@ -252,39 +233,25 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
         const uint32_t nfull_par = ((n + 1) >> 1) & 1;
         uint64_t* ng = &bars->g_full[p ^ 1];
         const uint32_t ng_par = ((n - 1) >> 1) & 1;  // meaningful for n >= 1
-        if (!(flags & 4)) {
-          (void)ptx::umma_bf16_x4_probe(d1, a_t0, w1_lo, idesc1, 0, 4, nfull, nfull_par);
-          const bool r1 = ptx::umma_bf16_x4_probe(d1, a_c, w1_lo + kT16, idesc1, 1, 4, ng, ng_par);
-          const bool r2 = ptx::umma_bf16_x4_probe(d1, a_t2, w1_lo + 2 * kT16, idesc1, 1, 4, nfull, nfull_par);
-          // aux: A = U (K columns 0..15 of the aux tile's rows), B = Q (K columns 16..31 of the same rows)
-          ptx::umma_bf16_lo(d1, s_lo + 3 * kT16, s_lo + 3 * kT16 + 2, idesc1, 1);
-          // residual: D2 = X_centre . I, GEMM2 accumulates onto it.  This D2 accumulator was last read by the residual
-          // epilogue of tile n - 4, which its group finished before it gated tile n - 2 (waited for above).
-          const uint32_t d2 = tmem + 256 + (p * 2 + ((n >> 1) & 1)) * 64;
+        (void)ptx::umma_bf16_x4_probe(d1, a_t0, w1_lo, idesc1, 0, 4, nfull, nfull_par);
+        const bool r1 = ptx::umma_bf16_x4_probe(d1, a_c, w1_lo + kT16, idesc1, 1, 4, ng, ng_par);
+        const bool r2 = ptx::umma_bf16_x4_probe(d1, a_t2, w1_lo + 2 * kT16, idesc1, 1, 4, nfull, nfull_par);
+        // aux: A = U (K columns 0..15 of the aux tile's rows), B = Q (K columns 16..31 of the same rows)
+        ptx::umma_bf16_lo(d1, s_lo + 3 * kT16, s_lo + 3 * kT16 + 2, idesc1, 1);
+        // residual: D2 = X_centre . I, GEMM2 accumulates onto it.  This D2 accumulator was last read by the residual
+        // epilogue of tile n - 4, which its group finished before it gated tile n - 2 (waited for above).
+        const uint32_t d2 = tmem + 256 + (p * 2 + ((n >> 1) & 1)) * 64;
 #pragma unroll
-          for (int k4 = 0; k4 < 4; ++k4) ptx::umma_bf16_lo(d2, a_c + 2 * k4, id_lo + 2 * k4, idesc2, k4 != 0);
-          ptx::umma_commit(&bars->empty[p]);
-          ptx::umma_commit(&bars->d1_full[p]);
-          full_ready = r2;
-          g_ready = r1 && n >= 1;
-        } else {
-          ptx::mbar_arrive(&bars->empty[p]);
-          ptx::mbar_arrive(&bars->d1_full[p]);
-          full_ready = g_ready = false;
-        }
-        acc_mma += (kProf ? clock64() : 0ll) - c_0;
+        for (int k4 = 0; k4 < 4; ++k4) ptx::umma_bf16_lo(d2, a_c + 2 * k4, id_lo + 2 * k4, idesc2, k4 != 0);
+        ptx::umma_commit(&bars->empty[p]);
+        ptx::umma_commit(&bars->d1_full[p]);
+        full_ready = r2;
+        g_ready = r1 && n >= 1;
       }
       for (int m = n >= 2 ? n - 2 : 0; m < n; ++m) {  // GEMM2 of the last two tiles
         ptx::mbar_wait(&bars->g_full[m & 1], (m >> 1) & 1);
         ptx::tc_fence_after();
         issue_gemm2(m);
-      }
-      if (kProf && a.dbg) {
-        a.dbg[blockIdx.x * 16 + 1] = acc_full;  // GEMM1 thread: waiting for operands
-        a.dbg[blockIdx.x * 16 + 2] = acc_g;     // GEMM1 thread: waiting for the accumulator to be gated out
-        a.dbg[blockIdx.x * 16 + 3] = (kProf ? clock64() : 0ll) - acc_total;
-        a.dbg[blockIdx.x * 16 + 4] = n;
-        a.dbg[blockIdx.x * 16 + 13] = acc_mma;  // GEMM1 thread: issue + commits
       }
     }
   } else if (warp < 6) {
@@ -303,7 +270,6 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
     };
     int ip_next, ifu_next;
     load_idx(blockIdx.x, ip_next, ifu_next);
-    long long acc_w = 0, acc_i = 0;
     int n = 0;
     for (int tile = blockIdx.x; tile < a.total_tiles; tile += gridDim.x, ++n) {
       const int b = tile / a.tiles_per_row, t0 = (tile - b * a.tiles_per_row) * 128;
@@ -312,10 +278,7 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
       const int ip = ip_next, ifu = ifu_next;
       load_idx(tile + gridDim.x, ip_next, ifu_next);
       const int st = n & 1;
-      long long c_0 = (kProf ? clock64() : 0ll);
       ptx::mbar_wait_warp(&bars->empty[st], ((n >> 1) & 1) ^ 1);
-      long long c_1 = (kProf ? clock64() : 0ll);
-      acc_w += c_1 - c_0;
       uint8_t* slot = stages + st * kFStage;
       {
         uint8_t* aux_s = slot + 3 * kFTile;
@@ -350,7 +313,7 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
           // row (16 cp.async per thread and tile were 1.7 k of the adaptive blocks' 4.1 k cycles per tile).
           const int base = __shfl_sync(0xffffffffu, src, lane & ~7);
           const unsigned lin = __ballot_sync(0xffffffffu, ok && src == base + (lane & 7));
-          if (((lin >> (lane & ~7)) & 0xffu) == 0xffu && !(flags & 64)) {
+          if (((lin >> (lane & ~7)) & 0xffu) == 0xffu) {
             if ((lane & 7) == 0) {
               fr_mbar_expect_tx(&bars->full[st], 1024u);
               ptx::tma_load_3d(dst + (r >> 3) * 1024, &tm_x8, &bars->full[st], 0, base, b);
@@ -364,13 +327,8 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
         }
       }
       fr_cp_async_arrive_noinc(&bars->full[st]);
-      acc_i += (kProf ? clock64() : 0ll) - c_1;
     }
     asm volatile("cp.async.wait_all;" ::: "memory");
-    if (kProf && a.dbg && r == 0) {
-      a.dbg[blockIdx.x * 16 + 14] = acc_w;  // gather: waiting for a free stage
-      a.dbg[blockIdx.x * 16 + 15] = acc_i;  // gather: issuing copies
-    }
   } else if (warp == 6) {
     // (idle: GEMM2 is issued by the GEMM1 thread, see there)
   } else {
@@ -388,39 +346,28 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
     const int q = warp & 3;
     const int row = q * 32 + lane;
     const uint32_t tlane = (uint32_t)(q * 32) << 16;
-    const bool elected = ((e & 7) == 0 && lane == 0);
     const bool qlead = (sub == 0 && lane == 0);  // issues the TMA stores of this lane quarter's 32 rows
     const uint32_t qbar = 1 + p * 4 + q;         // named barrier of the quarter's two warps
     const int my_tiles = a.total_tiles > (int)blockIdx.x ? (a.total_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
     const int own = my_tiles > p ? (my_tiles - 1 - p) / 2 + 1 : 0;  // tiles of this group
-    long long acc_d1 = 0, acc_gate = 0, acc_d2 = 0, acc_e2 = 0;
     uint8_t* gb = gbuf + p * kFTile;
     for (int k = 0; k < own; ++k) {
       const int n = p + 2 * k;
       const int tile = blockIdx.x + n * gridDim.x;
       const int b = tile / a.tiles_per_row, t0 = (tile - b * a.tiles_per_row) * 128;
-      long long c_0 = (kProf ? clock64() : 0ll);
       ptx::mbar_wait_warp(&bars->d1_full[p], k & 1);
       ptx::tc_fence_after();
-      acc_d1 += (kProf ? clock64() : 0ll) - c_0;
-      c_0 = (kProf ? clock64() : 0ll);
       if (k >= 1) {  // this quarter's rows of G[p] held the previous output tile: its TMA store must have read them
         if (qlead) ptx::bulk_wait_read_all();
         ptx::named_bar_sync(qbar, 64);
       }
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
-        if (flags & 1) break;
         const int c0 = 16 * (2 * i + sub);
         uint32_t ra[16], rb[16];
-        if (!(flags & 16)) {
-          ptx::tmem_ld16(tmem + tlane + p * 128 + c0, ra);
-          ptx::tmem_ld16(tmem + tlane + p * 128 + 64 + c0, rb);
-          ptx::tmem_ld_wait();
-        } else {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) ra[j] = rb[j] = 0x3dcccccdu + j;
-        }
+        ptx::tmem_ld16(tmem + tlane + p * 128 + c0, ra);
+        ptx::tmem_ld16(tmem + tlane + p * 128 + 64 + c0, rb);
+        ptx::tmem_ld_wait();
         uint32_t o[8];
 #pragma unroll
         for (int v = 0; v < 4; ++v) {
@@ -428,19 +375,12 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
           const float fa[4] = {__uint_as_float(ba.x), __uint_as_float(ba.y), __uint_as_float(ba.z), __uint_as_float(ba.w)};
           const float fb[4] = {__uint_as_float(bb.x), __uint_as_float(bb.y), __uint_as_float(bb.z), __uint_as_float(bb.w)};
           float z[4];
-          if (kProf && (flags & 2)) {  // ablation: no MUFU
+          // column pairs: FADD2 / FMUL2 / FFMA2 — same arithmetic per lane as tanh_approx(ya) * sigmoid_approx(yb)
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float ya = __uint_as_float(ra[4 * v + j]) + fa[j], yb = __uint_as_float(rb[4 * v + j]) + fb[j];
-              z[j] = ya * fmaf(yb, 0.25f, 0.5f);
-            }
-          } else {  // column pairs: FADD2 / FMUL2 / FFMA2 — same arithmetic per lane as tanh_approx(ya) * sigmoid_approx(yb)
-#pragma unroll
-            for (int j = 0; j < 4; j += 2) {
-              const uint64_t ya = ptx::f2_add(ptx::f2_pack(__uint_as_float(ra[4 * v + j]), __uint_as_float(ra[4 * v + j + 1])), ptx::f2_pack(fa[j], fa[j + 1]));
-              const uint64_t yb = ptx::f2_add(ptx::f2_pack(__uint_as_float(rb[4 * v + j]), __uint_as_float(rb[4 * v + j + 1])), ptx::f2_pack(fb[j], fb[j + 1]));
-              ptx::f2_unpack(ptx::f2_gate(yb, ya), z[j], z[j + 1]);
-            }
+          for (int j = 0; j < 4; j += 2) {
+            const uint64_t ya = ptx::f2_add(ptx::f2_pack(__uint_as_float(ra[4 * v + j]), __uint_as_float(ra[4 * v + j + 1])), ptx::f2_pack(fa[j], fa[j + 1]));
+            const uint64_t yb = ptx::f2_add(ptx::f2_pack(__uint_as_float(rb[4 * v + j]), __uint_as_float(rb[4 * v + j + 1])), ptx::f2_pack(fb[j], fb[j + 1]));
+            ptx::f2_unpack(ptx::f2_gate(yb, ya), z[j], z[j + 1]);
           }
           o[2 * v] = ptx::pack_bf16(z[0], z[1]);
           o[2 * v + 1] = ptx::pack_bf16(z[2], z[3]);
@@ -451,25 +391,15 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
       ptx::tc_fence_before();
       ptx::fence_proxy_async_smem();
       ptx::mbar_arrive(&bars->g_full[p]);
-      acc_gate += (kProf ? clock64() : 0ll) - c_0;
-      c_0 = (kProf ? clock64() : 0ll);
       const int j2 = p * 2 + (k & 1);
       ptx::mbar_wait_warp(&bars->d2_full[j2], (k >> 1) & 1);  // D2 = x + G . Wout^T is there, GEMM2 has read G[p]
       ptx::tc_fence_after();
-      acc_d2 += (kProf ? clock64() : 0ll) - c_0;
-      c_0 = (kProf ? clock64() : 0ll);
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
-        if (flags & 1) break;
         const int c0 = 16 * (2 * i + sub);
         uint32_t rd[16];
-        if (!(flags & 16)) {
-          ptx::tmem_ld16(tmem + tlane + 256 + j2 * 64 + c0, rd);
-          ptx::tmem_ld_wait();
-        } else {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) rd[j] = 0x3dcccccdu + j;
-        }
+        ptx::tmem_ld16(tmem + tlane + 256 + j2 * 64 + c0, rd);
+        ptx::tmem_ld_wait();
         uint32_t o[8];
 #pragma unroll
         for (int v = 0; v < 4; ++v) {
@@ -496,19 +426,12 @@ usfgan_block_fr_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
       ptx::fence_proxy_async_smem();
       // each TMEM lane quarter (two warps, 32 rows of the tile) stores its own rows
       ptx::named_bar_sync(qbar, 64);
-      if (qlead && !(flags & 8)) {
+      if (qlead) {
         ptx::tma_store_3d(&tm_xout, gb + q * 4096, 0, t0 + q * 32, b);
         ptx::bulk_commit_group();
       }
-      acc_e2 += (kProf ? clock64() : 0ll) - c_0;
     }
     if (qlead) ptx::bulk_wait_read_all();
-    if (kProf && a.dbg && elected) {  // slots 5..8 hold group 0, 9..12 group 1
-      a.dbg[blockIdx.x * 16 + 5 + 4 * p + 0] = acc_d1;    // epilogue: waiting for D1
-      a.dbg[blockIdx.x * 16 + 5 + 4 * p + 1] = acc_gate;  // epilogue: store-read wait + gating + G stores + arrive
-      a.dbg[blockIdx.x * 16 + 5 + 4 * p + 2] = acc_d2;    // epilogue: waiting for D2
-      a.dbg[blockIdx.x * 16 + 5 + 4 * p + 3] = acc_e2;    // epilogue: output maths + staging + TMA store issue
-    }
   }
 
   ptx::tc_fence_before();
@@ -561,10 +484,8 @@ int usfgan_block_fr_launch(const svsk_usfgan_block_params& p, void* stream) {
   cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
   static bool attr_set[64] = {false};
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(usfgan_block_fr_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(usfgan_block_fr_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(usfgan_block_fr_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(usfgan_block_fr_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+    cudaError_t e = cudaFuncSetAttribute(usfgan_block_fr_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(usfgan_block_fr_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
     if (e != cudaSuccess) return fail((int)e, "usfgan_block_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
   }
@@ -586,21 +507,12 @@ int usfgan_block_fr_launch(const svsk_usfgan_block_params& p, void* stream) {
   a.total_tiles = p.B * tiles_per_row;
   a.out_scale = p.out_scale;
   a.out_relu = p.out_relu;
-  a.dbg_flags = 0;
-  a.dbg = nullptr;
-  if (const char* e = getenv("SVSK_USFGAN_ABLATE")) a.dbg_flags = atoi(e);
-  if (const char* e = getenv("SVSK_USFGAN_TIMELINE")) a.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
   const int grid = a.total_tiles < num_sms ? a.total_tiles : num_sms;
-  const bool prof = a.dbg || a.dbg_flags;  // clock64 role accounting (distorts the timing) and / or ablation flags
-  const bool window = !p.adaptive && p.dilation >= 1 && p.dilation <= 8 && !getenv("SVSK_USFGAN_NO_WINDOW");
-  if (prof && window)
-    usfgan_block_fr_kernel<true, true><<<grid, kFThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_w1, tm_wout, tm_xout, tm_x8, tm_xw, a);
-  else if (prof)
-    usfgan_block_fr_kernel<true, false><<<grid, kFThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_w1, tm_wout, tm_xout, tm_x8, tm_xw, a);
-  else if (window)
-    usfgan_block_fr_kernel<false, true><<<grid, kFThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_w1, tm_wout, tm_xout, tm_x8, tm_xw, a);
+  const bool window = !p.adaptive && p.dilation >= 1 && p.dilation <= 8;
+  if (window)
+    usfgan_block_fr_kernel<true><<<grid, kFThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_w1, tm_wout, tm_xout, tm_x8, tm_xw, a);
   else
-    usfgan_block_fr_kernel<false, false><<<grid, kFThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_w1, tm_wout, tm_xout, tm_x8, tm_xw, a);
+    usfgan_block_fr_kernel<false><<<grid, kFThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_w1, tm_wout, tm_xout, tm_x8, tm_xw, a);
   return check_launch("usfgan_block_bf16 (frame-rate aux)");
 }
 

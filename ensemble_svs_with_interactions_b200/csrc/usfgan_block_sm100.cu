@@ -21,7 +21,6 @@
 // TMEM holds two D1 (2x128 columns) and two D2 (2x64) accumulators, so the MMAs of tile n+1 overlap the epilogue of
 // tile n.  The residual x(t) is prefetched by its epilogue thread (one 128-byte row per thread) at the top of the tile.
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "sm100_ptx.cuh"
 #include "svsk_common.cuh"
@@ -42,8 +41,6 @@ struct UsfganArgs {
   int B, T, A, dilation, adaptive, nstages, akb, last_ksteps, tiles_per_row, total_tiles;
   float out_scale;
   int out_relu;
-  unsigned long long* dbg;  // profiling only: [grid][16] accumulated clock64 deltas per role
-  int dbg_flags;  // profiling only: 1 = skip epilogue math/stores, 4 = skip MMAs, 8 = skip TMA loads after the first ring fill
 };
 
 struct __align__(8) UsfganBarriers {
@@ -68,7 +65,6 @@ __device__ __forceinline__ bool tile_needs_gather(int t0, int T, int d, int adap
   return (t0 - d < 0) || (last + d >= T);  // a reflected tap: rows are not a shifted copy any more
 }
 
-template <bool kProf, bool kFlags>
 __global__ void __launch_bounds__(kUThreads, 1)
 usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_aux,
                     const __grid_constant__ CUtensorMap tm_w1, const __grid_constant__ CUtensorMap tm_wout,
@@ -123,20 +119,12 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
       ptx::tma_load_2d(wout_s, &tm_wout, &bars->w_full, 0, 0);
       int s = 0;
       uint32_t ph = 0;
-      long long acc_p = 0;
       for (int tile = blockIdx.x; tile < a.total_tiles; tile += gridDim.x) {
         const int b = tile / a.tiles_per_row, t0 = (tile - b * a.tiles_per_row) * 128;
         const bool gather = tile_needs_gather(t0, T, a.dilation, a.adaptive);
         for (int kb = 0; kb < KB; ++kb) {
-          const long long c_0 = (kProf ? clock64() : 0ll);
           ptx::mbar_wait(&bars->empty[s], ph ^ 1);
-          acc_p += (kProf ? clock64() : 0ll) - c_0;
           uint8_t* slot = ring + s * kUTile;
-          if (((kFlags ? a.dbg_flags : 0) & 8) && (tile != blockIdx.x) && !(gather && (kb == 0 || kb == 2))) {
-            ptx::mbar_arrive(&bars->full_t[s]);
-            if (++s == a.nstages) { s = 0; ph ^= 1; }
-            continue;
-          }
           if (kb == 1) {
             ptx::mbar_arrive_expect_tx(&bars->full_t[s], kUTile);
             ptx::tma_load_3d(slot, &tm_x, &bars->full_t[s], 0, t0, b);
@@ -150,7 +138,6 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
           if (++s == a.nstages) { s = 0; ph ^= 1; }
         }
       }
-      if (kProf && a.dbg) a.dbg[blockIdx.x * 16 + 0] = acc_p;  // producer: cycles waiting for free slots
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
@@ -162,7 +149,6 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
       int s = 0;
       uint32_t ph = 0, pht = 0, phg = 0;  // per-slot phase bits of full_t / full_g (each toggles only when used)
       int n_issued = 0;  // tiles whose GEMM1 has been issued
-      long long acc_full = 0, acc_g = 0, acc_fence = 0, acc_commit = 0, acc_probe = 0, acc_mma = 0, acc_total = (kProf ? clock64() : 0ll);
       for (int tile = blockIdx.x;; tile += gridDim.x) {
         const bool have = tile < a.total_tiles;
         if (have) {
@@ -171,25 +157,16 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
           const int p = n_issued & 1;
           // D1[p] is free once the epilogue has gated tile n_issued - 2 out of it (GEMM2 has its own issuing thread, so
           // this thread has to observe g_full itself)
-          if (n_issued >= 2) {
-            const long long c_g = (kProf ? clock64() : 0ll);
-            ptx::mbar_wait(&bars->g_full[p], ((n_issued - 2) >> 1) & 1);
-            acc_g += (kProf ? clock64() : 0ll) - c_g;
-          }
+          if (n_issued >= 2) ptx::mbar_wait(&bars->g_full[p], ((n_issued - 2) >> 1) & 1);
           // the first k-block's barrier is probed here, every later one while the previous k-block's MMAs are issued
           bool ready = false;
           for (int kb = 0; kb < KB; ++kb) {
             const bool from_gather = gather && (kb == 0 || kb == 2);
             uint64_t* fb = from_gather ? &bars->full_g[s] : &bars->full_t[s];
             const uint32_t par = from_gather ? ((phg >> s) & 1) : ((pht >> s) & 1);
-            const long long c_0 = (kProf ? clock64() : 0ll);
             if (!ready) ptx::mbar_wait(fb, par);
             if (from_gather) { phg ^= 1u << s; ptx::fence_proxy_async_smem(); } else { pht ^= 1u << s; }
-            const long long c_1 = (kProf ? clock64() : 0ll);
-            acc_full += c_1 - c_0;
             ptx::tc_fence_after();
-            const long long c_2 = (kProf ? clock64() : 0ll);
-            acc_fence += c_2 - c_1;
             // probe the next k-block of this tile (the next tile's first k-block is waited for normally).  The probe is
             // issued before this k-block's MMAs and its result consumed after them (ptx::umma_bf16_x4_probe): a test whose
             // result is needed at once stalls this thread ~130 cycles per k-block (tools/ubench_umma.py).
@@ -197,39 +174,17 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
             const bool ng = gather && (kb + 1 == 0 || kb + 1 == 2);
             uint64_t* nbar = ng ? &bars->full_g[s_next] : &bars->full_t[s_next];
             const uint32_t npar = ng ? ((phg >> s_next) & 1) : ((pht >> s_next) & 1);
-            const long long c_2b = (kProf ? clock64() : 0ll);
-            acc_probe += c_2b - c_2;
             const uint32_t a_lo = ring_lo + s * (kUTile >> 4), b_lo = w1_lo + kb * (kUTile >> 4);
             const int ks = (kb == KB - 1) ? a.last_ksteps : 4;
-            ready = false;
-            if ((kFlags ? a.dbg_flags : 0) & 256) {  // A/B: the earlier synchronous probe
-              if (kb + 1 < KB) ready = ptx::mbar_test(nbar, npar);
-              ptx::umma_bf16_lo(tmem + p * 128, a_lo, b_lo, idesc1, kb != 0);
-              for (int k4 = 1; k4 < ks; ++k4) ptx::umma_bf16_lo(tmem + p * 128, a_lo + 2 * k4, b_lo + 2 * k4, idesc1, 1);
-            } else if (!((kFlags ? a.dbg_flags : 0) & 4)) {
-              const bool r = ptx::umma_bf16_x4_probe(tmem + p * 128, a_lo, b_lo, idesc1, kb != 0, ks, nbar, npar);
-              ready = r && (kb + 1 < KB);
-            }
-            const long long c_3 = (kProf ? clock64() : 0ll);
-            acc_mma += c_3 - c_2b;
-            if ((kFlags ? a.dbg_flags : 0) & 32) ptx::mbar_arrive(&bars->empty[s]); else ptx::umma_commit(&bars->empty[s]);
-            acc_commit += (kProf ? clock64() : 0ll) - c_3;
+            const bool r = ptx::umma_bf16_x4_probe(tmem + p * 128, a_lo, b_lo, idesc1, kb != 0, ks, nbar, npar);
+            ready = r && (kb + 1 < KB);
+            ptx::umma_commit(&bars->empty[s]);
             if (++s == a.nstages) { s = 0; ph ^= 1; }
           }
-          if ((kFlags ? a.dbg_flags : 0) & 32) ptx::mbar_arrive(&bars->d1_full[p]); else ptx::umma_commit(&bars->d1_full[p]);
+          ptx::umma_commit(&bars->d1_full[p]);
         }
         if (!have) break;
         ++n_issued;
-      }
-      if (kProf && a.dbg) {
-        a.dbg[blockIdx.x * 16 + 1] = acc_full;                 // MMA thread: waiting for operands
-        a.dbg[blockIdx.x * 16 + 2] = acc_g;                    // MMA thread: waiting for G
-        a.dbg[blockIdx.x * 16 + 3] = (kProf ? clock64() : 0ll) - acc_total;    // MMA thread: whole loop
-        a.dbg[blockIdx.x * 16 + 4] = n_issued;
-        a.dbg[blockIdx.x * 16 + 10] = acc_fence;
-        a.dbg[blockIdx.x * 16 + 11] = acc_commit;
-        a.dbg[blockIdx.x * 16 + 12] = acc_probe;
-        a.dbg[blockIdx.x * 16 + 13] = acc_mma;
       }
       (void)ph;
     }
@@ -308,12 +263,10 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
     const int sub = (warp - 6) >> 2;  // 0: 16-column chunks 0 and 2, 1: chunks 1 and 3
     const int row = q * 32 + lane;
     const uint32_t tlane = (uint32_t)(q * 32) << 16;
-    const bool elected = (warp == 6 && lane == 0);
     const bool qlead = (sub == 0 && lane == 0);  // issues the TMA stores of this lane quarter's 32 rows
     // Software-pipelined: iteration `it` gates tile it (so GEMM2(it) can be queued) and THEN finishes tile it-1, whose
     // GEMM2 ran behind GEMM1(it) in the in-order tensor pipe while this warp group was gating.
     const int my_tiles = a.total_tiles > (int)blockIdx.x ? (a.total_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
-    long long acc_d1 = 0, acc_gate = 0, acc_d2 = 0, acc_e2 = 0, acc_sync = 0;
     uint4 xr_prev[2][2], xr_cur[2][2];
 #pragma unroll
     for (int i = 0; i < 2; ++i) xr_prev[i][0] = xr_prev[i][1] = xr_cur[i][0] = xr_cur[i][1] = make_uint4(0, 0, 0, 0);
@@ -335,20 +288,14 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
           }
         }
         uint8_t* gb = gbuf + (it % 3) * kUTile;
-        long long c_0 = (kProf ? clock64() : 0ll);
         if (it >= 3) {  // buffer it%3 held the output tile of tile it-3: this quarter's TMA store must have read its rows
           if (qlead) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
           ptx::named_bar_sync(4 + q, 64);
         }
-        acc_sync += (kProf ? clock64() : 0ll) - c_0;
-        c_0 = (kProf ? clock64() : 0ll);
         ptx::mbar_wait_warp(&bars->d1_full[p], (it >> 1) & 1);
         ptx::tc_fence_after();
-        acc_d1 += (kProf ? clock64() : 0ll) - c_0;
-        c_0 = (kProf ? clock64() : 0ll);
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
-          if ((kFlags ? a.dbg_flags : 0) & 1) break;
           const int c0 = 16 * (2 * i + sub);
           uint32_t ra[16], rb[16];
           ptx::tmem_ld16(tmem + tlane + p * 128 + c0, ra);
@@ -369,21 +316,16 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
         ptx::tc_fence_before();
         ptx::fence_proxy_async_smem();
         ptx::mbar_arrive(&bars->g_full[p]);
-        acc_gate += (kProf ? clock64() : 0ll) - c_0;
       }
       if (it >= 1) {
         const int m = it - 1, p = m & 1;
         const int tile = blockIdx.x + m * gridDim.x;
         const int b = tile / a.tiles_per_row, t0 = (tile - b * a.tiles_per_row) * 128;
         uint8_t* gb = gbuf + (m % 3) * kUTile;
-        long long c_0 = (kProf ? clock64() : 0ll);
         ptx::mbar_wait_warp(&bars->d2_full[p], (m >> 1) & 1);
         ptx::tc_fence_after();
-        acc_d2 += (kProf ? clock64() : 0ll) - c_0;
-        c_0 = (kProf ? clock64() : 0ll);
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
-          if ((kFlags ? a.dbg_flags : 0) & 1) break;
           const int c0 = 16 * (2 * i + sub);
           uint32_t rd[16];
           ptx::tmem_ld16(tmem + tlane + 256 + p * 64 + c0, rd);
@@ -403,8 +345,6 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
         }
         ptx::tc_fence_before();
         ptx::fence_proxy_async_smem();
-        acc_e2 += (kProf ? clock64() : 0ll) - c_0;
-        c_0 = (kProf ? clock64() : 0ll);
         // each TMEM lane quarter (two warps, 32 rows of the tile) stores its own rows: a 64-thread barrier and four
         // TMA issuers instead of a CTA-wide barrier and one
         ptx::named_bar_sync(4 + q, 64);
@@ -412,19 +352,11 @@ usfgan_block_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_const
           ptx::tma_store_3d(&tm_xout, gb + q * 4096, 0, t0 + q * 32, b);
           ptx::bulk_commit_group();
         }
-        acc_sync += (kProf ? clock64() : 0ll) - c_0;
       }
 #pragma unroll
       for (int i = 0; i < 2; ++i) { xr_prev[i][0] = xr_cur[i][0]; xr_prev[i][1] = xr_cur[i][1]; }
     }
     if (qlead) ptx::bulk_wait_read_all();
-    if (kProf && a.dbg && elected) {
-      a.dbg[blockIdx.x * 16 + 5] = acc_d1;    // epilogue: waiting for D1
-      a.dbg[blockIdx.x * 16 + 6] = acc_gate;  // epilogue: gating + G stores + arrive
-      a.dbg[blockIdx.x * 16 + 7] = acc_d2;    // epilogue: waiting for D2
-      a.dbg[blockIdx.x * 16 + 8] = acc_e2;    // epilogue: residual maths + stores
-      a.dbg[blockIdx.x * 16 + 9] = acc_sync;  // epilogue: named barriers, TMA store issue, store-read waits
-    }
   }
 
   ptx::tc_fence_before();
@@ -524,9 +456,7 @@ extern "C" int svsk_usfgan_block_bf16(const svsk_usfgan_block_params* pp, void* 
   cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
   static bool attr_set[64] = {false};
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(usfgan_block_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(usfgan_block_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(usfgan_block_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+    cudaError_t e = cudaFuncSetAttribute(usfgan_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
     if (e != cudaSuccess) return fail((int)e, "usfgan_block_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
   }
@@ -546,16 +476,7 @@ extern "C" int svsk_usfgan_block_bf16(const svsk_usfgan_block_params* pp, void* 
   a.total_tiles = p.B * a.tiles_per_row;
   a.out_scale = p.out_scale;
   a.out_relu = p.out_relu;
-  a.dbg_flags = 0;
-  a.dbg = nullptr;
-  if (const char* e = getenv("SVSK_USFGAN_ABLATE")) a.dbg_flags = atoi(e);
-  if (const char* e = getenv("SVSK_USFGAN_TIMELINE")) a.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
   const int grid = a.total_tiles < num_sms ? a.total_tiles : num_sms;
-  if (a.dbg)  // clock64 role accounting (distorts the timing) + ablation flags
-    usfgan_block_kernel<true, true><<<grid, kUThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_aux, tm_w1, tm_wout, tm_xout, a);
-  else if (a.dbg_flags)  // ablation flags only
-    usfgan_block_kernel<false, true><<<grid, kUThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_aux, tm_w1, tm_wout, tm_xout, a);
-  else
-    usfgan_block_kernel<false, false><<<grid, kUThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_aux, tm_w1, tm_wout, tm_xout, a);
+  usfgan_block_kernel<<<grid, kUThreads, smem_bytes, as_stream(stream)>>>(tm_x, tm_aux, tm_w1, tm_wout, tm_xout, a);
   return check_launch("usfgan_block_bf16");
 }

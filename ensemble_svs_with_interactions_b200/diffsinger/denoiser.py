@@ -91,6 +91,7 @@ def _block_fp32(layer: ResidualBlock, x, cond, dp, skip=None, init_skip=True):
 
 
 _STACK_FIT_CACHE = {}
+_PCOND_BUDGET_BYTES = 16 << 30   # buffers of the precomputed conditioner projection (cond_projection_bf16)
 
 
 def _stack_tracks_per_launch(B, T, C, H):
@@ -244,10 +245,10 @@ class DiffNet(nn.Module):
             return None
         # three buffers of B * T * L * 2C bf16 each (GEMM output, gate half + filter half): 0.74 GB at BASELINE config 2,
         # 2.2 GB for a 6 x 6000 batch; a batch for which they would not be small next to the model's own tensors keeps the
-        # projection inside the GEMM (SVSK_PCOND_MAX_BYTES, default 16 GB)
+        # projection inside the GEMM (_PCOND_BUDGET_BYTES, 16 GB)
         tiles = 2 * ((T + 255) // 256)
         need = 2 * B * plan.L * 2 * plan.C * (2 * T + tiles * 128)
-        if need > int(os.environ.get("SVSK_PCOND_MAX_BYTES", str(16 << 30))):
+        if need > _PCOND_BUDGET_BYTES:
             return None
         p = ops.diffnet_cond_project(condb.contiguous(), plan.wcp_all)
         return ops.diffnet_pcond_pack(p, B, T, plan.L, plan.C)

@@ -30,7 +30,6 @@ tensor-core kernels at all: their forward stays libsvsk's fp32 path and their ba
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.nn.functional as F
@@ -324,11 +323,10 @@ def _set_launch_count(v):
 _GRAPHS = {}          # shape key -> _GraphedStack (at most _MAX_GRAPHS, least recently used first out)
 _SEEN = {}            # shape key -> times seen (a graph is captured the second time a shape comes by)
 _MAX_GRAPHS = 2
-USE_CUDA_GRAPHS = os.environ.get("SVSK_TRAIN_NO_GRAPH", "0") == "0"      # profiling switch: eager launches only
 
 
 def _graph_for(key, dilations, tensors, need_spec, need_cond):
-    if not USE_CUDA_GRAPHS or torch.cuda.is_current_stream_capturing():
+    if torch.cuda.is_current_stream_capturing():
         return None
     g = _GRAPHS.get(key)
     if g is not None:

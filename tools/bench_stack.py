@@ -1,4 +1,4 @@
-"""Timing and per-layer timeline of the one-launch residual stack at the BASELINE config-2 shape (profiling aid)."""
+"""Timing of the one-launch residual stack at the BASELINE config-2 shape (A/B aid for the stack kernel)."""
 import os
 import sys
 
@@ -60,24 +60,3 @@ b.record(); b.synchronize()
 us = a.elapsed_time(b) * 1e3 / 20
 flops = 2.0 * B * T * (2 * plan.C * (3 * plan.C + plan.H) + 2 * plan.C * plan.C) * plan.L
 print(f"B={B} T={T}: stack of {plan.L} blocks {us:8.1f} us/launch = {us / plan.L:6.2f} us/layer, {flops / us / 1e6:7.1f} TFLOP/s", flush=True)
-
-dbg = torch.zeros(512 * 32, dtype=torch.int64, device="cuda")
-os.environ["SVSK_DIFFNET_TIMELINE"] = str(dbg.data_ptr())
-launch()
-torch.cuda.synchronize()
-os.environ.pop("SVSK_DIFFNET_TIMELINE")
-d = dbg.view(512, 32).cpu()
-d = d[(d[:, 15] > 0) & (d[:, 2] > 0)]
-d[:, 18:] = torch.where(d[:, 18:] == 0, d[:, :1], d[:, 18:])   # stamps a mode does not take
-d[:, 1:16] = torch.where(d[:, 1:16] == 0, d[:, :1], d[:, 1:16])
-names = {24: "epilogue: D2[0] complete", 25: "residual written", 26: "D2[1] complete", 29: "8 skip slabs staged", 30: "G buffer released", 28: "edge thread (row 0) past halo_free", 9: "edge thread residual written",
-         10: "last epilogue warp residual written", 27: "layer 2: xc_ready seen (MMA thread)", 11: "flag published", 12: "neighbours' flags seen",
-         13: "halo loads issued", 14: "G buffer free", 2: "layer 1: centre rows ready (MMA thread)", 3: "halo rows landed", 4: "first cond tile + D1[1] drained", 5: "block 0 issued",
-         6: "block 1 issued", 7: "G ready", 8: "GEMM2 issued", 20: "gating 0 starts", 21: "gating 0 ends", 22: "gating 1 starts",
-         23: "gating 1 ends", 31: "all epilogue threads through layer 1", 18: "layer 2: centre rows ready (MMA thread)",
-         19: "layer 2: first weight tile landed", 15: "kernel end"}
-rel = (d - d[:, :1]).float().median(dim=0).values
-print(f"{d.shape[0]} leader CTAs; median cycles since CTA start: " + " | ".join(f"{n} @{int(rel[i])}" for i, n in names.items()))
-raw = d.float().median(dim=0).values
-print(f"   MMA thread: {int(raw[17])} of {plan.L * 40} ring entries not yet landed when reached, {int(raw[16])} cycles waiting for them")
-print(f"   whole kernel {int(rel[15])} cycles = {int(rel[15]) / plan.L:.0f} per layer")

@@ -1,6 +1,5 @@
 """Three launches of the two-tiles-per-pair C = 128 residual stack at the pipeline's bap shape (6 x 6000 frames, 10 blocks)
-for ncu (kernel replay cannot re-launch a cooperative grid: run with SVSK_STACK_NO_COOPERATIVE=1; 144 CTAs fit the device):
-SVSK_STACK_NO_COOPERATIVE=1 ncu --set full --import-source on -k regex:diffnet_stack_duo -c 3 python tools/prof_stack_duo.py"""
+for a kernel profiler (144 CTAs fit the device; the launch is cooperative, which kernel replay cannot re-launch)."""
 import os
 import sys
 
